@@ -5,6 +5,7 @@
 
     python bench.py [--gpus N --steps K --warmup W]          this repo's sm_100a path
     python bench.py --impl reference [...]                    the reference's CPU path (oracle port)
+    python bench.py [...] --dump-outputs DIR                  also write the last timed step's outputs as DIR/*.npy
 
 One step = MultimodalAttentionPool forward(return_info=True) + CurriculumMasking.entropy_loss +
 backward from an upstream gradient d_out (SURVEY.md section 8d), through the public module API.
@@ -61,7 +62,16 @@ def parse_args():
                     help="replay the step as one CUDA graph (aecf_b200.graphs) instead of enqueueing ~25 kernels from Python")
     ap.add_argument("--fold", choices=["auto", "on", "off"], default="auto",
                     help="folded key projection (auto: the module's choice, on for bf16)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one returned (pool output, info tensors, entropy loss, "
+                         "gradients of x, the fusion query and the parameters) as DIR/<name>.npy in float32, at most 64 MB "
+                         "in all; rank 0 only.  The inputs depend only on the arguments, so two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the sm_100a path: it needs --impl b200")
+    return args
 
 
 def ncu_traffic(kernel: str, args):
@@ -393,6 +403,34 @@ def kernel_averages(sites, steps):
     return {name: {"ms": total / count, "calls_per_step": count / steps} for name, (total, count) in sites.items()}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def sample_outputs(outputs, budget=DUMP_BYTES):
+    """{name: float32 device copy} of the tensors one step returned.  An array larger than its equal share of `budget`
+    keeps a fixed sample of its leading-dimension rows (the first rows of numpy's default_rng(0) permutation, in
+    order), so two builds run with the same arguments dump the same elements."""
+    import numpy as np
+    import torch
+    tensors = {k: v.detach() for k, v in outputs.items() if isinstance(v, torch.Tensor)}
+    share = budget // max(1, len(tensors))
+    kept = {}
+    for name, t in tensors.items():
+        if t.dim() and t.numel() * 4 > share:
+            rows = max(1, share // (4 * max(1, t[0].numel())))
+            idx = np.sort(np.random.default_rng(0).permutation(t.shape[0])[:rows])
+            t = t.index_select(0, torch.from_numpy(idx).to(t.device))
+        kept[name] = t.float().clone()
+    return kept
+
+
+def write_outputs(directory, kept):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in kept.items():
+        np.save(os.path.join(directory, name + ".npy"), t.cpu().numpy())
+
+
 def finish_process(world, nccl_in_graphs=True):
     """With the step captured into CUDA graphs that hold NCCL kernels, destroy_process_group() blocked for minutes on the
     8-GPU box (r1 run 16: the communicator waits for work it believes outstanding); in that case every rank has passed
@@ -457,12 +495,19 @@ def run_b200(args):
     x = xs[0]
     d_out = torch.randn(B, 1, D, device=dev, dtype=dtype)
 
-    def step(xin):
+    def step(xin, outputs=False):
+        """One step; returns the loss, or with `outputs` every tensor its caller receives (static tensors when the step
+        is a graph replay) for --dump-outputs."""
         out, info = pool(query.expand(B, -1, -1), xin, return_info=True)
         loss = cm.entropy_loss(info["entropy"])
         out.backward(d_out)
         sync.finish()
-        return loss
+        if not outputs:
+            return loss
+        grads = {"grad_x": xin.grad, "grad_query": query.grad}
+        grads.update({"grad_" + name: p.grad for name, p in pool.named_parameters()})
+        # detached: a kept result must not hold the autograd graph of its step alive
+        return {k: v.detach() for k, v in {"out": out, **info, "entropy_loss": loss, **grads}.items() if v is not None}
 
     def clear():
         for xi in xs:
@@ -487,10 +532,12 @@ def run_b200(args):
     barrier()
     launches0 = _lib.launch_count()
     turn = [0]
+    dump = bool(args.dump_outputs) and rank == 0
+    last = [None]                                                        # what the last timed step returned (dump only)
     if use_graph:
         graphs = []                                                      # one graph per input batch
         for xi in xs:
-            graphs.append(aecf_b200.graphs.GraphedStep(lambda xi=xi: step(xi), reset=clear, warmup=0, device=dev))
+            graphs.append(aecf_b200.graphs.GraphedStep(lambda xi=xi: step(xi, dump), reset=clear, warmup=0, device=dev))
             if len(graphs) == 1:
                 launches_per_step = _lib.launch_count() - launches0      # counted while capturing one step
         for i in range(max(args.warmup, rot)):
@@ -501,7 +548,10 @@ def run_b200(args):
             turn[0] += 1
     else:
         def run_step():
-            step(xs[turn[0] % rot]); clear()
+            final = dump and turn[0] == args.steps - 1                  # only the last step's outputs are kept
+            result = step(xs[turn[0] % rot], final); clear()
+            if final:
+                last[0] = result
             turn[0] += 1
     barrier()
     launches0 = _lib.launch_count()
@@ -520,6 +570,10 @@ def run_b200(args):
         barrier()
         ms = start.elapsed_time(end) / args.steps
         launches = launches_per_step * args.steps if use_graph else (_lib.launch_count() - launches0)
+        # copied on the device now: the parameter gradients live in the GradientSync bucket, which region B rewrites
+        if dump and use_graph:
+            last[0] = graphs[(args.steps - 1) % rot].result                # the static outputs of the last replay
+        dumped = sample_outputs(last[0]) if dump else None
         clear()
         # region B measures each kernel ON ITS OWN: the gradient tail, which the timed step runs on a side stream next to the
         # [dWv;R] and dX products, is serialised onto the compute stream here (next to a product its kernels take several
@@ -738,6 +792,8 @@ def run_b200(args):
                                           + ("unmodified reference (baseline/_ref), autograd" if kind == "reference"
                                              else "oracle port, closed-form backward")
                                           + f" ({cpu_model()})", "ms_per_step": cpu_ms}
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     print(json.dumps(line))
     barrier()
     finish_process(world, nccl_captured)

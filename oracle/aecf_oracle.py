@@ -16,9 +16,9 @@ at ``:515-521``); torch is an unpinned dependency (``requirements.txt:1``
 reference ``aecf/AECFLayer.py:130-283`` (masking) and ``:285-314`` (loss).
 
 Parity pin.  The reference ships no tests or golden vectors (SURVEY.md section 4), so
-the pin is the reference itself, run in the build container with the shared
-Philox uniforms injected: ``tests/golden/make_golden.py`` imports
-``/root/reference`` and writes ``tests/golden/*.npz``;
+the pin is the reference itself, run with the shared Philox uniforms injected:
+``tests/golden/make_golden.py`` imports the reference checkout that
+``AECF_REFERENCE`` names and writes ``tests/golden/*.npz``;
 ``tests/test_oracle_golden.py`` checks every function here against them.
 
 Random numbers are *inputs* (``u_mask``, ``u_drop``; see ``oracle/philox.py``):

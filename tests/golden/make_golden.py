@@ -1,13 +1,13 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference on the shared cases.
 
-Runs only in the build container (needs /root/reference).  The reference's two random
+Needs a checkout of the reference implementation, named by AECF_REFERENCE.  The reference's two random
 draws are replaced by the shared Philox uniforms exactly as SURVEY.md Appendix C
 describes -- both call sites resolve the function at call time:
 
   * curriculum mask:  ``torch.bernoulli(p)``             (reference aecf/AECFLayer.py:204)
   * attention dropout ``torch.nn.functional.dropout``    (torch/nn/functional.py:6645)
 
-    python tests/golden/make_golden.py            # rewrites every fixture
+    AECF_REFERENCE=<reference checkout> python tests/golden/make_golden.py      # rewrites every fixture
 """
 from __future__ import annotations
 
@@ -20,8 +20,11 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
+MAX_FILE_BYTES = 1_000_000          # no committed fixture file is larger
 sys.path.insert(0, ROOT)
-REFERENCE = os.environ.get("AECF_REFERENCE", "/root/reference")
+REFERENCE = os.environ.get("AECF_REFERENCE", "")
+if not os.path.isfile(os.path.join(REFERENCE, "aecf", "AECFLayer.py")):     # not this repository's alias package
+    sys.exit("set AECF_REFERENCE to a checkout of the reference implementation")
 sys.path.insert(0, REFERENCE)
 
 import aecf as ref  # noqa: E402  (the reference package)
@@ -93,8 +96,13 @@ def main():
     torch.set_num_threads(1)
     for case in CASES + MULTI_QUERY_CASES:
         arrays = run_reference(case)
-        path = os.path.join(HERE, case.name + ".npz")
+        path, more = os.path.join(HERE, case.name + ".npz"), os.path.join(HERE, case.name + ".more.npz")
+        if os.path.exists(more):                      # tests/helpers.py load_golden would merge a stale one
+            os.remove(more)
         np.savez_compressed(path, **arrays)
+        if os.path.getsize(path) > MAX_FILE_BYTES:    # the out-projection weight gradient goes to a second file
+            np.savez_compressed(more, grad_out_proj_weight=arrays.pop("grad_out_proj_weight"))
+            np.savez_compressed(path, **arrays)
         ent = arrays["entropy"].reshape(-1)
         norm = ent / np.log(case.M) if case.M > 1 else ent
         q = np.quantile(norm, [0.1, 0.5, 0.9]) if ent.size else [0, 0, 0]

@@ -17,6 +17,10 @@ GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 def load_golden(case: Case) -> Dict[str, np.ndarray]:
     with np.load(os.path.join(GOLDEN_DIR, case.name + ".npz")) as z:
         g = {k: z[k] for k in z.files}
+    more = os.path.join(GOLDEN_DIR, case.name + ".more.npz")      # what did not fit in one file of at most 1 MB
+    if os.path.exists(more):
+        with np.load(more) as z:
+            g.update({k: z[k] for k in z.files})
     assert json.loads(str(g["meta"])) == case.meta(), "fixture is stale: rerun tests/golden/make_golden.py"
     return g
 

@@ -45,3 +45,37 @@ def test_reference_arm_runs_on_rank_zero_only():
 def test_b200_arm_fails_loudly_without_a_gpu():
     res = _run(["--steps", "1", "--warmup", "1", "--no-e2e", "--no-cpu-baseline"])
     assert res.returncode != 0 and "no CPU path" in res.stderr
+
+
+def test_steps_below_one_are_refused():
+    res = _run(["--steps", "0", "--warmup", "1"])
+    assert res.returncode != 0 and "--steps" in res.stderr
+
+
+def test_dump_outputs_is_refused_for_the_reference_arm(tmp_path):
+    res = _run(["--impl", "reference", "--steps", "1", "--warmup", "1", "--batch", "64", "--dump-outputs", str(tmp_path / "d")])
+    assert res.returncode != 0 and "--dump-outputs" in res.stderr and not os.path.exists(tmp_path / "d")
+
+
+def test_dumped_outputs_are_a_fixed_float32_sample_within_the_budget(tmp_path):
+    import numpy as np
+
+    import bench
+    torch.manual_seed(0)
+    outputs = {"out": torch.randn(1000, 1, 64).bfloat16(), "grad_x": torch.randn(1000, 3, 64),
+               "grad_w": torch.randn(48, 64), "entropy_loss": torch.tensor(0.25), "note": None}
+    budget = 256 << 10
+    a, b = bench.sample_outputs(outputs, budget), bench.sample_outputs(outputs, budget)
+    assert set(a) == {"out", "grad_x", "grad_w", "entropy_loss"}
+    assert sum(t.numel() * 4 for t in a.values()) <= budget
+    assert all(t.dtype == torch.float32 and torch.equal(t, b[k]) for k, t in a.items())
+    assert torch.equal(a["grad_w"], outputs["grad_w"]) and a["entropy_loss"].item() == 0.25     # small arrays whole
+    for k in ("out", "grad_x"):                                  # too large: the first rows of a seeded permutation
+        n = a[k].shape[0]
+        assert 1 <= n < 1000 and a[k].shape[1:] == outputs[k].shape[1:]
+        rows = torch.from_numpy(np.sort(np.random.default_rng(0).permutation(1000)[:n]))
+        assert torch.equal(a[k], outputs[k][rows].float())
+    bench.write_outputs(str(tmp_path), a)
+    for k, t in a.items():
+        got = np.load(tmp_path / f"{k}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, t.numpy())

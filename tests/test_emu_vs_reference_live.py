@@ -1,10 +1,11 @@
-"""The product path (module API -> C ABI -> the CUDA sources under the host emulation, tests/cuda_emu) against the
-UNMODIFIED reference imported live from /root/reference, on the same inputs with the shared Philox draws injected into the
-reference's two RNG call sites (tests/golden/make_golden.py, SURVEY.md Appendix C).  No oracle in between.
+"""The product path (module API -> C ABI -> the CUDA sources under the host emulation, tests/cuda_emu) on seeded random
+shapes and options, including shapes no fixture has (D = 768, H = 3, M = 7 ...).
 
-Runs only where the reference checkout exists (the build container); skipped elsewhere.  The committed fixtures
-(tests/golden/*.npz) are the travelling form of the same comparison for twelve + four fixed cases; here the shapes and
-options are drawn at random (seeded), including shapes no fixture has (D = 768, H = 3, M = 7 ...).
+With AECF_REFERENCE naming a checkout of the reference implementation, the comparison is against that UNMODIFIED
+reference imported live, on the same inputs with the shared Philox draws injected into its two RNG call sites
+(tests/golden/make_golden.py, SURVEY.md Appendix C).  The reference is not part of this repository; without it the same
+cases are compared with the oracle (oracle/aecf_oracle.py), which tests/test_oracle_golden.py pins to the reference's own
+outputs on the committed fixtures.
 """
 import os
 import random
@@ -16,17 +17,18 @@ import torch
 
 import aecf_b200
 from tests.emu_support import cuda_emulation  # noqa: F401  (fixture)
+from oracle import aecf_oracle as oracle
 from tests.golden.cases import PHILOX_SEED, Case, build_inputs, masking_kwargs
-from tests.helpers import assert_close
+from tests.helpers import assert_close, run_oracle
 
-REFERENCE = os.environ.get("AECF_REFERENCE", "/root/reference")
-pytestmark = [pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "aecf")), reason="needs the reference checkout"),
-              pytest.mark.usefixtures("cuda_emulation")]
+REFERENCE = os.environ.get("AECF_REFERENCE", "")
+pytestmark = pytest.mark.usefixtures("cuda_emulation")
 
 
 def _reference_module():
     """The reference's ``aecf`` package under a private name (this repo ships an alias package called ``aecf`` too)."""
     import importlib.util
+    assert os.path.isfile(os.path.join(REFERENCE, "aecf", "AECFLayer.py")), f"AECF_REFERENCE={REFERENCE!r} is not a reference checkout"
     spec = importlib.util.spec_from_file_location("aecf_reference_live", os.path.join(REFERENCE, "aecf", "AECFLayer.py"))
     mod = importlib.util.module_from_spec(spec)
     sys.modules[spec.name] = mod
@@ -68,10 +70,30 @@ class _NoInjection:
         return False
 
 
-@pytest.mark.parametrize("seed", range(6))
-def test_random_cases_against_the_live_reference(monkeypatch, seed):
+def _want_from_reference(case, inp, multi):
     from tests.golden.injection import inject_uniforms
     ref_mod = _reference_module()
+    ref_cm = ref_mod.CurriculumMasking(**masking_kwargs(case))
+    ref_pool = ref_mod.MultimodalAttentionPool(case.D, num_heads=case.H, dropout=case.dropout, curriculum_masking=ref_cm)
+    _load(ref_pool, inp)
+    ref_pool.train(case.training)
+    want = _run(ref_mod, ref_pool, ref_cm, case, inp, multi, inject_uniforms(inp["u_mask"], inp["u_drop"]))
+    return want, ref_cm._last_seq_len
+
+
+def _want_from_oracle(case, inp, multi):
+    """The same step through the oracle: forward, closed-form backward of the same loss, the reference's info keys."""
+    fwd, grads = run_oracle(case, inp)
+    info = {k: v for k, v in fwd.info.items() if k not in ("mask", "keep_prob")}
+    last = case.M if (case.training and case.M > 1) else 2          # the reference's _last_seq_len (AECFLayer.py:99, :187)
+    want = {"out": fwd.out, "info": info, "entropy_loss": oracle.entropy_loss(info["entropy"], last, case.entropy_target),
+            "x": grads["key"], "query": grads["query" if multi else "query0"], "in_w": grads["in_proj_weight"],
+            "in_b": grads["in_proj_bias"], "out_w": grads["out_proj.weight"], "out_b": grads["out_proj.bias"]}
+    return want, last
+
+
+@pytest.mark.parametrize("seed", range(6))
+def test_random_cases_against_the_live_reference(monkeypatch, seed):
     rng = random.Random(7000 + seed)
     multi = seed % 3 == 2
     hd, heads = rng.choice([16, 32, 64, 128]), rng.choice([1, 2, 3, 4, 6, 8])
@@ -83,12 +105,7 @@ def test_random_cases_against_the_live_reference(monkeypatch, seed):
                 training=rng.random() < 0.8, kpm=rng.random() < 0.3, pooled_grad=rng.random() < 0.5, offset=rng.randint(0, 99),
                 row0=rng.choice([0, 11]), data_seed=rng.randint(1000, 10 ** 6), peak=rng.choice([0.5, 1.0, 2.0]))
     inp = build_inputs(case)
-
-    ref_cm = ref_mod.CurriculumMasking(**masking_kwargs(case))
-    ref_pool = ref_mod.MultimodalAttentionPool(case.D, num_heads=case.H, dropout=case.dropout, curriculum_masking=ref_cm)
-    _load(ref_pool, inp)
-    ref_pool.train(case.training)
-    want = _run(ref_mod, ref_pool, ref_cm, case, inp, multi, inject_uniforms(inp["u_mask"], inp["u_drop"]))
+    want, want_last_seq_len = (_want_from_reference if REFERENCE else _want_from_oracle)(case, inp, multi)
 
     cm = aecf_b200.CurriculumMasking(**masking_kwargs(case))
     pool = aecf_b200.MultimodalAttentionPool(case.D, num_heads=case.H, dropout=case.dropout, curriculum_masking=cm)
@@ -111,7 +128,7 @@ def test_random_cases_against_the_live_reference(monkeypatch, seed):
     assert torch.equal((got["info"]["masked_attention_weights"] > 0) & live, want["info"]["masked_attention_weights"] > 0), "active sets differ"
     assert_close("masked_attention_weights", got["info"]["masked_attention_weights"], want["info"]["masked_attention_weights"], tol, atol=tol)
     assert_close("entropy_loss", got["entropy_loss"], want["entropy_loss"], tol, atol=tol)
-    assert cm._last_seq_len == ref_cm._last_seq_len
+    assert cm._last_seq_len == want_last_seq_len
     for name in ("x", "query", "in_w", "out_w", "out_b"):
         assert_close("grad " + name, got[name], want[name], tol)
     scale = float(want["in_b"].abs().max())

@@ -1,5 +1,5 @@
 """Pin the oracle: every function of oracle/aecf_oracle.py against the reference's own outputs
-(tests/golden/*.npz, written by tests/golden/make_golden.py from /root/reference)."""
+(tests/golden/*.npz, written by tests/golden/make_golden.py from the reference checkout that AECF_REFERENCE names)."""
 import math
 
 import numpy as np
