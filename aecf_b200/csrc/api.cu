@@ -75,6 +75,7 @@ struct PoolPlan {
     MultiQuery mq;          // several queries per sample (desc.tgt_len > 1), pool_multi.cuh
     int M, J;
     bool drop, bf16, fold, multi;
+    bool pad;               // padded lane map: head_dim is not a power-of-two number of 16-byte chunks (pool_core.cuh)
 };
 
 // Validate a descriptor and derive the lane/head geometry (pool_core.cuh).  `fold`: the folded-key-projection
@@ -91,21 +92,22 @@ static int make_plan(const aecf_pool_desc* d, PoolPlan* plan, bool fold = false)
     const int V = d->dtype == AECF_BF16 ? 8 : 4;
     const int D = d->embed_dim, H = d->num_heads, hd = D / H;
     if (hd % V != 0) return AECF_ERR_UNSUPPORTED;
-    const int G = hd / V;
-    if (!is_pow2(G)) return AECF_ERR_UNSUPPORTED;
+    const int GR = hd / V;                           // real chunks per head
+    const int G = 1 << ilog2(GR);                    // the head's span in the lane map: GR, or padded to a power of two
     const int NC = D / V;
+    const int NCV = H * G;                           // chunks of the lane map's row (NC unless padded)
     // J chunk columns per lane: enough to hold a whole head in one warp (R <= J), and two columns
     // (512 contiguous bytes x 2 per token) whenever the row is long enough.
     const int R = G < 32 ? 1 : G / 32;
-    int J = NC > 32 ? 2 : 1;
+    int J = NCV > 32 ? 2 : 1;
     if (J < R) J = R;
     if (J > 4) return AECF_ERR_UNSUPPORTED;          // head_dim > 128 * V elements
-    int WPS = (NC + 32 * J - 1) / (32 * J);
+    int WPS = (NCV + 32 * J - 1) / (32 * J);
     // a row must split over a power-of-two number of warps: rows of 3 * 2^k slices (D = 768 in fp32, 1536 in bf16)
     // take wider slices instead, whose last warp is then partly idle
     while ((WPS > POOL_WARPS || !is_pow2(WPS)) && J < 4) {
         J *= 2;
-        WPS = (NC + 32 * J - 1) / (32 * J);
+        WPS = (NCV + 32 * J - 1) / (32 * J);
     }
     if (WPS > POOL_WARPS || !is_pow2(WPS)) return AECF_ERR_UNSUPPORTED;
 
@@ -113,6 +115,7 @@ static int make_plan(const aecf_pool_desc* d, PoolPlan* plan, bool fold = false)
     std::memset(&p, 0, sizeof(p));
     p.B = d->batch; p.D = D; p.H = H; p.NC = NC; p.G = G; p.logG = ilog2(G);
     p.LG = G < 32 ? G : 32; p.R = R; p.WPS = WPS; p.SPC = POOL_WARPS / WPS;
+    p.GR = GR;
     p.scale = static_cast<float>(std::sqrt(1.0 / static_cast<double>(hd)));   // math.sqrt(1.0 / float(E)), functional.py:6632
     p.p_drop = d->dropout_p;
     p.one_minus_p = static_cast<float>(1.0 - static_cast<double>(d->dropout_p));
@@ -167,7 +170,50 @@ static int make_plan(const aecf_pool_desc* d, PoolPlan* plan, bool fold = false)
     plan->M = d->num_tokens; plan->J = J;
     plan->drop = d->training && d->dropout_p > 0.f;
     plan->bf16 = d->dtype == AECF_BF16;
+    plan->pad = GR != G;
     return AECF_OK;
+}
+
+// (dtype, dropout, lane map) -> the instantiation set of pool_dispatch.cuh
+template <bool PAD>
+static int launch_fwd(const PoolPlan& plan, const PoolParams& p, int grid, int sms, bool fold, void* stream) {
+    if (plan.bf16)
+        return plan.drop ? launch_pool_fwd<__nv_bfloat16, true, PAD>(plan.M, plan.J, p, grid, sms, fold, stream)
+                         : launch_pool_fwd<__nv_bfloat16, false, PAD>(plan.M, plan.J, p, grid, sms, fold, stream);
+    return plan.drop ? launch_pool_fwd<float, true, PAD>(plan.M, plan.J, p, grid, sms, fold, stream)
+                     : launch_pool_fwd<float, false, PAD>(plan.M, plan.J, p, grid, sms, fold, stream);
+}
+template <bool PAD>
+static int launch_fwd_multi(const PoolPlan& plan, const PoolParams& p, int grid, void* stream) {
+    if (plan.bf16)
+        return plan.drop ? launch_pool_fwd_multi<__nv_bfloat16, true, PAD>(plan.M, plan.J, p, plan.mq, grid, stream)
+                         : launch_pool_fwd_multi<__nv_bfloat16, false, PAD>(plan.M, plan.J, p, plan.mq, grid, stream);
+    return plan.drop ? launch_pool_fwd_multi<float, true, PAD>(plan.M, plan.J, p, plan.mq, grid, stream)
+                     : launch_pool_fwd_multi<float, false, PAD>(plan.M, plan.J, p, plan.mq, grid, stream);
+}
+template <bool PAD>
+static int launch_bwd(const PoolPlan& plan, const PoolParams& p, int grid, bool fold, void* stream) {
+    if (plan.bf16)
+        return plan.drop ? launch_pool_bwd<__nv_bfloat16, true, PAD>(plan.M, plan.J, p, grid, fold, stream)
+                         : launch_pool_bwd<__nv_bfloat16, false, PAD>(plan.M, plan.J, p, grid, fold, stream);
+    return plan.drop ? launch_pool_bwd<float, true, PAD>(plan.M, plan.J, p, grid, fold, stream)
+                     : launch_pool_bwd<float, false, PAD>(plan.M, plan.J, p, grid, fold, stream);
+}
+template <bool PAD>
+static int launch_bwd_multi(const PoolPlan& plan, const PoolParams& p, int grid, void* stream) {
+    if (plan.bf16)
+        return plan.drop ? launch_pool_bwd_multi<__nv_bfloat16, true, PAD>(plan.M, plan.J, p, plan.mq, grid, stream)
+                         : launch_pool_bwd_multi<__nv_bfloat16, false, PAD>(plan.M, plan.J, p, plan.mq, grid, stream);
+    return plan.drop ? launch_pool_bwd_multi<float, true, PAD>(plan.M, plan.J, p, plan.mq, grid, stream)
+                     : launch_pool_bwd_multi<float, false, PAD>(plan.M, plan.J, p, plan.mq, grid, stream);
+}
+template <bool PAD>
+static int bwd_blocks_per_sm(const PoolPlan& plan, bool fold) {
+    if (plan.bf16)
+        return plan.drop ? pool_bwd_blocks_per_sm<__nv_bfloat16, true, PAD>(plan.M, plan.J, fold)
+                         : pool_bwd_blocks_per_sm<__nv_bfloat16, false, PAD>(plan.M, plan.J, fold);
+    return plan.drop ? pool_bwd_blocks_per_sm<float, true, PAD>(plan.M, plan.J, fold)
+                     : pool_bwd_blocks_per_sm<float, false, PAD>(plan.M, plan.J, fold);
 }
 
 }  // namespace aecf
@@ -232,18 +278,10 @@ static int pool_fwd_impl(const aecf_pool_desc* desc, bool fold, const void* q, c
         plan.mq.bias = score_bias;
         p.bias = nullptr;
         const int rows_grid = static_cast<int>((p.B * plan.mq.S + p.SPC - 1) / p.SPC);
-        if (plan.bf16)
-            return plan.drop ? launch_pool_fwd_multi<__nv_bfloat16, true>(plan.M, plan.J, p, plan.mq, rows_grid, stream)
-                             : launch_pool_fwd_multi<__nv_bfloat16, false>(plan.M, plan.J, p, plan.mq, rows_grid, stream);
-        return plan.drop ? launch_pool_fwd_multi<float, true>(plan.M, plan.J, p, plan.mq, rows_grid, stream)
-                         : launch_pool_fwd_multi<float, false>(plan.M, plan.J, p, plan.mq, rows_grid, stream);
+        return plan.pad ? launch_fwd_multi<true>(plan, p, rows_grid, stream) : launch_fwd_multi<false>(plan, p, rows_grid, stream);
     }
     const int grid = static_cast<int>((p.B + p.SPC - 1) / p.SPC);
-    if (plan.bf16)
-        return plan.drop ? launch_pool_fwd<__nv_bfloat16, true>(plan.M, plan.J, p, grid, sms, fold, stream)
-                         : launch_pool_fwd<__nv_bfloat16, false>(plan.M, plan.J, p, grid, sms, fold, stream);
-    return plan.drop ? launch_pool_fwd<float, true>(plan.M, plan.J, p, grid, sms, fold, stream)
-                     : launch_pool_fwd<float, false>(plan.M, plan.J, p, grid, sms, fold, stream);
+    return plan.pad ? launch_fwd<true>(plan, p, grid, sms, fold, stream) : launch_fwd<false>(plan, p, grid, sms, fold, stream);
 }
 
 extern "C" {
@@ -305,10 +343,7 @@ static int pool_bwd_impl(const aecf_pool_desc* desc, bool fold, const void* q, c
 
     int per_sm;
     if (plan.multi) per_sm = 1;                         // pool_bwd_multi_kernel: __launch_bounds__(256, 1)
-    else if (plan.bf16) per_sm = plan.drop ? pool_bwd_blocks_per_sm<__nv_bfloat16, true>(plan.M, plan.J, fold)
-                                      : pool_bwd_blocks_per_sm<__nv_bfloat16, false>(plan.M, plan.J, fold);
-    else per_sm = plan.drop ? pool_bwd_blocks_per_sm<float, true>(plan.M, plan.J, fold)
-                            : pool_bwd_blocks_per_sm<float, false>(plan.M, plan.J, fold);
+    else per_sm = plan.pad ? bwd_blocks_per_sm<true>(plan, fold) : bwd_blocks_per_sm<false>(plan, fold);
     if (per_sm <= 0) per_sm = 1;
     long long want = (p.B + p.SPC - 1) / p.SPC;
     long long cap = static_cast<long long>(sm_count(desc->device)) * per_sm;   // persistent: one resident wave
@@ -334,18 +369,9 @@ static int pool_bwd_impl(const aecf_pool_desc* desc, bool fold, const void* q, c
         if (plan.multi) {
             plan.mq.bias = score_bias;
             p.bias = nullptr;
-            if (plan.bf16)
-                rc = plan.drop ? launch_pool_bwd_multi<__nv_bfloat16, true>(plan.M, plan.J, p, plan.mq, grid, stream)
-                               : launch_pool_bwd_multi<__nv_bfloat16, false>(plan.M, plan.J, p, plan.mq, grid, stream);
-            else
-                rc = plan.drop ? launch_pool_bwd_multi<float, true>(plan.M, plan.J, p, plan.mq, grid, stream)
-                               : launch_pool_bwd_multi<float, false>(plan.M, plan.J, p, plan.mq, grid, stream);
-        } else if (plan.bf16)
-            rc = plan.drop ? launch_pool_bwd<__nv_bfloat16, true>(plan.M, plan.J, p, grid, fold, stream)
-                           : launch_pool_bwd<__nv_bfloat16, false>(plan.M, plan.J, p, grid, fold, stream);
-        else
-            rc = plan.drop ? launch_pool_bwd<float, true>(plan.M, plan.J, p, grid, fold, stream)
-                           : launch_pool_bwd<float, false>(plan.M, plan.J, p, grid, fold, stream);
+            rc = plan.pad ? launch_bwd_multi<true>(plan, p, grid, stream) : launch_bwd_multi<false>(plan, p, grid, stream);
+        } else
+            rc = plan.pad ? launch_bwd<true>(plan, p, grid, fold, stream) : launch_bwd<false>(plan, p, grid, fold, stream);
     }
     if (rc != AECF_OK) return rc;
     if (no_sums) return AECF_OK;                        // the caller forms the batch sums itself (grad_tail.cu)

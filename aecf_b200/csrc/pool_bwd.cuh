@@ -29,13 +29,14 @@ struct BwdSmem {
 // FOLD (folded key projection, DESIGN.md): kv holds the values only, the scores come precomputed, there is no
 // key pass -- the score gradient ds[b, m, h] itself is stored next to dV (d_kv rows are [dV (D) | ds (HSP)]) and
 // the dX / dW GEMMs that follow contract over D + HSP, which applies and accumulates the rank-H key-side terms.
-template <typename T, int M, int J, bool DROP, bool FOLD>
+// PAD: the padded lane map (pool_core.cuh).
+template <typename T, int M, int J, bool DROP, bool FOLD, bool PAD>
 // The folded variant has no key pass and fits 80 registers without spilling for M * J <= 10 (ptxas -v): three CTAs
 // per SM instead of two, i.e. half as many loads again in flight for a kernel that waits on HBM latency
 // (ncu r1 run 18: long-scoreboard stalls dominate, 25 % of the warp slots occupied).
 __global__ void __launch_bounds__(POOL_WARPS * 32, (FOLD && M * J <= 10 && J <= 2) ? 3 : 2)
 pool_bwd_kernel(const PoolParams p) {
-    using Core = PoolCore<T, M, J, DROP>;
+    using Core = PoolCore<T, M, J, DROP, PAD>;
     using Smem = BwdSmem<J, Core::V>;
     constexpr int V = Core::V;
     constexpr int Q4 = V / 4;
@@ -91,15 +92,22 @@ pool_bwd_kernel(const PoolParams p) {
 
         const char* kv_row = static_cast<const char*>(p.kv) + Core::row_offset(p, src, c0);
         char* dkv_row = static_cast<char*>(p.d_kv) + Core::drow_offset(p, src, c0);
-        auto valid = [&](int j) { return c0 + 32 * j < p.NC; };
+        auto valid = [&](int j) { return Core::valid(p, c0, j); };
 
         // upstream gradient of the context and the values, issued first
         uint4 dcraw[J];
         {
             const char* dc = static_cast<const char*>(p.d_ctx) + static_cast<size_t>(src) * p.D * sizeof(T)
-                             + static_cast<size_t>(c0) * 16;
+                             + Core::lane_bytes(p, c0);
+            // (the power-of-two map keeps the spelling it was measured with: the same arithmetic through Core::col_bytes
+            // changes the register allocation of some of its instantiations, J = 1 above all -- scripts/sass_diff.py)
+            if constexpr (PAD) {
 #pragma unroll
-            for (int j = 0; j < J; ++j) dcraw[j] = valid(j) ? ldg_stream(dc + j * 512) : make_uint4(0, 0, 0, 0);
+                for (int j = 0; j < J; ++j) dcraw[j] = valid(j) ? ldg_stream(dc + Core::col_bytes(p, c0, j)) : make_uint4(0, 0, 0, 0);
+            } else {
+#pragma unroll
+                for (int j = 0; j < J; ++j) dcraw[j] = valid(j) ? ldg_stream(dc + j * 512) : make_uint4(0, 0, 0, 0);
+            }
         }
         uint4 vraw[PRELOAD_V ? M : 1][PRELOAD_V ? J : 1];
         if (PRELOAD_V) {
@@ -108,7 +116,7 @@ pool_bwd_kernel(const PoolParams p) {
 #pragma unroll
                 for (int j = 0; j < J; ++j)
                     vraw[PRELOAD_V ? m : 0][PRELOAD_V ? j : 0] =
-                        valid(j) ? ldg_stream(kv_row + Core::kv_rel(p, m, VHALF, j)) : make_uint4(0, 0, 0, 0);
+                        valid(j) ? ldg_stream(kv_row + Core::kv_rel(p, c0, m, VHALF, j)) : make_uint4(0, 0, 0, 0);
         }
 
         float w[M][J], wd[M][J];
@@ -120,7 +128,7 @@ pool_bwd_kernel(const PoolParams p) {
         } else {
             Core::attention_weights(
                 p, rng, row, c0, qs,
-                [&](int m, int j) { return valid(j) ? ldg_cached(kv_row + Core::kv_rel(p, m, 0, j)) : make_uint4(0, 0, 0, 0); },
+                [&](int m, int j) { return valid(j) ? ldg_cached(kv_row + Core::kv_rel(p, c0, m, 0, j)) : make_uint4(0, 0, 0, 0); },
                 w, wd, keep);
         }
 
@@ -134,7 +142,7 @@ pool_bwd_kernel(const PoolParams p) {
 #pragma unroll
             for (int m = 0; m < M; ++m) {
                 if (PRELOAD_V) raw[m] = vraw[PRELOAD_V ? m : 0][PRELOAD_V ? j : 0];
-                else raw[m] = valid(j) ? ldg_stream(kv_row + Core::kv_rel(p, m, VHALF, j)) : make_uint4(0, 0, 0, 0);
+                else raw[m] = valid(j) ? ldg_stream(kv_row + Core::kv_rel(p, c0, m, VHALF, j)) : make_uint4(0, 0, 0, 0);
             }
             float sum_wd = 0.f;
 #pragma unroll
@@ -146,7 +154,7 @@ pool_bwd_kernel(const PoolParams p) {
                 for (int v = 0; v < V; ++v) { a = fmaf(dc[v], f[v], a); dv[v] = wd[m][j] * dc[v]; }
                 dwd[m][j] = a;
                 sum_wd += wd[m][j];
-                if (row_ok && valid(j)) stg_vec(dkv_row + Core::dkv_rel(p, m, VHALF, j), Vec<T>::pack(dv));
+                if (row_ok && valid(j)) stg_vec(dkv_row + Core::dkv_rel(p, c0, m, VHALF, j), Vec<T>::pack(dv));
             }
             if (row_ok && sums) {
 #pragma unroll
@@ -208,7 +216,7 @@ pool_bwd_kernel(const PoolParams p) {
             if (row_ok && valid(j) && sums) acc_sds[j * 32 + lane] += sum_ds;
             if (FOLD && p.rowsum != nullptr && row_ok) {     // the first lane of each head: [s | sum_m ds] of this sample
                 const int c = c0 + 32 * j;
-                if (c < p.NC && (c & (p.G - 1)) == 0) {
+                if (valid(j) && (c & (p.G - 1)) == 0) {
                     float s_wd = 0.f;
 #pragma unroll
                     for (int m = 0; m < M; ++m) s_wd += wd[m][j];
@@ -227,7 +235,7 @@ pool_bwd_kernel(const PoolParams p) {
 #pragma unroll
                 for (int j = 0; j < J; ++j) {
                     const int c = c0 + 32 * j;
-                    if (c < p.NC && (c & (p.G - 1)) == 0) {
+                    if (valid(j) && (c & (p.G - 1)) == 0) {
                         const int head = c >> p.logG;
 #pragma unroll
                         for (int m = 0; m < M; ++m) line[m * p.dkv_sm + head] = from_float<T>(ds[m][j]);
@@ -245,7 +253,7 @@ pool_bwd_kernel(const PoolParams p) {
             uint4 raw[M];
 #pragma unroll
             for (int m = 0; m < M; ++m)
-                raw[m] = valid(j) ? ldg_cached(kv_row + Core::kv_rel(p, m, 0, j)) : make_uint4(0, 0, 0, 0);
+                raw[m] = valid(j) ? ldg_cached(kv_row + Core::kv_rel(p, c0, m, 0, j)) : make_uint4(0, 0, 0, 0);
             float dq[V];
 #pragma unroll
             for (int v = 0; v < V; ++v) dq[v] = 0.f;
@@ -260,7 +268,7 @@ pool_bwd_kernel(const PoolParams p) {
                     dq[v] = fmaf(ds[m][j], f[v], dq[v]);
                 }
                 sum_ds += ds[m][j];
-                if (row_ok && valid(j)) stg_vec(dkv_row + Core::dkv_rel(p, m, 0, j), Vec<T>::pack(dk));
+                if (row_ok && valid(j)) stg_vec(dkv_row + Core::dkv_rel(p, c0, m, 0, j), Vec<T>::pack(dk));
             }
             if (row_ok) {
                 if (p.q_shared) {
@@ -277,7 +285,7 @@ pool_bwd_kernel(const PoolParams p) {
                     for (int v = 0; v < V; ++v) o[v] = dq[v] * p.scale;
                     if (valid(j))
                         stg_vec(static_cast<char*>(p.d_q) + static_cast<size_t>(row) * p.D * sizeof(T)
-                                    + static_cast<size_t>(c0) * 16 + j * 512, Vec<T>::pack(o));
+                                    + Core::lane_bytes(p, c0) + Core::col_bytes(p, c0, j), Vec<T>::pack(o));
 #pragma unroll
                     for (int q4 = 0; q4 < Q4; ++q4) {
                         float4 a = acc_q[(j * Q4 + q4) * 32 + lane];
@@ -300,7 +308,8 @@ pool_bwd_kernel(const PoolParams p) {
     const float* strips = smem + POOL_WARPS * M;
     for (int i = threadIdx.x + (FOLD ? D : 0); i < 3 * D; i += blockDim.x) {     // folded: there is no d_q third
         const int which = i / D, d = i - which * D;
-        const int c = d / V, v = d - c * V;
+        const int rc = d / V, v = d - rc * V;
+        const int c = Core::virtual_chunk(p, rc);                 // the strips are laid out by lane, i.e. by virtual chunk
         const int sl = c / Core::CPW, cl = c - sl * Core::CPW;
         const int j = cl >> 5, ln = cl & 31;
         const int idx = ((j * Q4 + (v >> 2)) * 32 + ln) * 4 + (v & 3);

@@ -9,9 +9,17 @@
 // inside one chunk column, for G > 32 it is all 32 lanes of R = G / 32 consecutive columns
 // (R <= J, so a head never straddles warps).  Per-head dot products are segmented xor-shuffle
 // reductions; afterwards every lane of a head holds the head's value.
+// Heads of GR chunks with GR not a power of two (head_dim 48, 80, 96, ...: the PAD instantiations) are
+// padded in the lane map to G = the next power of two: slices, J and WPS are then those of a VIRTUAL row
+// of H * G chunks, virtual chunk v belongs to head v >> logG at offset o = v & (G - 1), and it is real chunk
+// (v >> logG) * GR + o when o < GR, else an idle lane that loads zeros, joins its head's butterflies
+// and stores nothing.  Everything per head (butterflies, head sums, Philox keys) is the same code for
+// both maps; only addresses, validity tests and the indices of real columns go through the map.
 // Heads are independent everywhere except the head-mean of the forward (and of the eval-mode
 // entropy gradient), which crosses warps through shared memory when WPS > 1.
 #pragma once
+
+#include <cstddef>
 
 #include "common.cuh"
 
@@ -21,7 +29,8 @@ constexpr int POOL_WARPS = 8;               // warps per CTA for both directions
 
 struct PoolParams {
     long long B;
-    int D, H, NC, G, logG, LG, R;           // LG = min(G, 32) lanes per head group, R = max(1, G / 32)
+    int D, H, NC, G, logG, LG, R;           // LG = min(G, 32) lanes per head group, R = max(1, G / 32); G = 2^logG is the
+                                            // head's span in the lane map (padded map: GR rounded up, see the end)
     int WPS, SPC;                           // warps per sample, samples per CTA (WPS * SPC = POOL_WARPS)
     float scale, p_drop, one_minus_p, base_mask_prob, log_m;   // one_minus_p = float(1.0 - double(p_drop))
     int training, masking, min_active, q_shared;   // masking: 0 off, 1 training-mode stage, 2 eval-mode stage
@@ -63,7 +72,13 @@ struct PoolParams {
     float* loss_partials;                   // [gridDim.x] per-CTA sums of (scrubbed entropy - target)^2
     unsigned* loss_ticket;                  // [2]: CTAs done; zero on entry and on exit
     float loss_target;
+    // padded lane map (PoolCore<..., PAD = true>): GR real chunks per head (power-of-two heads: GR = G; only the PAD
+    // instantiations read it).  It fills the 4 bytes of tail padding behind loss_target: sizeof(PoolParams) is unchanged,
+    // and with it the code of the existing kernels (a larger parameter block changes their register allocation).
+    int GR;
 };
+static_assert(sizeof(PoolParams) % 8 == 0 && offsetof(PoolParams, GR) + sizeof(int) == sizeof(PoolParams),
+              "GR must sit in the tail padding of PoolParams");
 
 constexpr int POOL_LOSS_MAX_CTAS = 4096;    // loss workspace: POOL_LOSS_MAX_CTAS floats + 64 bytes of counters
 
@@ -87,36 +102,72 @@ __device__ __forceinline__ long long source_row(const PoolParams& p, long long r
     return p.row_index != nullptr ? __ldg(p.row_index + row) : row;
 }
 
-template <typename T, int M, int J, bool DROP>
+// PAD: the padded lane map (head of GR chunks, GR not a power of two; see the top of the file).  PAD = false is the
+// power-of-two map, and every function below reduces to the same expression it has always been for it.
+template <typename T, int M, int J, bool DROP, bool PAD = false>
 struct PoolCore {
     static constexpr int V = Vec<T>::N;
     static constexpr int CPW = 32 * J;               // chunks per warp slice
 
+    // ---- lane map: the lane with first chunk c0 owns the (virtual) chunks c0 + 32 j, j < J --------------------------
+    // real chunk of virtual chunk v (meaningful when v is valid)
+    static __device__ __forceinline__ int real_chunk(const PoolParams& p, int v) {
+        if constexpr (PAD) return (v >> p.logG) * p.GR + (v & (p.G - 1));
+        else return v;
+    }
+    // virtual chunk of real chunk c (the per-warp strips are laid out by virtual chunk)
+    static __device__ __forceinline__ int virtual_chunk(const PoolParams& p, int c) {
+        if constexpr (PAD) return ((c / p.GR) << p.logG) + c % p.GR;
+        else return c;
+    }
+    // column j of this lane holds a real chunk ...
+    static __device__ __forceinline__ bool valid(const PoolParams& p, int c0, int j) {
+        if constexpr (PAD) return c0 + 32 * j < (p.H << p.logG) && ((c0 + 32 * j) & (p.G - 1)) < p.GR;
+        else return c0 + 32 * j < p.NC;
+    }
+    // ... or at least lies inside a head (an idle padding lane still holds its head's reduced values)
+    static __device__ __forceinline__ bool in_head(const PoolParams& p, int c0, int j) {
+        if constexpr (PAD) return c0 + 32 * j < (p.H << p.logG);
+        else return c0 + 32 * j < p.NC;
+    }
+    // byte offset of this lane's column-0 chunk inside a row, and of its column j relative to that.  Padded: 32 lanes
+    // still cover 32 / G whole heads = 32 GR / G contiguous real chunks, so a warp access stays one contiguous run.
+    // Column j starts 32 j virtual chunks after column 0 at the same offset inside a head (G <= 32), or at offset + 32 j
+    // inside the same slice of heads (G > 32: slices start on head boundaries): either way real_chunk(32 j) real chunks
+    // further, the same for every lane, so the offsets stay in uniform registers.
+    static __device__ __forceinline__ size_t lane_bytes(const PoolParams& p, int c0) {
+        return static_cast<size_t>(real_chunk(p, c0)) * 16;
+    }
+    static __device__ __forceinline__ int col_bytes(const PoolParams& p, int c0, int j) {
+        if constexpr (PAD) return real_chunk(p, 32 * j) * 16;
+        else return j * 512;
+    }
+
     // byte offset of this lane's first chunk (c0) of `row` inside kv / d_kv ...
     static __device__ __forceinline__ size_t row_offset(const PoolParams& p, long long row, int c0) {
-        return static_cast<size_t>(row) * p.kv_sb * sizeof(T) + static_cast<size_t>(c0) * 16;
+        return static_cast<size_t>(row) * p.kv_sb * sizeof(T) + lane_bytes(p, c0);
     }
     // ... and, relative to it, of chunk column j of the K half (half = 0) or V half (half = 1) of token m
-    static __device__ __forceinline__ int kv_rel(const PoolParams& p, int m, int half, int j) {
-        return (m * static_cast<int>(p.kv_sm) + half * p.D) * static_cast<int>(sizeof(T)) + j * 512;
+    static __device__ __forceinline__ int kv_rel(const PoolParams& p, int c0, int m, int half, int j) {
+        return (m * static_cast<int>(p.kv_sm) + half * p.D) * static_cast<int>(sizeof(T)) + col_bytes(p, c0, j);
     }
 
     // the same two offsets inside d_kv (its rows are wider than kv's in the folded layout)
     static __device__ __forceinline__ size_t drow_offset(const PoolParams& p, long long row, int c0) {
-        return static_cast<size_t>(row) * p.dkv_sb * sizeof(T) + static_cast<size_t>(c0) * 16;
+        return static_cast<size_t>(row) * p.dkv_sb * sizeof(T) + lane_bytes(p, c0);
     }
-    static __device__ __forceinline__ long long dkv_rel(const PoolParams& p, int m, int half, int j) {
-        return (m * p.dkv_sm + half * p.D) * static_cast<long long>(sizeof(T)) + j * 512;
+    static __device__ __forceinline__ long long dkv_rel(const PoolParams& p, int c0, int m, int half, int j) {
+        return (m * p.dkv_sm + half * p.D) * static_cast<long long>(sizeof(T)) + col_bytes(p, c0, j);
     }
 
     // projected query chunks, pre-multiplied by scale (torch/nn/functional.py:6632)
     static __device__ __forceinline__ void load_query(const PoolParams& p, long long row, int c0, float (&qs)[J][V]) {
 #pragma unroll
         for (int j = 0; j < J; ++j) {
-            const int c = c0 + 32 * j;
+            const int c = real_chunk(p, c0 + 32 * j);
 #pragma unroll
             for (int v = 0; v < V; ++v) qs[j][v] = 0.f;
-            if (c < p.NC) {
+            if (valid(p, c0, j)) {
                 if (p.q_shared) {
                     const float* q = static_cast<const float*>(p.q) + static_cast<size_t>(c) * V;
 #pragma unroll
@@ -198,7 +249,7 @@ struct PoolCore {
         for (int m = 0; m < M; ++m) {
             float t = 0.f;
 #pragma unroll
-            for (int j = 0; j < J; ++j) t += (c0 + 32 * j < p.NC) ? x[m][j] : 0.f;
+            for (int j = 0; j < J; ++j) t += in_head(p, c0, j) ? x[m][j] : 0.f;
             part[m] = t;
         }
         if (p.LG == 8) butterfly<8, 32>(part);       // distances LG .. 16; the two common geometries unrolled

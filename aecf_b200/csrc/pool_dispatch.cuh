@@ -27,14 +27,15 @@ namespace aecf {
         default: return AECF_ERR_UNSUPPORTED;                 \
     }
 
-// J = chunk columns per lane (1, 2, 4); DROP = attention dropout active.
+// J = chunk columns per lane (1, 2, 4); DROP = attention dropout active; PAD = padded lane map (head_dim not a
+// power-of-two number of chunks, pool_core.cuh).
 // grid: CTAs of the slice kernel; sms: SM count (the streaming kernel sizes its persistent grid from it)
 // fold: the folded-key-projection variants (values only in kv, precomputed scores)
-template <typename T, bool DROP> int launch_pool_fwd(int M, int J, const PoolParams& p, int grid, int sms, bool fold, void* stream);
-template <typename T, bool DROP> int launch_pool_bwd(int M, int J, const PoolParams& p, int grid, bool fold, void* stream);
-template <typename T, bool DROP> int pool_bwd_blocks_per_sm(int M, int J, bool fold);
+template <typename T, bool DROP, bool PAD> int launch_pool_fwd(int M, int J, const PoolParams& p, int grid, int sms, bool fold, void* stream);
+template <typename T, bool DROP, bool PAD> int launch_pool_bwd(int M, int J, const PoolParams& p, int grid, bool fold, void* stream);
+template <typename T, bool DROP, bool PAD> int pool_bwd_blocks_per_sm(int M, int J, bool fold);
 // several fusion queries per sample (pool_multi.cuh); the backward runs one CTA per SM
-template <typename T, bool DROP> int launch_pool_fwd_multi(int M, int J, const PoolParams& p, const MultiQuery& mq, int grid, void* stream);
-template <typename T, bool DROP> int launch_pool_bwd_multi(int M, int J, const PoolParams& p, const MultiQuery& mq, int grid, void* stream);
+template <typename T, bool DROP, bool PAD> int launch_pool_fwd_multi(int M, int J, const PoolParams& p, const MultiQuery& mq, int grid, void* stream);
+template <typename T, bool DROP, bool PAD> int launch_pool_bwd_multi(int M, int J, const PoolParams& p, const MultiQuery& mq, int grid, void* stream);
 
 }  // namespace aecf

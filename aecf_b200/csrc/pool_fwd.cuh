@@ -88,10 +88,11 @@ __device__ __forceinline__ void masking_stage(const PoolParams& p, const RngKey&
 }
 
 // FOLD: folded key projection -- kv holds the values only and the scores come precomputed (pool_core.cuh).
-template <typename T, int M, int J, bool DROP, bool FOLD>
+// PAD: the padded lane map (pool_core.cuh).
+template <typename T, int M, int J, bool DROP, bool FOLD, bool PAD>
 __global__ void __launch_bounds__(POOL_WARPS * 32)
 pool_fwd_kernel(const PoolParams p) {
-    using Core = PoolCore<T, M, J, DROP>;
+    using Core = PoolCore<T, M, J, DROP, PAD>;
     constexpr int V = Core::V;
     constexpr int VHALF = FOLD ? 0 : 1;                 // which D-wide half of a kv row holds the values
     __shared__ float xchg[POOL_WARPS * M];
@@ -110,7 +111,7 @@ pool_fwd_kernel(const PoolParams p) {
 
     const char* kv_row = static_cast<const char*>(p.kv) + Core::row_offset(p, src, c0);
     auto load_kv = [&](int m, int half, int j) -> uint4 {
-        return (c0 + 32 * j < p.NC) ? ldg_stream(kv_row + Core::kv_rel(p, m, half, j)) : make_uint4(0, 0, 0, 0);
+        return Core::valid(p, c0, j) ? ldg_stream(kv_row + Core::kv_rel(p, c0, m, half, j)) : make_uint4(0, 0, 0, 0);
     };
 
     // Issue the value loads first when they fit in registers: the whole slice is then in flight
@@ -157,10 +158,16 @@ pool_fwd_kernel(const PoolParams p) {
         }
     }
     if (row_ok) {
-        char* ctx = static_cast<char*>(p.ctx) + static_cast<size_t>(src) * p.D * sizeof(T) + static_cast<size_t>(c0) * 16;
+        char* ctx = static_cast<char*>(p.ctx) + static_cast<size_t>(src) * p.D * sizeof(T) + Core::lane_bytes(p, c0);
+        if constexpr (PAD) {
 #pragma unroll
-        for (int j = 0; j < J; ++j)
-            if (c0 + 32 * j < p.NC) stg_vec(ctx + j * 512, Vec<T>::pack(acc[j]));
+            for (int j = 0; j < J; ++j)
+                if (Core::valid(p, c0, j)) stg_vec(ctx + Core::col_bytes(p, c0, j), Vec<T>::pack(acc[j]));
+        } else {    // the original spelling, which compiles to the measured kernels' code (see pool_bwd.cuh)
+#pragma unroll
+            for (int j = 0; j < J; ++j)
+                if (c0 + 32 * j < p.NC) stg_vec(ctx + j * 512, Vec<T>::pack(acc[j]));
+        }
     }
 
     // ---- head sums of the post-dropout weights -> shared memory ----------------------------------
@@ -210,10 +217,13 @@ pool_fwd_kernel(const PoolParams p) {
 // DENSE (folded only): every lane owns J valid chunks (D = 32 J chunks exactly) and a sample's M value rows are contiguous,
 // so chunk (m, j) sits at the compile-time offset (m J + j) * 512 and no access needs a validity test -- 50 of the generic
 // kernel's 493 instructions per sample were address arithmetic and tests of exactly that (ncu source page, r2 run 26).
-template <typename T, int M, int J, bool DROP, bool FOLD, bool DENSE = false>
+// PAD (padded lane map) is never DENSE: each lane copies exactly its own valid chunks, at their real addresses, into its own
+// ring slots and reads back only those, so the ring keeps its own-copies-only wait.
+template <typename T, int M, int J, bool DROP, bool FOLD, bool DENSE, bool PAD>
 __global__ void __launch_bounds__((FOLD && J <= 2) ? 768 : 512, 1)
 pool_fwd_stream_kernel(const PoolParams p, const long long rows_per_warp) {
-    using Core = PoolCore<T, M, J, DROP>;
+    static_assert(!(DENSE && PAD), "the dense specialisation assumes the power-of-two lane map");
+    using Core = PoolCore<T, M, J, DROP, PAD>;
     constexpr int V = Core::V;
     constexpr int HALVES = FOLD ? 1 : 2;                // folded: only the values are staged
     constexpr int VHALF = FOLD ? 0 : 1;
@@ -248,9 +258,9 @@ pool_fwd_stream_kernel(const PoolParams p, const long long rows_per_warp) {
             for (int half = 0; half < HALVES; ++half)
 #pragma unroll
                 for (int j = 0; j < J; ++j)
-                    if (DENSE || c0 + 32 * j < p.NC)
+                    if (DENSE || Core::valid(p, c0, j))
                         cp_async16(&my[(stage * CH + (m * HALVES + half) * J + j) * 32 + lane],
-                                   src + (DENSE ? (m * J + j) * 512 : Core::kv_rel(p, m, half, j)));
+                                   src + (DENSE ? (m * J + j) * 512 : Core::kv_rel(p, c0, m, half, j)));
         cp_async_commit();
     };
     if (row_begin < row_end) prefetch(row_begin, 0);
@@ -282,7 +292,7 @@ pool_fwd_stream_kernel(const PoolParams p, const long long rows_per_warp) {
         }
         cp_async_wait<1>();                             // this row's chunks have landed (own copies only)
         auto staged = [&](int m, int half, int j) -> uint4 {
-            return (DENSE || c0 + 32 * j < p.NC) ? my[(stage * CH + (m * HALVES + half) * J + j) * 32 + lane] : make_uint4(0, 0, 0, 0);
+            return (DENSE || Core::valid(p, c0, j)) ? my[(stage * CH + (m * HALVES + half) * J + j) * 32 + lane] : make_uint4(0, 0, 0, 0);
         };
 
         float w[M][J], wd[M][J];
@@ -304,10 +314,16 @@ pool_fwd_stream_kernel(const PoolParams p, const long long rows_per_warp) {
 #pragma unroll
                 for (int v = 0; v < V; ++v) acc[j][v] = fmaf(wd[m][j], f[v], acc[j][v]);
             }
-        char* ctx = static_cast<char*>(p.ctx) + static_cast<size_t>(row) * p.D * sizeof(T) + static_cast<size_t>(c0) * 16;
+        char* ctx = static_cast<char*>(p.ctx) + static_cast<size_t>(row) * p.D * sizeof(T) + Core::lane_bytes(p, c0);
+        if constexpr (PAD) {
 #pragma unroll
-        for (int j = 0; j < J; ++j)
-            if (DENSE || c0 + 32 * j < p.NC) stg_vec(ctx + j * 512, Vec<T>::pack(acc[j]));
+            for (int j = 0; j < J; ++j)
+                if (Core::valid(p, c0, j)) stg_vec(ctx + Core::col_bytes(p, c0, j), Vec<T>::pack(acc[j]));
+        } else {    // the original spelling, which compiles to the measured kernels' code (see pool_bwd.cuh)
+#pragma unroll
+            for (int j = 0; j < J; ++j)
+                if (DENSE || c0 + 32 * j < p.NC) stg_vec(ctx + j * 512, Vec<T>::pack(acc[j]));
+        }
 
         float total[M];
         Core::head_sum_partial(p, c0, wd, total);       // WPS == 1: the warp holds every head

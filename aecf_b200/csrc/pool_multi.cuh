@@ -34,10 +34,11 @@ __device__ __forceinline__ void add_score_bias(const PoolParams& p, const MultiQ
     }
 }
 
-template <typename T, int M, int J, bool DROP>
+// PAD: the padded lane map (pool_core.cuh).
+template <typename T, int M, int J, bool DROP, bool PAD>
 __global__ void __launch_bounds__(POOL_WARPS * 32)
 pool_fwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
-    using Core = PoolCore<T, M, J, DROP>;
+    using Core = PoolCore<T, M, J, DROP, PAD>;
     constexpr int V = Core::V;
     __shared__ float xchg[POOL_WARPS * M];
     __shared__ float head_sums[POOL_WARPS * M];       // [row slot][m], written by the slice-0 warps
@@ -58,7 +59,7 @@ pool_fwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
 
     const char* kv_row = static_cast<const char*>(p.kv) + Core::row_offset(p, b, c0);
     auto load_kv = [&](int m, int half, int j) -> uint4 {
-        return (c0 + 32 * j < p.NC) ? ldg_cached(kv_row + Core::kv_rel(p, m, half, j)) : make_uint4(0, 0, 0, 0);
+        return Core::valid(p, c0, j) ? ldg_cached(kv_row + Core::kv_rel(p, c0, m, half, j)) : make_uint4(0, 0, 0, 0);
     };
 
     float qs[J][V];
@@ -85,10 +86,16 @@ pool_fwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
             for (int v = 0; v < V; ++v) acc[j][v] = fmaf(wd[m][j], f[v], acc[j][v]);
         }
     if (row_ok) {
-        char* ctx = static_cast<char*>(p.ctx) + static_cast<size_t>(qrow) * p.D * sizeof(T) + static_cast<size_t>(c0) * 16;
+        char* ctx = static_cast<char*>(p.ctx) + static_cast<size_t>(qrow) * p.D * sizeof(T) + Core::lane_bytes(p, c0);
+        if constexpr (PAD) {
 #pragma unroll
-        for (int j = 0; j < J; ++j)
-            if (c0 + 32 * j < p.NC) stg_vec(ctx + j * 512, Vec<T>::pack(acc[j]));
+            for (int j = 0; j < J; ++j)
+                if (Core::valid(p, c0, j)) stg_vec(ctx + Core::col_bytes(p, c0, j), Vec<T>::pack(acc[j]));
+        } else {    // the original spelling, which compiles to the measured kernels' code (see pool_bwd.cuh)
+#pragma unroll
+            for (int j = 0; j < J; ++j)
+                if (c0 + 32 * j < p.NC) stg_vec(ctx + j * 512, Vec<T>::pack(acc[j]));
+        }
     }
 
     // ---- head sums of the post-dropout weights -> shared memory; warp 0 finishes the CTA's rows -----
@@ -125,10 +132,10 @@ pool_fwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
 // the sums over its S rows, d_q is per row.  The strips accumulate d_bias_v and d_bias_k (= sum dK) as in the
 // per-row-query mode of pool_bwd_kernel, and are folded into partials in the same layout, so the same finalize
 // kernel applies.  One CTA per SM: the fp32 dK / dV accumulators take 2*M*J*V registers per lane.
-template <typename T, int M, int J, bool DROP>
+template <typename T, int M, int J, bool DROP, bool PAD>
 __global__ void __launch_bounds__(POOL_WARPS * 32, 1)
 pool_bwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
-    using Core = PoolCore<T, M, J, DROP>;
+    using Core = PoolCore<T, M, J, DROP, PAD>;
     using Smem = BwdSmem<J, Core::V>;
     constexpr int V = Core::V;
     constexpr int Q4 = V / 4;
@@ -147,7 +154,7 @@ pool_bwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
 
     const int slice = warp % p.WPS;
     const int c0 = slice * Core::CPW + lane;
-    auto valid = [&](int j) { return c0 + 32 * j < p.NC; };
+    auto valid = [&](int j) { return Core::valid(p, c0, j); };
 
     const long long stride = static_cast<long long>(gridDim.x) * p.SPC;
     for (long long base = static_cast<long long>(blockIdx.x) * p.SPC; base < p.B; base += stride) {
@@ -157,7 +164,7 @@ pool_bwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
         const char* kv_row = static_cast<const char*>(p.kv) + Core::row_offset(p, b, c0);
         char* dkv_row = static_cast<char*>(p.d_kv) + Core::drow_offset(p, b, c0);
         auto load_kv = [&](int m, int half, int j) -> uint4 {
-            return valid(j) ? ldg_cached(kv_row + Core::kv_rel(p, m, half, j)) : make_uint4(0, 0, 0, 0);
+            return valid(j) ? ldg_cached(kv_row + Core::kv_rel(p, c0, m, half, j)) : make_uint4(0, 0, 0, 0);
         };
 
         float dk_acc[M][J][V], dv_acc[M][J][V];
@@ -176,9 +183,14 @@ pool_bwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
             uint4 dcraw[J];
             {
                 const char* dc = static_cast<const char*>(p.d_ctx) + static_cast<size_t>(qrow) * p.D * sizeof(T)
-                                 + static_cast<size_t>(c0) * 16;
+                                 + Core::lane_bytes(p, c0);
+                if constexpr (PAD) {
 #pragma unroll
-                for (int j = 0; j < J; ++j) dcraw[j] = valid(j) ? ldg_stream(dc + j * 512) : make_uint4(0, 0, 0, 0);
+                    for (int j = 0; j < J; ++j) dcraw[j] = valid(j) ? ldg_stream(dc + Core::col_bytes(p, c0, j)) : make_uint4(0, 0, 0, 0);
+                } else {    // the original spelling, which compiles to the measured kernels' code (see pool_bwd.cuh)
+#pragma unroll
+                    for (int j = 0; j < J; ++j) dcraw[j] = valid(j) ? ldg_stream(dc + j * 512) : make_uint4(0, 0, 0, 0);
+                }
             }
 
             float sc[M][J], w[M][J], wd[M][J];
@@ -286,7 +298,7 @@ pool_bwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
                     for (int v = 0; v < V; ++v) o[v] = dq[v] * p.scale;
                     if (valid(j))
                         stg_vec(static_cast<char*>(p.d_q) + static_cast<size_t>(qrow) * p.D * sizeof(T)
-                                    + static_cast<size_t>(c0) * 16 + j * 512, Vec<T>::pack(o));
+                                    + Core::lane_bytes(p, c0) + Core::col_bytes(p, c0, j), Vec<T>::pack(o));
 #pragma unroll
                     for (int q4 = 0; q4 < Q4; ++q4) {                  // d_bias_k = sum dK
                         float4 a = acc_bk[(j * Q4 + q4) * 32 + lane];
@@ -304,8 +316,8 @@ pool_bwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
 #pragma unroll
                 for (int j = 0; j < J; ++j)
                     if (valid(j)) {
-                        stg_vec(dkv_row + Core::dkv_rel(p, m, 0, j), Vec<T>::pack(dk_acc[m][j]));
-                        stg_vec(dkv_row + Core::dkv_rel(p, m, 1, j), Vec<T>::pack(dv_acc[m][j]));
+                        stg_vec(dkv_row + Core::dkv_rel(p, c0, m, 0, j), Vec<T>::pack(dk_acc[m][j]));
+                        stg_vec(dkv_row + Core::dkv_rel(p, c0, m, 1, j), Vec<T>::pack(dv_acc[m][j]));
                     }
         }
     }
@@ -318,7 +330,8 @@ pool_bwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
     const float* strips = smem + POOL_WARPS * M;
     for (int i = threadIdx.x; i < 3 * D; i += blockDim.x) {
         const int which = i / D, d = i - which * D;
-        const int c = d / V, v = d - c * V;
+        const int rc = d / V, v = d - rc * V;
+        const int c = Core::virtual_chunk(p, rc);
         const int sl = c / Core::CPW, cl = c - sl * Core::CPW;
         const int j = cl >> 5, ln = cl & 31;
         const int idx = ((j * Q4 + (v >> 2)) * 32 + ln) * 4 + (v & 3);

@@ -73,7 +73,7 @@ typedef struct aecf_pool_desc {
     int64_t  batch;           /* B: rows in this call (>= 0; 0 is a no-op) */
     int32_t  num_tokens;      /* M: modality tokens per row, 1..AECF_MAX_TOKENS */
     int32_t  embed_dim;       /* D */
-    int32_t  num_heads;       /* H, divides D; D/H must be (16 bytes / element size) * 2^k */
+    int32_t  num_heads;       /* H, divides D; D/H must be a multiple of 16 bytes, at most 128 such chunks */
     int32_t  training;        /* attention module in training mode (enables dropout) */
     int32_t  masking;         /* 0: no CurriculumMasking stage; 1: module in training mode; 2: in eval mode */
     int32_t  min_active;      /* CurriculumMasking.min_active */

@@ -17,7 +17,7 @@ rng = random.Random(int(sys.argv[1]) if len(sys.argv) > 1 else 0)
 budget = float(sys.argv[2]) if len(sys.argv) > 2 else 300
 t0 = time.time(); n = 0; fails = 0
 while time.time() - t0 < budget:
-    hd = rng.choice([8, 16, 32, 64, 128])
+    hd = rng.choice([8, 16, 24, 32, 48, 64, 80, 96, 128])    # 24 .. 96: heads of a non-power-of-two number of chunks
     H = rng.choice([1, 2, 3, 4, 5, 6, 8, 12, 16])
     D = hd * H
     if D > 768: continue

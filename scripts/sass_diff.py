@@ -2,6 +2,9 @@
 
     python scripts/sass_diff.py snapshot DIR          # cuobjdump -sass of every aecf_b200/csrc/build/*.o into DIR
     python scripts/sass_diff.py compare BEFORE AFTER   # functions whose instruction stream differs, added, removed
+    python scripts/sass_diff.py compare BEFORE AFTER --pair ARG
+                                                       # the same, after a new trailing template argument: an old function
+                                                       # is compared with the new one whose last template argument is ARG
     python scripts/sass_diff.py manifest DIR OUT.json  # {demangled function: [sha1, instructions]} of a snapshot
     python scripts/sass_diff.py check OUT.json DIR     # a snapshot against a committed manifest (exit 1 on a change)
 
@@ -54,8 +57,28 @@ def load(directory):
     return table
 
 
-def compare(before, after):
+def paired(a, b, arg):
+    """Rename the functions of `b` whose last template argument is `arg` to the name they had without it (when `a` has
+    that name), e.g. f<float, 3, false> -> f<float, 3> for arg = "false"."""
+    names = demangle_all(sorted(b))
+    old = {v: k for k, v in demangle_all(sorted(a)).items()}
+    out, pairs = {}, 0
+    for k, v in b.items():
+        head, sep, tail = names[k].rpartition(f", {arg}>(")
+        key = old.get(head + ">(" + tail) if sep else None
+        if key is not None:
+            out[key] = v
+            pairs += 1
+        else:
+            out[k] = v
+    print(f"{pairs} functions paired with their name before the trailing template argument {arg}")
+    return out
+
+
+def compare(before, after, pair=None):
     a, b = load(before), load(after)
+    if pair is not None:
+        b = paired(a, b, pair)
     changed = sorted(k for k in a if k in b and a[k] != b[k])
     removed = sorted(k for k in a if k not in b)
     added = sorted(k for k in b if k not in a)
@@ -104,7 +127,7 @@ if __name__ == "__main__":
     if len(sys.argv) >= 3 and sys.argv[1] == "snapshot":
         snapshot(sys.argv[2])
     elif len(sys.argv) >= 4 and sys.argv[1] == "compare":
-        sys.exit(compare(sys.argv[2], sys.argv[3]))
+        sys.exit(compare(sys.argv[2], sys.argv[3], sys.argv[5] if len(sys.argv) >= 6 and sys.argv[4] == "--pair" else None))
     elif len(sys.argv) >= 4 and sys.argv[1] == "manifest":
         manifest(sys.argv[2], sys.argv[3])
     elif len(sys.argv) >= 4 and sys.argv[1] == "check":
