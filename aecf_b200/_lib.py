@@ -12,7 +12,7 @@ from typing import Optional
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "csrc", "libaecf_b200.so")
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 # enums of include/aecf_b200.h
 F32, BF16 = 0, 1
@@ -89,7 +89,6 @@ class FusionGrads(C.Structure):
         "side_stream", "fork_event", "fork_event2", "join_event")] + [("dp", C.POINTER(DpDesc))]
 
 
-BWD_ALL, BWD_OUT_PROJ, BWD_REST = 0, 1, 2
 SITE_COUNT = 21
 
 
@@ -166,8 +165,7 @@ def _declare(lib):
     lib.aecf_fusion_fwd.restype = C.c_int
     lib.aecf_fusion_fwd.argtypes = [C.POINTER(PoolDesc), C.POINTER(FusionTensors), vp, C.c_size_t, vp]
     lib.aecf_fusion_bwd.restype = C.c_int
-    lib.aecf_fusion_bwd.argtypes = [C.POINTER(PoolDesc), C.POINTER(FusionTensors), C.POINTER(FusionGrads), C.c_int32,
-                                    vp, C.c_size_t, vp]
+    lib.aecf_fusion_bwd.argtypes = [C.POINTER(PoolDesc), C.POINTER(FusionTensors), C.POINTER(FusionGrads), vp, C.c_size_t, vp]
     lib.aecf_fusion_workspace_bytes.restype = C.c_size_t
     lib.aecf_fusion_workspace_bytes.argtypes = [C.POINTER(PoolDesc)]
     lib.aecf_peer_flag_bytes.restype = C.c_size_t

@@ -58,7 +58,6 @@ struct Workspace {
     float* d_qp;       // [D]
     float* d_bias_kv;  // [2D]
     float* d_bq;       // [D] (per-row query)
-    float* fold_g;     // [D + HSP, D] fp32: [dWv ; R] of the folded backward
     // folded backward with the fused gradient tail (grad_tail.cu): the two weight-gradient products leave their split-K
     // partials side by side, then the raw sums and the tail's scratch
     char* gemm_o; size_t gemm_o_bytes;
@@ -123,8 +122,6 @@ static int carve(const aecf_pool_desc* d, const Geometry& g, void* base, Workspa
     w->d_qp = reinterpret_cast<float*>(b + off); off += align256(sizeof(float) * g.D);
     w->d_bias_kv = reinterpret_cast<float*>(b + off); off += align256(sizeof(float) * 2 * g.D);
     w->d_bq = reinterpret_cast<float*>(b + off); off += align256(sizeof(float) * g.D);
-    w->fold_g = reinterpret_cast<float*>(b + off);
-    if (g.fold) off += align256(sizeof(float) * (g.D + g.HSP) * g.D);
     w->gemm_o = w->gemm_g = w->tail = nullptr; w->sums = nullptr; w->rowsum = nullptr;
     w->gemm_o_bytes = w->gemm_g_bytes = w->tail_bytes = w->rowsum_bytes = 0;
     if (g.fold) {
@@ -145,7 +142,7 @@ static int carve(const aecf_pool_desc* d, const Geometry& g, void* base, Workspa
     return AECF_OK;
 }
 
-// ---- the folded backward, whole (phase AECF_BWD_ALL): five launches on `s`, the gradient tail next to them ----
+// ---- the folded backward: five launches on `s`, the gradient tail next to them ----
 //   s    : dWo partials -> d_ctx -> pool backward -(fork)-> [dWv ; R] partials -(fork 2)-> dX -(join)->
 //   side :                                          colsum(d_out), dWo fold,  [dWv ; R] fold, partial folds -> [peer sum] -> finish
 //                                                   bias sums over d_ctx
@@ -333,11 +330,11 @@ int aecf_fusion_fwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, vo
     return AECF_OK;
 }
 
-int aecf_fusion_bwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, const aecf_fusion_grads* gr, int32_t phase,
-                    void* workspace, size_t workspace_bytes, void* stream) {
+int aecf_fusion_bwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, const aecf_fusion_grads* gr, void* workspace,
+                    size_t workspace_bytes, void* stream) {
     Geometry g;
     AECF_TRY(geometry(desc, &g));
-    if (!t || !gr || !workspace || phase < AECF_BWD_ALL || phase > AECF_BWD_REST) return AECF_ERR_INVALID;
+    if (!t || !gr || !workspace) return AECF_ERR_INVALID;
     if (!t->query || !t->key || !t->in_proj_weight || !t->out_proj_weight || !t->q_proj || !t->kv || !t->ctx ||
         !gr->d_out || !gr->d_ctx || !gr->d_kv)
         return AECF_ERR_INVALID;
@@ -350,55 +347,25 @@ int aecf_fusion_bwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, co
     const long long DD = static_cast<long long>(D) * D;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
 
-    if (g.fold && phase == AECF_BWD_ALL) {
+    if (g.fold) {
         if (t->value || !t->scores || !t->folded_w) return AECF_ERR_INVALID;
         return folded_backward(desc, g, t, gr, w, s);
     }
-    if (phase != AECF_BWD_REST) {
-        // ---- out-projection backward: its two parameter gradients are final first -------------------
-        if (gr->d_out_proj_bias) {
-            ScopedSite site(AECF_SITE_D_OUT_BIAS);
-            AECF_TRY(aecf_colsum(dev, dt, dt, gr->d_out, g.QR, D, D, gr->d_out_proj_bias, w.colsum, w.colsum_bytes, stream));
-        }
-        if (gr->d_out_proj_weight) {                         // dWo = g^T ctx
-            ScopedSite site(AECF_SITE_D_OUT_WEIGHT);
-            const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.QR, D, D, D);
-            AECF_TRY(aecf_gemm(&d, gr->d_out, t->ctx, nullptr, gr->d_out_proj_weight, w.gemm, w.gemm_bytes, stream));
-        }
-        {                                                    // d_ctx = g Wo
-            ScopedSite site(AECF_SITE_D_CTX);
-            const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_K_MAJOR, AECF_MN_MAJOR, g.QR, D, D, D, D, D);
-            AECF_TRY(aecf_gemm(&d, gr->d_out, t->out_proj_weight, nullptr, gr->d_ctx, w.gemm, w.gemm_bytes, stream));
-        }
-        if (phase == AECF_BWD_OUT_PROJ) return AECF_OK;
+    // ---- out-projection backward ----------------------------------------------------------------------
+    if (gr->d_out_proj_bias) {
+        ScopedSite site(AECF_SITE_D_OUT_BIAS);
+        AECF_TRY(aecf_colsum(dev, dt, dt, gr->d_out, g.QR, D, D, gr->d_out_proj_bias, w.colsum, w.colsum_bytes, stream));
     }
-
-    if (g.fold) {
-        if (t->value || !t->scores || !t->folded_w) return AECF_ERR_INVALID;
-        const int KF = D + g.HSP;                            // contraction / row width of d_vs = [dV | ds]
-        if (desc->row_index != nullptr)
-            AECF_CUDA_OK(cudaMemsetAsync(gr->d_kv, 0, static_cast<size_t>(g.rows) * KF * es, s));
-        {
-            ScopedSite site(AECF_SITE_POOL_BWD);
-            AECF_TRY(aecf_pool_bwd_folded(desc, t->q_proj, t->scores, t->kv, t->score_bias, gr->d_ctx, gr->d_pooled,
-                                          gr->d_entropy, gr->d_kv, w.d_bias_kv, w.pool, w.pool_bytes, stream));
-        }
-        if (gr->d_key) {                                     // dX = [dV | ds] . [Wv ; Qk]
-            ScopedSite site(AECF_SITE_D_X);
-            const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_K_MAJOR, AECF_MN_MAJOR, g.rows, D, KF, KF, D, D);
-            AECF_TRY(aecf_gemm(&d, gr->d_kv, t->folded_w, nullptr, gr->d_key, w.gemm, w.gemm_bytes, stream));
-        }
-        if (gr->d_in_proj_weight || gr->d_query || gr->d_in_proj_bias) {
-            {                                                // [dWv ; R] = [dV | ds]^T . X   (fp32)
-                ScopedSite site(AECF_SITE_D_KV_WEIGHT);
-                const aecf_gemm_desc d = gemm_desc(dev, dt, dt, AECF_F32, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, KF, D, g.rows, KF, D, D);
-                AECF_TRY(aecf_gemm(&d, gr->d_kv, t->key, nullptr, w.fold_g, w.gemm, w.gemm_bytes, stream));
-            }
-            ScopedSite site(AECF_SITE_FOLD_FINISH);          // dWv, dWk = scale q (x) R, d_qp = scale Wk . R
-            AECF_TRY(aecf_fold_finish(dev, dt, D, g.H, w.fold_g, static_cast<const float*>(t->q_proj), t->in_proj_weight,
-                                      gr->d_in_proj_weight, w.d_qp, stream));
-        }
-    } else {
+    if (gr->d_out_proj_weight) {                             // dWo = g^T ctx
+        ScopedSite site(AECF_SITE_D_OUT_WEIGHT);
+        const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.QR, D, D, D);
+        AECF_TRY(aecf_gemm(&d, gr->d_out, t->ctx, nullptr, gr->d_out_proj_weight, w.gemm, w.gemm_bytes, stream));
+    }
+    {                                                        // d_ctx = g Wo
+        ScopedSite site(AECF_SITE_D_CTX);
+        const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_K_MAJOR, AECF_MN_MAJOR, g.QR, D, D, D, D, D);
+        AECF_TRY(aecf_gemm(&d, gr->d_out, t->out_proj_weight, nullptr, gr->d_ctx, w.gemm, w.gemm_bytes, stream));
+    }
     if (desc->row_index != nullptr)
         AECF_CUDA_OK(cudaMemsetAsync(gr->d_kv, 0, static_cast<size_t>(g.rows) * 2 * D * es, s));
     {   // ---- fused recompute backward of the pool ---------------------------------------------------
@@ -436,7 +403,6 @@ int aecf_fusion_bwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, co
                                    w.gemm_bytes, stream));
             }
         }
-    }
     }
     if (g.shared) {
         // ---- query side, shared query: dWq = d_qp (x) q0, d_query = d_qp . Wq, [d_bq | d_bk | d_bv] -- one launch

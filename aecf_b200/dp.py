@@ -16,8 +16,7 @@ fusion parameter gradients per step (1 051 136 parameters at D = 512).
   * ``collective="nccl"`` / ``"peer"``: the backward writes its parameter gradients into one flat bucket (no copies) and
     ``finish()`` reduces it with ONE all-reduce after the backward -- ``torch.distributed`` (NCCL on the GPUs, gloo in the
     CPU tests of the host logic) or ``PeerAllReduce`` (csrc/peer_allreduce.cu).  This is also what runs wherever the
-    fused tail does not apply (unfolded key projection, per-row queries).  ``overlap=True`` (AECF_DP_OVERLAP=1) reduces in
-    two groups in readiness order instead; it measured slower in round 1 (the NCCL kernel displaces persistent CTAs).
+    fused tail does not apply (unfolded key projection, per-row queries).
 """
 from __future__ import annotations
 
@@ -28,7 +27,6 @@ import torch
 import torch.distributed as dist
 
 PARAM_ORDER = ("out_proj.bias", "out_proj.weight", "in_proj_weight", "in_proj_bias", "query")
-EARLY = ("out_proj.bias", "out_proj.weight")            # final after the first backward phase
 
 
 def shard_rows(global_batch: int, rank: int, world_size: int) -> Tuple[int, int]:
@@ -211,21 +209,17 @@ class GradientSync:
     """
 
     def __init__(self, pool, query: Optional[torch.nn.Parameter] = None, process_group=None,
-                 average: bool = True, overlap: Optional[bool] = None, collective: Optional[str] = None):
+                 average: bool = True, collective: Optional[str] = None):
         self.pool, self.query, self.group, self.average = pool, query, process_group, average
         att = pool.attention
         device, dtype = att.in_proj_weight.device, att.in_proj_weight.dtype
         self.cuda = device.type == "cuda"
         if collective is None:
-            collective = os.environ.get("AECF_DP_COLLECTIVE") or ("peer" if os.environ.get("AECF_DP_PEER", "0") == "1" else None)
-        if collective is None:
-            collective = "fused" if self.cuda else "nccl"
+            collective = os.environ.get("AECF_DP_COLLECTIVE") or ("fused" if self.cuda else "nccl")
         if collective not in ("fused", "nccl", "peer"):
             raise ValueError(f"collective must be 'fused', 'nccl' or 'peer', got {collective!r}")
         self.collective = collective
-        if overlap is None:
-            overlap = os.environ.get("AECF_DP_OVERLAP", "0") == "1"
-        self.overlap = overlap
+        self.overlap = False                             # read by bench.py: the bucket is always reduced in one piece
         self.params: Dict[str, torch.nn.Parameter] = {}
         for name, p in (("out_proj.bias", att.out_proj.bias), ("out_proj.weight", att.out_proj.weight),
                         ("in_proj_weight", att.in_proj_weight), ("in_proj_bias", att.in_proj_bias), ("query", query)):
@@ -240,15 +234,9 @@ class GradientSync:
                 k = self.params[name].numel()
                 self.slices[name] = slice(n, n + k)
                 n += (k + 7) // 8 * 8                       # keep every slice 16-byte aligned
-            if name == EARLY[-1]:
-                self.early_end = n
         self.bucket = torch.zeros(n, dtype=dtype, device=device)
         self.views = {name: self.bucket[sl].view(self.params[name].shape) for name, sl in self.slices.items()}
-        self.comm_stream = torch.cuda.Stream(device=device) if self.cuda else None
-        self.pending: List[object] = []
         self.reported: set = set()
-        self.accumulated: set = set()                    # reported, but autograd adds them into the bucket after the backward
-        self.reduced_upto = 0
         self.bucket_is_reduced = False                   # the bucket holds a cross-rank result (a finished step)
         self.enabled = True                              # False: gradients stay local (gradient accumulation, measurements)
         self.peer = None
@@ -261,12 +249,10 @@ class GradientSync:
                 self.fused = None                        # no fused tail for this pool: bucket + NCCL
         if self.cuda and multi and collective == "peer":
             self.peer = PeerAllReduce(self.bucket, process_group, average)     # one kernel for the whole bucket
-            self.overlap = False
 
     # -- wiring -----------------------------------------------------------------------------
     def attach(self) -> "GradientSync":
         self.pool._grad_ready = self.on_ready
-        self.pool._grad_ready_early = bool(self.overlap)
         self.pool._grad_buffers = _BucketViews(self)     # the fused backward writes its gradients here
         self.pool._dp = self.fused
         if self.query is not None:
@@ -307,23 +293,6 @@ class GradientSync:
         self.pool.row_offset = row0
         return row0, rows
 
-    def _reduce(self, lo: int, hi: int, side_stream: bool) -> None:
-        if hi <= lo:
-            return
-        view = self.bucket[lo:hi]
-        avg = self.average and dist.get_backend(self.group) == "nccl"
-        op = dist.ReduceOp.AVG if avg else dist.ReduceOp.SUM
-        if self.cuda and side_stream:
-            ready = torch.cuda.Event()
-            ready.record(torch.cuda.current_stream(self.bucket.device))
-            with torch.cuda.stream(self.comm_stream):
-                self.comm_stream.wait_event(ready)
-                self.pending.append(dist.all_reduce(view, op=op, group=self.group, async_op=True))
-        else:
-            self.pending.append(dist.all_reduce(view, op=op, group=self.group, async_op=True))
-        if self.average and not avg:
-            self._scale_later = True
-
     # -- called from the backward (autograd worker thread) -----------------------------------
     def on_ready(self, name: str, grad: torch.Tensor) -> None:
         if name not in self.slices or self.world_size == 1:
@@ -346,14 +315,9 @@ class GradientSync:
                 self._reduce_now(grad)
                 return
             # ... onto local, unreduced gradients (enabled=False micro-batches): the bucket is reduced whole in finish()
-            self.accumulated.add(name)
         elif grad.data_ptr() != view.data_ptr():                       # produced elsewhere: copy into the bucket
             view.copy_(grad.reshape(view.shape))
         self.reported.add(name)
-        if (self.overlap and not self.accumulated and self.reduced_upto == 0
-                and all(n in self.reported for n in EARLY if n in self.slices)):
-            self._reduce(0, self.early_end, side_stream=False if self.accumulated else True)
-            self.reduced_upto = self.early_end
 
     def _reduce_now(self, tensor: torch.Tensor) -> None:
         avg = self.average and dist.get_backend(self.group) == "nccl"
@@ -363,28 +327,18 @@ class GradientSync:
 
     # -- called by the training loop after loss.backward() -----------------------------------
     def finish(self) -> None:
-        """Reduce what is left, wait for the collectives and store the results in ``param.grad``."""
+        """Reduce the bucket (one all-reduce) and point every reported ``param.grad`` at its slice."""
         if self._fused_ran():
             self.fused.ran = False                       # the backward summed over the ranks itself: .grad is final
-            self.reported.clear(); self.accumulated.clear()
+            self.reported.clear()
             return
         if not self.reported:
             return
         if self.peer is not None:
             self.peer()                                  # in place, on the compute stream, complete when it returns on-stream
         else:
-            self._reduce(self.reduced_upto, self.bucket.numel(), side_stream=False)
-            for work in self.pending:
-                work.wait()
-            if self.cuda and self.overlap:
-                torch.cuda.current_stream(self.bucket.device).wait_stream(self.comm_stream)
-            if getattr(self, "_scale_later", False):
-                self.bucket.mul_(1.0 / self.world_size)
-                self._scale_later = False
+            self._reduce_now(self.bucket)
         for name in self.reported:
             self.params[name].grad = self.views[name]
         self.bucket_is_reduced = True
-        self.pending.clear()
         self.reported.clear()
-        self.accumulated.clear()
-        self.reduced_upto = 0

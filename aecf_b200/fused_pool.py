@@ -39,10 +39,8 @@ class PoolConfig:
     want_mask_bits: bool = False
     bias_strides: tuple = (0, 0)        # (batch, head[, query]) element strides of the additive score bias
     tgt_len: int = 1            # fusion queries per sample; > 1: per-row queries [B, S, D] / [S, B, D], rows (b, s)
-    # data-parallel hook: called in backward with (name, grad tensor) as soon as a parameter
-    # gradient is final, so that its all-reduce overlaps the rest of the backward
+    # data-parallel hook: called in backward with (name, grad tensor) for each parameter gradient it produced
     grad_ready: Optional[Callable[[str, torch.Tensor], None]] = None
-    grad_ready_early: bool = False      # True: two-phase backward, the out-projection gradients are reported before the rest
     # data-parallel: {parameter name: tensor} the backward writes that parameter's gradient into
     # (slices of the all-reduce bucket), instead of allocating it
     grad_buffers: Optional[dict] = None
@@ -86,8 +84,7 @@ def _rows(x3d: torch.Tensor) -> torch.Tensor:
 class FusedPoolFunction(torch.autograd.Function):
     """out, pooled, entropy, mask_rate, masked, mask_bits = f(query, key, value, params...).
 
-    One C-ABI call for the forward (``aecf_fusion_fwd``), one or two for the backward
-    (``aecf_fusion_bwd``; two phases when a data-parallel hook wants the out-projection gradients early).
+    One C-ABI call for the forward (``aecf_fusion_fwd``), one for the backward (``aecf_fusion_bwd``).
     """
 
     @staticmethod
@@ -193,7 +190,7 @@ class FusedPoolFunction(torch.autograd.Function):
         d_q_rows = None if cfg.q_shared else new((R, D))
         d_key = new(key.shape) if need_key else None
         d_value = new(value.shape) if (value is not None and need_value) else None
-        # fused tail: the folded backward as one call (phase ALL); with cfg.dp the cross-rank sum happens inside it and the
+        # fused tail: the folded backward as one call; with cfg.dp the cross-rank sum happens inside it and the
         # gradients come back final, so they go to fresh tensors autograd owns, not into the all-reduce bucket
         fused_dp = cfg.dp if (cfg.fold and cfg.dp is not None and cfg.dp.usable(ctx.desc)) else None
         bufs = {} if fused_dp is not None else (cfg.grad_buffers or {})
@@ -229,26 +226,12 @@ class FusedPoolFunction(torch.autograd.Function):
             grads.dp = fused_dp.pointer()
             fused_dp.ran = True
         ws = ops.fusion_workspace(ctx.desc, dev)
-        if notify is None or not cfg.grad_ready_early:
-            ops.fusion_bwd(ctx.desc, tensors, grads, _lib.BWD_ALL, ws, dev)
-            if notify is not None:                      # one bucket all-reduce after the backward (GradientSync.finish)
-                for name, t in (("out_proj.bias", d_out_b), ("out_proj.weight", d_out_w), ("in_proj_weight", d_in_w),
-                                ("in_proj_bias", d_in_b)):
-                    if t is not None:
-                        notify(name, t)
-        else:
-            # the out-projection gradients are final first: hand them to the all-reduce while the pool
-            # backward and the in-projection GEMMs run (two-phase call: the sequence without the fused tail)
-            ops.fusion_bwd(ctx.desc, tensors, grads, _lib.BWD_OUT_PROJ, ws, dev)
-            if d_out_b is not None:
-                notify("out_proj.bias", d_out_b)
-            if d_out_w is not None:
-                notify("out_proj.weight", d_out_w)
-            ops.fusion_bwd(ctx.desc, tensors, grads, _lib.BWD_REST, ws, dev)
-            if d_in_w is not None:
-                notify("in_proj_weight", d_in_w)
-            if d_in_b is not None:
-                notify("in_proj_bias", d_in_b)
+        ops.fusion_bwd(ctx.desc, tensors, grads, ws, dev)
+        if notify is not None:                          # one bucket all-reduce after the backward (GradientSync.finish)
+            for name, t in (("out_proj.bias", d_out_b), ("out_proj.weight", d_out_w), ("in_proj_weight", d_in_w),
+                            ("in_proj_bias", d_in_b)):
+                if t is not None:
+                    notify(name, t)
         if d_q is not None:
             d_q = d_q.reshape(ctx.q_shape)
         return d_q, d_key, d_value, d_in_w, d_in_b, d_out_w, d_out_b, None, None

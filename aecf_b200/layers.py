@@ -260,7 +260,6 @@ class MultimodalAttentionPool(nn.Module):
         self.row_offset = 0
         self._grad_ready = None
         self._grad_buffers = None
-        self._grad_ready_early = False                # data parallelism: report the out-projection gradients early
         self._dp = None                               # data parallelism: aecf_b200.dp.FusedGradSum
         self._side = None                             # SideStream of the backward's gradient tail, made on first use
         self._want_mask_bits = False
@@ -424,7 +423,6 @@ class MultimodalAttentionPool(nn.Module):
             seed=seed, offset=offset, rng_state=rng_state, row0=int(self.row_offset), q_shared=q_shared,
             seq_first=not self.batch_first, fold=fold, want_mask_bits=self._want_mask_bits, bias_strides=bias_strides,
             tgt_len=tgt_len, grad_ready=self._grad_ready, grad_buffers=self._grad_buffers,
-            grad_ready_early=bool(self._grad_ready_early),
             loss_target=cm._loss_target() if (masking == 1 and return_info and os.environ.get("AECF_FUSED_LOSS", "1") != "0") else None,
             side=self._side_stream(key.device) if fold else None, dp=self._dp, sample_index=index)
         info_rows = batch if index is None else int(index.numel())

@@ -344,8 +344,7 @@ def fusion_fwd(desc: _lib.PoolDesc, tensors: _lib.FusionTensors, dev: torch.devi
     _lib.check(rc, f"aecf_fusion_fwd B={desc.batch} M={desc.num_tokens} D={desc.embed_dim} H={desc.num_heads}")
 
 
-def fusion_bwd(desc: _lib.PoolDesc, tensors: _lib.FusionTensors, grads: _lib.FusionGrads, phase: int,
-               ws: torch.Tensor, dev: torch.device) -> None:
-    rc = _lib.load().aecf_fusion_bwd(C.byref(desc), C.byref(tensors), C.byref(grads), phase, ws.data_ptr(), ws.numel(),
-                                     _stream(dev))
-    _lib.check(rc, f"aecf_fusion_bwd phase={phase} B={desc.batch} M={desc.num_tokens} D={desc.embed_dim}")
+def fusion_bwd(desc: _lib.PoolDesc, tensors: _lib.FusionTensors, grads: _lib.FusionGrads, ws: torch.Tensor,
+               dev: torch.device) -> None:
+    rc = _lib.load().aecf_fusion_bwd(C.byref(desc), C.byref(tensors), C.byref(grads), ws.data_ptr(), ws.numel(), _stream(dev))
+    _lib.check(rc, f"aecf_fusion_bwd B={desc.batch} M={desc.num_tokens} D={desc.embed_dim}")

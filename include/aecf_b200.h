@@ -45,7 +45,7 @@ extern "C" {
 #define AECF_API
 #endif
 
-#define AECF_ABI_VERSION 4
+#define AECF_ABI_VERSION 5
 #define AECF_MAX_TOKENS 8
 
 typedef enum aecf_status {
@@ -351,7 +351,7 @@ typedef struct aecf_fusion_grads {
     void* d_in_proj_bias;          /* [3D] */
     void* d_out_proj_weight;       /* [D, D] */
     void* d_out_proj_bias;         /* [D] */
-    /* Folded backward, phase AECF_BWD_ALL: the small kernels that finish the parameter gradients (split-K folds, column
+    /* Folded backward: the small kernels that finish the parameter gradients (split-K folds, column
      * sums, the rank-H key/query terms, conversion to dtype; csrc/grad_tail.cu) run on `side_stream` NEXT TO the products on
      * `stream`: fork_event is recorded on `stream` after the pool backward (the column sums of d_out and the dWo fold then run
      * next to the [dWv ; R] product), fork_event2 after that product (the rest runs next to dX), join_event on `side_stream` after the last of them, and
@@ -364,14 +364,10 @@ typedef struct aecf_fusion_grads {
     const aecf_dp_desc* dp;        /* nullable: sum the gradients over the ranks inside the backward (see aecf_dp_desc) */
 } aecf_fusion_grads;
 
-enum { AECF_BWD_ALL = 0, AECF_BWD_OUT_PROJ = 1, AECF_BWD_REST = 2 };
-
 AECF_API int aecf_fusion_fwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, void* workspace,
                              size_t workspace_bytes, void* stream);
-/* phase AECF_BWD_OUT_PROJ computes d_out_proj_{bias,weight} and d_ctx; AECF_BWD_REST everything else
- * (a data-parallel caller starts the all-reduce of the out-projection gradients in between). */
 AECF_API int aecf_fusion_bwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, const aecf_fusion_grads* g,
-                             int32_t phase, void* workspace, size_t workspace_bytes, void* stream);
+                             void* workspace, size_t workspace_bytes, void* stream);
 AECF_API size_t aecf_fusion_workspace_bytes(const aecf_pool_desc* desc);
 /* bytes of ONE raw-sum (or reduced-sum) buffer of aecf_dp_desc for this descriptor; 0 where the backward has no fused tail
  * (unfolded key projection, per-row queries) */

@@ -15,9 +15,9 @@ run() {   # tag, env assignments, bench arguments
   echo "$tag exit $?" >> gpurun_out/r2_n${N}_$tag.err
   echo "== $tag"; python scripts/show_bench.py gpurun_out/r2_n${N}_$tag.json 2>/dev/null | head -3; tail -2 gpurun_out/r2_n${N}_$tag.err | cut -c1-300
 }
-run weak_nccl  "AECF_DP_PEER=0"
-run weak_peer  "AECF_DP_PEER=1"
-run strong_nccl "AECF_DP_PEER=0" --global-batch 65536
-run strong_peer "AECF_DP_PEER=1" --global-batch 65536
+run weak_nccl  "AECF_DP_COLLECTIVE=nccl"
+run weak_peer  "AECF_DP_COLLECTIVE=peer"
+run strong_nccl "AECF_DP_COLLECTIVE=nccl" --global-batch 65536
+run strong_peer "AECF_DP_COLLECTIVE=peer" --global-batch 65536
 timeout 200 python bench.py --gpus 1 --steps 20 --warmup 5 --no-cpu-baseline --no-e2e > gpurun_out/r2_n${N}_same_box_n1.json 2> gpurun_out/r2_n${N}_same_box_n1.err
 echo "== n1 on the same box"; python scripts/show_bench.py gpurun_out/r2_n${N}_same_box_n1.json 2>/dev/null | head -2

@@ -21,7 +21,7 @@ def test_library_loads_and_exports_every_declared_symbol():
     lib = _lib.load()
     for name in declared:
         assert hasattr(lib, name), name
-    assert lib.aecf_abi_version() == _lib.ABI_VERSION == 4
+    assert lib.aecf_abi_version() == _lib.ABI_VERSION == 5
     assert b"sm_100a" in lib.aecf_build_info()
     assert lib.aecf_strerror(-2).decode().startswith("shape or dtype outside")
 
@@ -252,7 +252,7 @@ def test_multi_query_host_plumbing(monkeypatch, batch_first):
     monkeypatch.setattr(torch.cuda, "is_current_stream_capturing", lambda: False)
     monkeypatch.setattr(ops, "fusion_workspace", lambda desc, dev: torch.empty(1))
     monkeypatch.setattr(ops, "fusion_fwd", lambda desc, tensors, dev: calls.setdefault("fwd", (desc, tensors)))
-    monkeypatch.setattr(ops, "fusion_bwd", lambda desc, tensors, grads, phase, ws, dev: calls.setdefault("bwd", (desc, grads, phase)))
+    monkeypatch.setattr(ops, "fusion_bwd", lambda desc, tensors, grads, ws, dev: calls.setdefault("bwd", []).append((desc, grads)))
     pool = aecf.MultimodalAttentionPool(D, num_heads=H, curriculum_masking=aecf.CurriculumMasking(), batch_first=batch_first)
     q = torch.randn(B, S, D, requires_grad=True) if batch_first else torch.randn(S, B, D, requires_grad=True)
     k = torch.randn(B, M, D, requires_grad=True) if batch_first else torch.randn(M, B, D, requires_grad=True)
@@ -268,8 +268,9 @@ def test_multi_query_host_plumbing(monkeypatch, batch_first):
     assert info["attention_weights"].shape == (B, S, M) and info["masked_attention_weights"].shape == (B, S, M)
     assert info["entropy"].shape == info["mask_rate"].shape == info["target_entropy"].shape == (B, S)
     (out.sum() + info["attention_weights"].sum()).backward()
-    desc_b, grads, phase = calls["bwd"]
-    assert desc_b is desc and phase == _lib.BWD_ALL and grads.d_q_rows and grads.d_pooled and grads.d_query
+    assert len(calls["bwd"]) == 1                        # the whole backward in one call
+    desc_b, grads = calls["bwd"][0]
+    assert desc_b is desc and grads.d_q_rows and grads.d_pooled and grads.d_query
     assert q.grad.shape == q.shape and k.grad.shape == k.shape
     assert pool.attention.in_proj_weight.grad.shape == (3 * D, D)
     with pytest.raises(RuntimeError, match=r"2D attn_mask is \(1, 4\), but should be \(3, 4\)"):

@@ -2,7 +2,7 @@
 
 The compute inside each rank is the CPU oracle (the CUDA path needs a GPU); what is tested here is
 what ``aecf_b200/dp.py`` adds -- row sharding, Philox offsets keyed on the global row, the flat fp32
-gradient bucket and its overlapped all-reduce -- i.e. that an N-rank run reproduces the 1-rank run.
+gradient bucket and its one all-reduce -- i.e. that an N-rank run reproduces the 1-rank run.
 """
 import os
 import socket
@@ -65,19 +65,19 @@ class _Params(torch.nn.Module):
         self._grad_buffers = None
 
 
-def _worker(rank, port, out_dir, overlap):
+def _worker(rank, port, out_dir):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=WORLD)
     try:
         t = _inputs()
         pool = _Params(t)
         query = torch.nn.Parameter(t["q0"].clone())
-        sync = GradientSync(pool, query, average=False, overlap=overlap).attach()
+        sync = GradientSync(pool, query, average=False).attach()
         row0, rows = sync.set_shard(B)
         assert pool.row_offset == row0 and pool._grad_ready is not None and set(pool._grad_buffers) == set(PARAM_ORDER)
         fwd, grads = _step(t, row0, rows)
         # report in the order the fused backward produces them: out_proj first, in_proj and query last
-        for i, name in enumerate(PARAM_ORDER):
+        for name in PARAM_ORDER:
             if name == "query":
                 sync._query_hook(grads[name])
             elif name == "in_proj_weight":                # what the fused backward does: write in place
@@ -85,11 +85,11 @@ def _worker(rank, port, out_dir, overlap):
                 pool._grad_ready(name, pool._grad_buffers[name])
             else:                                         # a gradient produced elsewhere is copied in
                 pool._grad_ready(name, grads[name])
-            # overlap=True: the out-projection group is reduced as soon as both of its members are in;
-            # the default (overlap=False) reduces the whole bucket once, in finish()
-            assert len(sync.pending) == ((1 if i >= 1 else 0) if overlap else 0)
+            # nothing is reduced yet: the whole bucket is reduced once, in finish()
+            assert not sync.bucket_is_reduced and name in sync.reported
+            assert torch.equal(sync.views[name], grads[name].reshape(sync.views[name].shape))
         sync.finish()
-        assert not sync.pending and not sync.reported
+        assert sync.bucket_is_reduced and not sync.reported
         assert pool.attention.in_proj_weight.grad.data_ptr() == pool._grad_buffers["in_proj_weight"].data_ptr()
         np.savez(os.path.join(out_dir, f"rank{rank}.npz"), row0=row0, rows=rows,
                  mask=fwd.info["mask"].numpy(), out=fwd.out.numpy(),
@@ -98,10 +98,9 @@ def _worker(rank, port, out_dir, overlap):
         dist.destroy_process_group()
 
 
-@pytest.mark.parametrize("overlap", [False, True], ids=["one_all_reduce", "overlapped_groups"])
-def test_two_ranks_reproduce_one_rank(tmp_path, overlap):
+def test_two_ranks_reproduce_one_rank(tmp_path):
     port = _free_port()
-    mp.spawn(_worker, args=(port, str(tmp_path), overlap), nprocs=WORLD, join=True)
+    mp.spawn(_worker, args=(port, str(tmp_path)), nprocs=WORLD, join=True)
     t = _inputs()
     full_fwd, full_grads = _step(t, 0, B)
     shards = [np.load(tmp_path / f"rank{r}.npz") for r in range(WORLD)]
@@ -137,7 +136,7 @@ def test_single_process_sync_leaves_gradients_alone():
     pool.attention.out_proj.weight.grad = g.clone()
     pool._grad_ready("out_proj.weight", g * 3)          # ignored: there is nobody to reduce with
     sync.finish()
-    assert torch.equal(pool.attention.out_proj.weight.grad, g) and not sync.pending
+    assert torch.equal(pool.attention.out_proj.weight.grad, g) and not sync.reported
 
 
 # ---- gradient accumulation (ADVICE r1, high): param.grad lives in the bucket after finish() ------------------------------

@@ -25,7 +25,7 @@ def _free_port() -> int:
         return s.getsockname()[1]
 
 
-def _step(dtype, fold, rank, world, sync_kwargs=None):
+def _step(dtype, fold, rank, world):
     """One training step of this rank's shard of CASE through the module API; returns arrays to compare."""
     import aecf_b200
     from aecf_b200.dp import GradientSync
@@ -41,7 +41,7 @@ def _step(dtype, fold, rank, world, sync_kwargs=None):
     pool.fold_key_projection = fold
     pool._want_mask_bits = True
     query = torch.nn.Parameter(inp["query0"].to(dtype).clone())
-    sync = GradientSync(pool, query, average=False, **(sync_kwargs or {})).attach()
+    sync = GradientSync(pool, query, average=False).attach()
     row0, rows = sync.set_shard(CASE.B)
     sl = slice(row0, row0 + rows)
     x = inp["x"][sl].to(dtype).clone().requires_grad_(True)
@@ -61,23 +61,22 @@ def _step(dtype, fold, rank, world, sync_kwargs=None):
     return got
 
 
-def _worker(rank, port, out_dir, dtype, fold, overlap):
+def _worker(rank, port, out_dir, dtype, fold):
     from tests.emu_support import enable_in_this_process
     enable_in_this_process()
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=WORLD)
     try:
-        np.savez(os.path.join(out_dir, f"rank{rank}.npz"), **_step(dtype, fold, rank, WORLD, {"overlap": overlap}))
+        np.savez(os.path.join(out_dir, f"rank{rank}.npz"), **_step(dtype, fold, rank, WORLD))
     finally:
         dist.destroy_process_group()
 
 
-@pytest.mark.parametrize("dtype,fold,overlap", [(torch.float32, True, True), (torch.bfloat16, None, False)],
-                         ids=["fp32_folded_overlapped", "bf16_default"])
-def test_two_emulated_ranks_reproduce_one(tmp_path, dtype, fold, overlap):
+@pytest.mark.parametrize("dtype,fold", [(torch.float32, True), (torch.bfloat16, None)], ids=["fp32_folded", "bf16_default"])
+def test_two_emulated_ranks_reproduce_one(tmp_path, dtype, fold):
     from tests.emu_support import enable_in_this_process, load_emulation
     load_emulation()                                     # build once, before the workers race for it
-    mp.spawn(_worker, args=(_free_port(), str(tmp_path), dtype, fold, overlap), nprocs=WORLD, join=True)
+    mp.spawn(_worker, args=(_free_port(), str(tmp_path), dtype, fold), nprocs=WORLD, join=True)
     shards = [np.load(tmp_path / f"rank{r}.npz") for r in range(WORLD)]
     assert sum(int(s["rows"]) for s in shards) == CASE.B and int(shards[1]["row0"]) == int(shards[0]["rows"])
 
