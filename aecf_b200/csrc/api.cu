@@ -4,6 +4,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 
 #include "pool_dispatch.cuh"
 
@@ -174,46 +175,13 @@ static int make_plan(const aecf_pool_desc* d, PoolPlan* plan, bool fold = false)
     return AECF_OK;
 }
 
-// (dtype, dropout, lane map) -> the instantiation set of pool_dispatch.cuh
-template <bool PAD>
-static int launch_fwd(const PoolPlan& plan, const PoolParams& p, int grid, int sms, bool fold, void* stream) {
-    if (plan.bf16)
-        return plan.drop ? launch_pool_fwd<__nv_bfloat16, true, PAD>(plan.M, plan.J, p, grid, sms, fold, stream)
-                         : launch_pool_fwd<__nv_bfloat16, false, PAD>(plan.M, plan.J, p, grid, sms, fold, stream);
-    return plan.drop ? launch_pool_fwd<float, true, PAD>(plan.M, plan.J, p, grid, sms, fold, stream)
-                     : launch_pool_fwd<float, false, PAD>(plan.M, plan.J, p, grid, sms, fold, stream);
-}
-template <bool PAD>
-static int launch_fwd_multi(const PoolPlan& plan, const PoolParams& p, int grid, void* stream) {
-    if (plan.bf16)
-        return plan.drop ? launch_pool_fwd_multi<__nv_bfloat16, true, PAD>(plan.M, plan.J, p, plan.mq, grid, stream)
-                         : launch_pool_fwd_multi<__nv_bfloat16, false, PAD>(plan.M, plan.J, p, plan.mq, grid, stream);
-    return plan.drop ? launch_pool_fwd_multi<float, true, PAD>(plan.M, plan.J, p, plan.mq, grid, stream)
-                     : launch_pool_fwd_multi<float, false, PAD>(plan.M, plan.J, p, plan.mq, grid, stream);
-}
-template <bool PAD>
-static int launch_bwd(const PoolPlan& plan, const PoolParams& p, int grid, bool fold, void* stream) {
-    if (plan.bf16)
-        return plan.drop ? launch_pool_bwd<__nv_bfloat16, true, PAD>(plan.M, plan.J, p, grid, fold, stream)
-                         : launch_pool_bwd<__nv_bfloat16, false, PAD>(plan.M, plan.J, p, grid, fold, stream);
-    return plan.drop ? launch_pool_bwd<float, true, PAD>(plan.M, plan.J, p, grid, fold, stream)
-                     : launch_pool_bwd<float, false, PAD>(plan.M, plan.J, p, grid, fold, stream);
-}
-template <bool PAD>
-static int launch_bwd_multi(const PoolPlan& plan, const PoolParams& p, int grid, void* stream) {
-    if (plan.bf16)
-        return plan.drop ? launch_pool_bwd_multi<__nv_bfloat16, true, PAD>(plan.M, plan.J, p, plan.mq, grid, stream)
-                         : launch_pool_bwd_multi<__nv_bfloat16, false, PAD>(plan.M, plan.J, p, plan.mq, grid, stream);
-    return plan.drop ? launch_pool_bwd_multi<float, true, PAD>(plan.M, plan.J, p, plan.mq, grid, stream)
-                     : launch_pool_bwd_multi<float, false, PAD>(plan.M, plan.J, p, plan.mq, grid, stream);
-}
-template <bool PAD>
-static int bwd_blocks_per_sm(const PoolPlan& plan, bool fold) {
-    if (plan.bf16)
-        return plan.drop ? pool_bwd_blocks_per_sm<__nv_bfloat16, true, PAD>(plan.M, plan.J, fold)
-                         : pool_bwd_blocks_per_sm<__nv_bfloat16, false, PAD>(plan.M, plan.J, fold);
-    return plan.drop ? pool_bwd_blocks_per_sm<float, true, PAD>(plan.M, plan.J, fold)
-                     : pool_bwd_blocks_per_sm<float, false, PAD>(plan.M, plan.J, fold);
+// Calls f(T{}, DROP, PAD) with the plan's element type and the std::bool_constant of its dropout and lane map: the
+// instantiation set of pool_dispatch.cuh that the plan runs.
+template <typename F>
+static int with_pool_types(const PoolPlan& plan, F&& f) {
+    auto pad = [&](auto t, auto drop) { return plan.pad ? f(t, drop, std::true_type{}) : f(t, drop, std::false_type{}); };
+    auto drop = [&](auto t) { return plan.drop ? pad(t, std::true_type{}) : pad(t, std::false_type{}); };
+    return plan.bf16 ? drop(__nv_bfloat16{}) : drop(float{});
 }
 
 }  // namespace aecf
@@ -278,10 +246,14 @@ static int pool_fwd_impl(const aecf_pool_desc* desc, bool fold, const void* q, c
         plan.mq.bias = score_bias;
         p.bias = nullptr;
         const int rows_grid = static_cast<int>((p.B * plan.mq.S + p.SPC - 1) / p.SPC);
-        return plan.pad ? launch_fwd_multi<true>(plan, p, rows_grid, stream) : launch_fwd_multi<false>(plan, p, rows_grid, stream);
+        return with_pool_types(plan, [&](auto t, auto drop, auto pad) {
+            return launch_pool_fwd_multi<decltype(t), drop, pad>(plan.M, plan.J, p, plan.mq, rows_grid, stream);
+        });
     }
     const int grid = static_cast<int>((p.B + p.SPC - 1) / p.SPC);
-    return plan.pad ? launch_fwd<true>(plan, p, grid, sms, fold, stream) : launch_fwd<false>(plan, p, grid, sms, fold, stream);
+    return with_pool_types(plan, [&](auto t, auto drop, auto pad) {
+        return launch_pool_fwd<decltype(t), drop, pad>(plan.M, plan.J, p, grid, sms, fold, stream);
+    });
 }
 
 extern "C" {
@@ -341,9 +313,11 @@ static int pool_bwd_impl(const aecf_pool_desc* desc, bool fold, const void* q, c
     p.partials = no_sums ? nullptr : static_cast<float*>(workspace);
     p.rowsum = no_sums ? rowsum : nullptr;
 
-    int per_sm;
-    if (plan.multi) per_sm = 1;                         // pool_bwd_multi_kernel: __launch_bounds__(256, 1)
-    else per_sm = plan.pad ? bwd_blocks_per_sm<true>(plan, fold) : bwd_blocks_per_sm<false>(plan, fold);
+    int per_sm = 1;                                     // pool_bwd_multi_kernel: __launch_bounds__(256, 1)
+    if (!plan.multi)
+        per_sm = with_pool_types(plan, [&](auto t, auto drop, auto pad) {
+            return pool_bwd_blocks_per_sm<decltype(t), drop, pad>(plan.M, plan.J, fold);
+        });
     if (per_sm <= 0) per_sm = 1;
     long long want = (p.B + p.SPC - 1) / p.SPC;
     long long cap = static_cast<long long>(sm_count(desc->device)) * per_sm;   // persistent: one resident wave
@@ -369,9 +343,11 @@ static int pool_bwd_impl(const aecf_pool_desc* desc, bool fold, const void* q, c
         if (plan.multi) {
             plan.mq.bias = score_bias;
             p.bias = nullptr;
-            rc = plan.pad ? launch_bwd_multi<true>(plan, p, grid, stream) : launch_bwd_multi<false>(plan, p, grid, stream);
-        } else
-            rc = plan.pad ? launch_bwd<true>(plan, p, grid, fold, stream) : launch_bwd<false>(plan, p, grid, fold, stream);
+        }
+        rc = with_pool_types(plan, [&](auto t, auto drop, auto pad) {
+            return plan.multi ? launch_pool_bwd_multi<decltype(t), drop, pad>(plan.M, plan.J, p, plan.mq, grid, stream)
+                              : launch_pool_bwd<decltype(t), drop, pad>(plan.M, plan.J, p, grid, fold, stream);
+        });
     }
     if (rc != AECF_OK) return rc;
     if (no_sums) return AECF_OK;                        // the caller forms the batch sums itself (grad_tail.cu)

@@ -26,6 +26,21 @@ struct BwdSmem {
     static constexpr int bytes(int M) { return (POOL_WARPS * M + POOL_WARPS * PER_WARP) * 4; }
 };
 
+// strip[j][.][lane] += a * x: one of a warp's batch-sum strips ([J][V / 4][32] float4).  The head-mean gradient, the
+// softmax backward and the strip fold are also in pool_bwd_multi_kernel, but stay inline in both: as shared helpers
+// they changed the SASS of 134, 365 and 328 of the 768 backward kernels (scripts/sass_diff.py).
+template <int V>
+__device__ __forceinline__ void strip_fma(float4* strip, int j, int lane, float a, const float (&x)[V]) {
+    constexpr int Q4 = V / 4;
+#pragma unroll
+    for (int q4 = 0; q4 < Q4; ++q4) {
+        float4 t = strip[(j * Q4 + q4) * 32 + lane];
+        t.x = fmaf(a, x[4 * q4], t.x); t.y = fmaf(a, x[4 * q4 + 1], t.y);
+        t.z = fmaf(a, x[4 * q4 + 2], t.z); t.w = fmaf(a, x[4 * q4 + 3], t.w);
+        strip[(j * Q4 + q4) * 32 + lane] = t;
+    }
+}
+
 // FOLD (folded key projection, DESIGN.md): kv holds the values only, the scores come precomputed, there is no
 // key pass -- the score gradient ds[b, m, h] itself is stored next to dV (d_kv rows are [dV (D) | ds (HSP)]) and
 // the dX / dW GEMMs that follow contract over D + HSP, which applies and accumulates the rank-H key-side terms.
@@ -96,19 +111,7 @@ pool_bwd_kernel(const PoolParams p) {
 
         // upstream gradient of the context and the values, issued first
         uint4 dcraw[J];
-        {
-            const char* dc = static_cast<const char*>(p.d_ctx) + static_cast<size_t>(src) * p.D * sizeof(T)
-                             + Core::lane_bytes(p, c0);
-            // (the power-of-two map keeps the spelling it was measured with: the same arithmetic through Core::col_bytes
-            // changes the register allocation of some of its instantiations, J = 1 above all -- scripts/sass_diff.py)
-            if constexpr (PAD) {
-#pragma unroll
-                for (int j = 0; j < J; ++j) dcraw[j] = valid(j) ? ldg_stream(dc + Core::col_bytes(p, c0, j)) : make_uint4(0, 0, 0, 0);
-            } else {
-#pragma unroll
-                for (int j = 0; j < J; ++j) dcraw[j] = valid(j) ? ldg_stream(dc + j * 512) : make_uint4(0, 0, 0, 0);
-            }
-        }
+        Core::load_row(p, p.d_ctx, src, c0, dcraw);
         uint4 vraw[PRELOAD_V ? M : 1][PRELOAD_V ? J : 1];
         if (PRELOAD_V) {
 #pragma unroll
@@ -156,15 +159,7 @@ pool_bwd_kernel(const PoolParams p) {
                 sum_wd += wd[m][j];
                 if (row_ok && valid(j)) stg_vec(dkv_row + Core::dkv_rel(p, c0, m, VHALF, j), Vec<T>::pack(dv));
             }
-            if (row_ok && sums) {
-#pragma unroll
-                for (int q4 = 0; q4 < Q4; ++q4) {
-                    float4 a = acc_bv[(j * Q4 + q4) * 32 + lane];
-                    a.x = fmaf(sum_wd, dc[4 * q4], a.x); a.y = fmaf(sum_wd, dc[4 * q4 + 1], a.y);
-                    a.z = fmaf(sum_wd, dc[4 * q4 + 2], a.z); a.w = fmaf(sum_wd, dc[4 * q4 + 3], a.w);
-                    acc_bv[(j * Q4 + q4) * 32 + lane] = a;
-                }
-            }
+            if (row_ok && sums) strip_fma(acc_bv, j, lane, sum_wd, dc);
         }
         Core::head_reduce(p, dwd);
 
@@ -286,13 +281,7 @@ pool_bwd_kernel(const PoolParams p) {
                     if (valid(j))
                         stg_vec(static_cast<char*>(p.d_q) + static_cast<size_t>(row) * p.D * sizeof(T)
                                     + Core::lane_bytes(p, c0) + Core::col_bytes(p, c0, j), Vec<T>::pack(o));
-#pragma unroll
-                    for (int q4 = 0; q4 < Q4; ++q4) {
-                        float4 a = acc_q[(j * Q4 + q4) * 32 + lane];
-                        a.x = fmaf(sum_ds, qs[j][4 * q4], a.x); a.y = fmaf(sum_ds, qs[j][4 * q4 + 1], a.y);
-                        a.z = fmaf(sum_ds, qs[j][4 * q4 + 2], a.z); a.w = fmaf(sum_ds, qs[j][4 * q4 + 3], a.w);
-                        acc_q[(j * Q4 + q4) * 32 + lane] = a;
-                    }
+                    strip_fma(acc_q, j, lane, sum_ds, qs[j]);
                 }
             }
         }

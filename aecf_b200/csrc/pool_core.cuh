@@ -160,6 +160,23 @@ struct PoolCore {
         return (m * p.dkv_sm + half * p.D) * static_cast<long long>(sizeof(T)) + col_bytes(p, c0, j);
     }
 
+    // This lane's chunks of `row` of a [rows][D] buffer (ctx, d_ctx).  The power-of-two map keeps the spelling it was
+    // measured with: the same arithmetic through col_bytes changes the register allocation of some of its instantiations,
+    // J = 1 above all (scripts/sass_diff.py).  The weighted value sums and the ctx stores stay inline in each forward
+    // kernel: as shared helpers they changed the SASS of 525 of the 1056 forward kernels (sums) and of slice and
+    // streaming kernels (stores).
+    static __device__ __forceinline__ void load_row(const PoolParams& p, const void* base, long long row, int c0,
+                                                    uint4 (&raw)[J]) {
+        const char* in = static_cast<const char*>(base) + static_cast<size_t>(row) * p.D * sizeof(T) + lane_bytes(p, c0);
+        if constexpr (PAD) {
+#pragma unroll
+            for (int j = 0; j < J; ++j) raw[j] = valid(p, c0, j) ? ldg_stream(in + col_bytes(p, c0, j)) : make_uint4(0, 0, 0, 0);
+        } else {
+#pragma unroll
+            for (int j = 0; j < J; ++j) raw[j] = valid(p, c0, j) ? ldg_stream(in + j * 512) : make_uint4(0, 0, 0, 0);
+        }
+    }
+
     // projected query chunks, pre-multiplied by scale (torch/nn/functional.py:6632)
     static __device__ __forceinline__ void load_query(const PoolParams& p, long long row, int c0, float (&qs)[J][V]) {
 #pragma unroll

@@ -87,6 +87,20 @@ __device__ __forceinline__ void masking_stage(const PoolParams& p, const RngKey&
     mask_rate = __fsub_rn(1.0f, static_cast<float>(active) / static_cast<float>(M));   // :275
 }
 
+// The info outputs of one row, as masking_stage left them.
+template <int M>
+__device__ __forceinline__ void store_info(const PoolParams& p, long long row, const float (&pw)[M], const float (&mw)[M],
+                                           float entropy, float mask_rate, unsigned bits) {
+#pragma unroll
+    for (int m = 0; m < M; ++m) {
+        p.pooled[static_cast<size_t>(row) * M + m] = pw[m];
+        if (p.masked) p.masked[static_cast<size_t>(row) * M + m] = mw[m];
+    }
+    if (p.entropy) p.entropy[row] = entropy;
+    if (p.mask_rate) p.mask_rate[row] = mask_rate;
+    if (p.mask_bits) p.mask_bits[row] = static_cast<uint8_t>(bits);
+}
+
 // FOLD: folded key projection -- kv holds the values only and the scores come precomputed (pool_core.cuh).
 // PAD: the padded lane map (pool_core.cuh).
 template <typename T, int M, int J, bool DROP, bool FOLD, bool PAD>
@@ -163,7 +177,7 @@ pool_fwd_kernel(const PoolParams p) {
 #pragma unroll
             for (int j = 0; j < J; ++j)
                 if (Core::valid(p, c0, j)) stg_vec(ctx + Core::col_bytes(p, c0, j), Vec<T>::pack(acc[j]));
-        } else {    // the original spelling, which compiles to the measured kernels' code (see pool_bwd.cuh)
+        } else {    // the original spelling (see PoolCore::load_row)
 #pragma unroll
             for (int j = 0; j < J; ++j)
                 if (c0 + 32 * j < p.NC) stg_vec(ctx + j * 512, Vec<T>::pack(acc[j]));
@@ -198,14 +212,7 @@ pool_fwd_kernel(const PoolParams p) {
     float entropy, mask_rate;
     unsigned bits;
     masking_stage<M>(p, rng, my_row, pw, mw, entropy, mask_rate, bits);
-#pragma unroll
-    for (int m = 0; m < M; ++m) {
-        p.pooled[static_cast<size_t>(my_row) * M + m] = pw[m];
-        if (p.masked) p.masked[static_cast<size_t>(my_row) * M + m] = mw[m];
-    }
-    if (p.entropy) p.entropy[my_row] = entropy;
-    if (p.mask_rate) p.mask_rate[my_row] = mask_rate;
-    if (p.mask_bits) p.mask_bits[my_row] = static_cast<uint8_t>(bits);
+    store_info<M>(p, my_row, pw, mw, entropy, mask_rate, bits);
 }
 
 // ---- streaming variant (one warp owns a whole sample, WPS == 1): the headline path ----------------------
@@ -319,7 +326,7 @@ pool_fwd_stream_kernel(const PoolParams p, const long long rows_per_warp) {
 #pragma unroll
             for (int j = 0; j < J; ++j)
                 if (Core::valid(p, c0, j)) stg_vec(ctx + Core::col_bytes(p, c0, j), Vec<T>::pack(acc[j]));
-        } else {    // the original spelling, which compiles to the measured kernels' code (see pool_bwd.cuh)
+        } else {    // the original spelling (see PoolCore::load_row)
 #pragma unroll
             for (int j = 0; j < J; ++j)
                 if (DENSE || c0 + 32 * j < p.NC) stg_vec(ctx + j * 512, Vec<T>::pack(acc[j]));
@@ -340,14 +347,7 @@ pool_fwd_stream_kernel(const PoolParams p, const long long rows_per_warp) {
                 float entropy, mask_rate;
                 unsigned bits;
                 masking_stage<M>(p, rng, my_row, pw, mw, entropy, mask_rate, bits);
-#pragma unroll
-                for (int m = 0; m < M; ++m) {
-                    p.pooled[static_cast<size_t>(my_row) * M + m] = pw[m];
-                    if (p.masked) p.masked[static_cast<size_t>(my_row) * M + m] = mw[m];
-                }
-                if (p.entropy) p.entropy[my_row] = entropy;
-                if (p.mask_rate) p.mask_rate[my_row] = mask_rate;
-                if (p.mask_bits) p.mask_bits[my_row] = static_cast<uint8_t>(bits);
+                store_info<M>(p, my_row, pw, mw, entropy, mask_rate, bits);
                 if (p.loss_out != nullptr) {            // reference aecf/AECFLayer.py:299-311, the per-sample term
                     bool fin;
                     const float d = scrub_entropy(entropy, &fin) - p.loss_target;

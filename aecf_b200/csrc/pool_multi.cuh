@@ -91,7 +91,7 @@ pool_fwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
 #pragma unroll
             for (int j = 0; j < J; ++j)
                 if (Core::valid(p, c0, j)) stg_vec(ctx + Core::col_bytes(p, c0, j), Vec<T>::pack(acc[j]));
-        } else {    // the original spelling, which compiles to the measured kernels' code (see pool_bwd.cuh)
+        } else {    // the original spelling (see PoolCore::load_row)
 #pragma unroll
             for (int j = 0; j < J; ++j)
                 if (c0 + 32 * j < p.NC) stg_vec(ctx + j * 512, Vec<T>::pack(acc[j]));
@@ -118,14 +118,7 @@ pool_fwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
     float entropy, mask_rate;
     unsigned bits;
     masking_stage<M>(p, rng, my_row, pw, mw, entropy, mask_rate, bits);
-#pragma unroll
-    for (int m = 0; m < M; ++m) {
-        p.pooled[static_cast<size_t>(my_row) * M + m] = pw[m];
-        if (p.masked) p.masked[static_cast<size_t>(my_row) * M + m] = mw[m];
-    }
-    if (p.entropy) p.entropy[my_row] = entropy;
-    if (p.mask_rate) p.mask_rate[my_row] = mask_rate;
-    if (p.mask_bits) p.mask_bits[my_row] = static_cast<uint8_t>(bits);
+    store_info<M>(p, my_row, pw, mw, entropy, mask_rate, bits);
 }
 
 // Backward.  Same closed form as pool_bwd_kernel (SURVEY.md Appendix B) per (b, s) row; dK and dV of a sample are
@@ -181,17 +174,7 @@ pool_bwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
             float qs[J][V];
             Core::load_query(p, qrow, c0, qs);
             uint4 dcraw[J];
-            {
-                const char* dc = static_cast<const char*>(p.d_ctx) + static_cast<size_t>(qrow) * p.D * sizeof(T)
-                                 + Core::lane_bytes(p, c0);
-                if constexpr (PAD) {
-#pragma unroll
-                    for (int j = 0; j < J; ++j) dcraw[j] = valid(j) ? ldg_stream(dc + Core::col_bytes(p, c0, j)) : make_uint4(0, 0, 0, 0);
-                } else {    // the original spelling, which compiles to the measured kernels' code (see pool_bwd.cuh)
-#pragma unroll
-                    for (int j = 0; j < J; ++j) dcraw[j] = valid(j) ? ldg_stream(dc + j * 512) : make_uint4(0, 0, 0, 0);
-                }
-            }
+            Core::load_row(p, p.d_ctx, qrow, c0, dcraw);
 
             float sc[M][J], w[M][J], wd[M][J];
             unsigned keep;
@@ -219,15 +202,7 @@ pool_bwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
                     dwd[m][j] = a;
                     sum_wd += wd[m][j];
                 }
-                if (row_ok) {
-#pragma unroll
-                    for (int q4 = 0; q4 < Q4; ++q4) {
-                        float4 a = acc_bv[(j * Q4 + q4) * 32 + lane];
-                        a.x = fmaf(sum_wd, dc[4 * q4], a.x); a.y = fmaf(sum_wd, dc[4 * q4 + 1], a.y);
-                        a.z = fmaf(sum_wd, dc[4 * q4 + 2], a.z); a.w = fmaf(sum_wd, dc[4 * q4 + 3], a.w);
-                        acc_bv[(j * Q4 + q4) * 32 + lane] = a;
-                    }
-                }
+                if (row_ok) strip_fma(acc_bv, j, lane, sum_wd, dc);
             }
             Core::head_reduce(p, dwd);
 
@@ -299,13 +274,7 @@ pool_bwd_multi_kernel(const PoolParams p, const MultiQuery mq) {
                     if (valid(j))
                         stg_vec(static_cast<char*>(p.d_q) + static_cast<size_t>(qrow) * p.D * sizeof(T)
                                     + Core::lane_bytes(p, c0) + Core::col_bytes(p, c0, j), Vec<T>::pack(o));
-#pragma unroll
-                    for (int q4 = 0; q4 < Q4; ++q4) {                  // d_bias_k = sum dK
-                        float4 a = acc_bk[(j * Q4 + q4) * 32 + lane];
-                        a.x = fmaf(sum_ds, qs[j][4 * q4], a.x); a.y = fmaf(sum_ds, qs[j][4 * q4 + 1], a.y);
-                        a.z = fmaf(sum_ds, qs[j][4 * q4 + 2], a.z); a.w = fmaf(sum_ds, qs[j][4 * q4 + 3], a.w);
-                        acc_bk[(j * Q4 + q4) * 32 + lane] = a;
-                    }
+                    strip_fma(acc_bk, j, lane, sum_ds, qs[j]);          // d_bias_k = sum dK
                 }
             }
         }
