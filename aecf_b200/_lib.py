@@ -19,6 +19,7 @@ F32, BF16 = 0, 1
 K_MAJOR, MN_MAJOR = 0, 1
 GEMM_AUTO, GEMM_SIMT, GEMM_TCGEN05 = 0, 1, 2
 OK, ERR_INVALID, ERR_UNSUPPORTED, ERR_ALIGNMENT, ERR_WORKSPACE, ERR_CUDA = 0, -1, -2, -3, -4, -5
+PARAM_CAST_MAX_SEGMENTS = 8
 
 EXPORTS = (
     "aecf_pool_fwd", "aecf_pool_bwd", "aecf_pool_bwd_workspace_bytes",
@@ -28,7 +29,7 @@ EXPORTS = (
     "aecf_gemm", "aecf_gemm_aux", "aecf_gemm_workspace_bytes",
     "aecf_colsum", "aecf_colsum_workspace_bytes",
     "aecf_entropy_loss_fwd", "aecf_entropy_loss_bwd", "aecf_curriculum_mask", "aecf_curriculum_mask_bwd", "aecf_entropy_bwd", "aecf_sdpa_fwd", "aecf_sdpa_bwd",
-    "aecf_fusion_fwd", "aecf_fusion_bwd", "aecf_fusion_workspace_bytes", "aecf_fusion_grad_sums_bytes",
+    "aecf_param_cast", "aecf_fusion_fwd", "aecf_fusion_bwd", "aecf_fusion_workspace_bytes", "aecf_fusion_grad_sums_bytes",
     "aecf_peer_flag_bytes", "aecf_peer_enable_access", "aecf_peer_allreduce", "aecf_peer_export", "aecf_peer_import",
     "aecf_timing_enable", "aecf_timing_collect", "aecf_timing_site_name", "aecf_timing_site_gemm_kernel",
     "aecf_abi_version", "aecf_strerror", "aecf_last_cuda_error", "aecf_launch_count", "aecf_build_info",
@@ -49,7 +50,7 @@ class PoolDesc(C.Structure):
         ("fold_key", C.c_int32), ("tgt_len", C.c_int32),
         ("rng_state", C.c_void_p),
         ("q_stride_b", C.c_int64), ("q_stride_s", C.c_int64), ("bias_stride_s", C.c_int64),
-        ("loss_out", C.c_void_p), ("loss_workspace", C.c_void_p), ("loss_target", C.c_float), ("reserved0", C.c_int32),
+        ("loss_out", C.c_void_p), ("loss_workspace", C.c_void_p), ("loss_target", C.c_float), ("param_grads_f32", C.c_int32),
         ("row_index", C.c_void_p), ("src_rows", C.c_int64),
     ]
 
@@ -89,7 +90,7 @@ class FusionGrads(C.Structure):
         "side_stream", "fork_event", "fork_event2", "join_event")] + [("dp", C.POINTER(DpDesc))]
 
 
-SITE_COUNT = 21
+SITE_COUNT = 22
 
 
 class AecfError(RuntimeError):
@@ -162,6 +163,8 @@ def _declare(lib):
     lib.aecf_sdpa_bwd.restype = C.c_int
     lib.aecf_sdpa_bwd.argtypes = [C.c_int32, C.c_int32, vp, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, C.c_int64, C.c_int32, C.c_int32,
                                   C.c_int32, vp]
+    lib.aecf_param_cast.restype = C.c_int
+    lib.aecf_param_cast.argtypes = [C.c_int32, C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), vp, vp]
     lib.aecf_fusion_fwd.restype = C.c_int
     lib.aecf_fusion_fwd.argtypes = [C.POINTER(PoolDesc), C.POINTER(FusionTensors), vp, C.c_size_t, vp]
     lib.aecf_fusion_bwd.restype = C.c_int

@@ -70,8 +70,9 @@ struct TimedLaunch {                                          // brackets the la
         if (err__ != cudaSuccess) return ::aecf::set_cuda_error(err__, #call); \
     } while (0)
 
-// fold.cu: dWq, d_query and the packed in-projection bias gradient of a shared query, one launch
-int launch_query_tail(int dtype, int D, const float* d_qp, const void* q0, const void* in_proj_weight,
+// fold.cu: dWq, d_query and the packed in-projection bias gradient of a shared query, one launch; the gradients in
+// grad_dtype (dtype, or fp32 next to bf16 parameters in mixed precision)
+int launch_query_tail(int dtype, int grad_dtype, int D, const float* d_qp, const void* q0, const void* in_proj_weight,
                       const float* d_bias_kv, void* d_in_proj_weight, void* d_query, void* d_in_proj_bias, cudaStream_t s);
 
 // ---- programmatic dependent launch (PDL) -----------------------------------------------------

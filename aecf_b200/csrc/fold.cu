@@ -182,13 +182,14 @@ fold_finish_kernel(const float* __restrict__ g, const float* __restrict__ q_proj
 // The query-side tail of the backward for a shared query, one launch instead of three (outer product, GEMV, pack):
 //   dWq[i, :]  = d_qp[i] * q0[:]                 rows [0, D) of d_in_proj_weight        (torch/nn/functional.py:5854)
 //   d_query[i] = sum_k d_qp[k] * Wq[k, i]
-//   d_in_proj_bias = [ d_qp | d_bias_kv ]        in the parameter dtype
-// Block b owns the 8 indices i = 8b .. 8b+7.
-template <typename T>
+//   d_in_proj_bias = [ d_qp | d_bias_kv ]
+// Block b owns the 8 indices i = 8b .. 8b+7.  T: the parameters it reads; G: the gradients it writes (the parameter dtype,
+// or fp32 next to bf16 shadows of fp32 parameters in mixed precision).
+template <typename T, typename G>
 __global__ void __launch_bounds__(256)
 query_tail_kernel(const float* __restrict__ d_qp, const T* __restrict__ q0, const T* __restrict__ in_proj_weight,
-                  const float* __restrict__ d_bias_kv, int D, T* __restrict__ d_in_proj_weight, T* __restrict__ d_query,
-                  T* __restrict__ d_in_proj_bias) {
+                  const float* __restrict__ d_bias_kv, int D, G* __restrict__ d_in_proj_weight, G* __restrict__ d_query,
+                  G* __restrict__ d_in_proj_bias) {
     __shared__ float red[32][9];
     pdl_wait();
     const int i0 = blockIdx.x * 8;
@@ -196,8 +197,8 @@ query_tail_kernel(const float* __restrict__ d_qp, const T* __restrict__ q0, cons
     if (d_in_proj_weight != nullptr && i0 + warp < D) {
         const int i = i0 + warp;
         const float g = __ldg(d_qp + i);
-        T* row = d_in_proj_weight + static_cast<size_t>(i) * D;
-        for (int d = lane; d < D; d += 32) row[d] = from_float<T>(g * to_float<T>(q0[d]));
+        G* row = d_in_proj_weight + static_cast<size_t>(i) * D;
+        for (int d = lane; d < D; d += 32) row[d] = from_float<G>(g * to_float<T>(q0[d]));
     }
     if (d_query != nullptr) {
         const int ii = threadIdx.x & 7, kl = threadIdx.x >> 3;           // 8 columns x 32 row lanes
@@ -210,27 +211,33 @@ query_tail_kernel(const float* __restrict__ d_qp, const T* __restrict__ q0, cons
             float s = 0.f;
 #pragma unroll
             for (int k = 0; k < 32; ++k) s += red[k][threadIdx.x];
-            d_query[i0 + threadIdx.x] = from_float<T>(s);
+            d_query[i0 + threadIdx.x] = from_float<G>(s);
         }
     }
     if (d_in_proj_bias != nullptr && threadIdx.x < 8 && i0 + threadIdx.x < D) {
         const int i = i0 + threadIdx.x;
-        d_in_proj_bias[i] = from_float<T>(d_qp[i]);
-        d_in_proj_bias[D + i] = from_float<T>(d_bias_kv[i]);
-        d_in_proj_bias[2 * D + i] = from_float<T>(d_bias_kv[D + i]);
+        d_in_proj_bias[i] = from_float<G>(d_qp[i]);
+        d_in_proj_bias[D + i] = from_float<G>(d_bias_kv[i]);
+        d_in_proj_bias[2 * D + i] = from_float<G>(d_bias_kv[D + i]);
     }
 }
 
-int launch_query_tail(int dtype, int D, const float* d_qp, const void* q0, const void* in_proj_weight,
+int launch_query_tail(int dtype, int grad_dtype, int D, const float* d_qp, const void* q0, const void* in_proj_weight,
                       const float* d_bias_kv, void* d_in_proj_weight, void* d_query, void* d_in_proj_bias, cudaStream_t s) {
     const dim3 grid((D + 7) / 8), block(256);
-    if (dtype == AECF_BF16)
-        AECF_CUDA_OK(launch_pdl(query_tail_kernel<__nv_bfloat16>, grid, block, 0, s, d_qp, static_cast<const __nv_bfloat16*>(q0),
+    if (dtype != grad_dtype) {
+        if (dtype != AECF_BF16 || grad_dtype != AECF_F32) return AECF_ERR_INVALID;
+        AECF_CUDA_OK(launch_pdl(query_tail_kernel<__nv_bfloat16, float>, grid, block, 0, s, d_qp, static_cast<const __nv_bfloat16*>(q0),
+                                static_cast<const __nv_bfloat16*>(in_proj_weight), d_bias_kv, D,
+                                static_cast<float*>(d_in_proj_weight), static_cast<float*>(d_query),
+                                static_cast<float*>(d_in_proj_bias)));
+    } else if (dtype == AECF_BF16)
+        AECF_CUDA_OK(launch_pdl(query_tail_kernel<__nv_bfloat16, __nv_bfloat16>, grid, block, 0, s, d_qp, static_cast<const __nv_bfloat16*>(q0),
                                 static_cast<const __nv_bfloat16*>(in_proj_weight), d_bias_kv, D,
                                 static_cast<__nv_bfloat16*>(d_in_proj_weight), static_cast<__nv_bfloat16*>(d_query),
                                 static_cast<__nv_bfloat16*>(d_in_proj_bias)));
     else
-        AECF_CUDA_OK(launch_pdl(query_tail_kernel<float>, grid, block, 0, s, d_qp, static_cast<const float*>(q0),
+        AECF_CUDA_OK(launch_pdl(query_tail_kernel<float, float>, grid, block, 0, s, d_qp, static_cast<const float*>(q0),
                                 static_cast<const float*>(in_proj_weight), d_bias_kv, D, static_cast<float*>(d_in_proj_weight),
                                 static_cast<float*>(d_query), static_cast<float*>(d_in_proj_bias)));
     count_launch();

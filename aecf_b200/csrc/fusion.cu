@@ -7,7 +7,7 @@
 
 namespace aecf {
 
-// [d_qp fp32 D | d_bias_kv fp32 2D] -> in_proj_bias gradient [3D] in the parameter dtype
+// [d_qp fp32 D | d_bias_kv fp32 2D] -> in_proj_bias gradient [3D] in the gradient dtype
 template <typename T>
 __global__ void pack_in_bias_kernel(const float* __restrict__ d_q, const float* __restrict__ d_bias_kv, int D,
                                     T* __restrict__ out) {
@@ -20,6 +20,7 @@ __global__ void pack_in_bias_kernel(const float* __restrict__ d_q, const float* 
 struct Geometry {
     long long B, rows, QR;     // samples, key/value rows (B * M), query rows (B * S)
     int M, D, H, es, dt;
+    int gdt, ges;      // dtype and element size of the parameter gradients (fp32 in mixed precision, else dt)
     bool shared, fold;
     int HS, HSP;       // folded key projection: score columns (fp32, H rounded up to 4) / score-gradient columns (dt, 16-byte multiple)
 };
@@ -27,6 +28,7 @@ struct Geometry {
 static int geometry(const aecf_pool_desc* d, Geometry* g) {
     if (!d || d->batch < 0 || d->embed_dim <= 0 || d->num_tokens <= 0) return AECF_ERR_INVALID;
     if (d->dtype != AECF_F32 && d->dtype != AECF_BF16) return AECF_ERR_INVALID;
+    if (d->param_grads_f32 != 0 && (d->param_grads_f32 != 1 || d->dtype != AECF_BF16)) return AECF_ERR_INVALID;
     g->B = d->batch; g->M = d->num_tokens; g->D = d->embed_dim;
     // row indirection: the pool kernels take the `batch` listed rows, the products around them all `src_rows` samples
     const long long samples = d->row_index != nullptr ? d->src_rows : d->batch;
@@ -34,6 +36,7 @@ static int geometry(const aecf_pool_desc* d, Geometry* g) {
     g->rows = samples * g->M;
     g->QR = samples * (d->tgt_len > 1 ? d->tgt_len : 1);
     g->dt = d->dtype; g->es = d->dtype == AECF_BF16 ? 2 : 4; g->shared = d->q_is_shared != 0;
+    g->gdt = d->param_grads_f32 ? AECF_F32 : d->dtype; g->ges = g->gdt == AECF_BF16 ? 2 : 4;
     g->H = d->num_heads; g->fold = d->fold_key != 0;
     g->HS = (g->H + 3) & ~3; g->HSP = aecf_fold_score_cols(d->dtype, g->H);
     if (g->fold && (!g->shared || g->H <= 0 || g->H > 32)) return AECF_ERR_UNSUPPORTED;
@@ -87,12 +90,12 @@ static aecf_gemm_desc gemm_desc(int device, int dta, int dtb, int dtc, int dtbia
 
 // Largest GEMM workspace any product of the step can ask for (split-K partials of the weight gradients).
 static size_t max_gemm_workspace(const aecf_pool_desc* d, const Geometry& g) {
-    const int dt = g.dt, D = g.D;
+    const int dt = g.dt, gdt = g.gdt, D = g.D;
     size_t need = 16;
     const aecf_gemm_desc probes[] = {
-        gemm_desc(d->device, dt, dt, dt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, 2 * D, D, g.rows, 2 * D, D, D),   // dW_kv
-        gemm_desc(d->device, dt, dt, dt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.rows, 2 * D, D, D),       // dW_k / dW_v
-        gemm_desc(d->device, dt, dt, dt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.QR, D, D, D),             // dW_o, dW_q
+        gemm_desc(d->device, dt, dt, gdt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, 2 * D, D, g.rows, 2 * D, D, D),  // dW_kv
+        gemm_desc(d->device, dt, dt, gdt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.rows, 2 * D, D, D),      // dW_k / dW_v
+        gemm_desc(d->device, dt, dt, gdt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.QR, D, D, D),            // dW_o, dW_q
         gemm_desc(d->device, dt, dt, dt, dt, AECF_K_MAJOR, AECF_K_MAJOR, g.rows, 2 * D, D, D, D, 2 * D),     // kv
         gemm_desc(d->device, dt, dt, dt, dt, AECF_K_MAJOR, AECF_MN_MAJOR, g.rows, D, 2 * D, 2 * D, D, D),    // dX
         gemm_desc(d->device, dt, dt, AECF_F32, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D + g.HSP, D, g.rows, D + g.HSP, D, D),   // folded [dWv ; R]
@@ -159,7 +162,7 @@ static int folded_backward(const aecf_pool_desc* desc, const Geometry& g, const 
                         gr->join_event != nullptr && want_tail;
     cudaStream_t side = forked ? static_cast<cudaStream_t>(gr->side_stream) : s;
     GradTailArgs a{};
-    a.dtype = dt; a.D = D; a.H = g.H; a.HSP = g.HSP; a.sms = sm_count(dev);
+    a.dtype = dt; a.grad_dtype = g.gdt; a.D = D; a.H = g.H; a.HSP = g.HSP; a.sms = sm_count(dev);
     a.scratch = w.tail;
     a.sums = dp ? static_cast<float*>(dp->sums[dp->rank]) : w.sums;
     a.q_proj = static_cast<const float*>(t->q_proj); a.in_proj_weight = t->in_proj_weight; a.query = t->query;
@@ -343,7 +346,7 @@ int aecf_fusion_bwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, co
     Workspace w;
     carve(desc, g, workspace, &w);
     if (workspace_bytes < w.total) return AECF_ERR_WORKSPACE;
-    const int dt = g.dt, es = g.es, D = g.D, dev = desc->device;
+    const int dt = g.dt, es = g.es, gdt = g.gdt, ges = g.ges, D = g.D, dev = desc->device;
     const long long DD = static_cast<long long>(D) * D;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
 
@@ -354,11 +357,11 @@ int aecf_fusion_bwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, co
     // ---- out-projection backward ----------------------------------------------------------------------
     if (gr->d_out_proj_bias) {
         ScopedSite site(AECF_SITE_D_OUT_BIAS);
-        AECF_TRY(aecf_colsum(dev, dt, dt, gr->d_out, g.QR, D, D, gr->d_out_proj_bias, w.colsum, w.colsum_bytes, stream));
+        AECF_TRY(aecf_colsum(dev, dt, gdt, gr->d_out, g.QR, D, D, gr->d_out_proj_bias, w.colsum, w.colsum_bytes, stream));
     }
     if (gr->d_out_proj_weight) {                             // dWo = g^T ctx
         ScopedSite site(AECF_SITE_D_OUT_WEIGHT);
-        const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.QR, D, D, D);
+        const aecf_gemm_desc d = gemm_desc(dev, dt, dt, gdt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.QR, D, D, D);
         AECF_TRY(aecf_gemm(&d, gr->d_out, t->ctx, nullptr, gr->d_out_proj_weight, w.gemm, w.gemm_bytes, stream));
     }
     {                                                        // d_ctx = g Wo
@@ -394,12 +397,12 @@ int aecf_fusion_bwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, co
         {
             ScopedSite site(AECF_SITE_D_KV_WEIGHT);
             if (!t->value) {          // dW_kv = dKV^T X
-                const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, 2 * D, D, g.rows, 2 * D, D, D);
-                AECF_TRY(aecf_gemm(&d, gr->d_kv, t->key, nullptr, at(gr->d_in_proj_weight, DD, es), w.gemm, w.gemm_bytes, stream));
+                const aecf_gemm_desc d = gemm_desc(dev, dt, dt, gdt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, 2 * D, D, g.rows, 2 * D, D, D);
+                AECF_TRY(aecf_gemm(&d, gr->d_kv, t->key, nullptr, at(gr->d_in_proj_weight, DD, ges), w.gemm, w.gemm_bytes, stream));
             } else {
-                const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.rows, 2 * D, D, D);
-                AECF_TRY(aecf_gemm(&d, gr->d_kv, t->key, nullptr, at(gr->d_in_proj_weight, DD, es), w.gemm, w.gemm_bytes, stream));
-                AECF_TRY(aecf_gemm(&d, at(gr->d_kv, D, es), t->value, nullptr, at(gr->d_in_proj_weight, 2 * DD, es), w.gemm,
+                const aecf_gemm_desc d = gemm_desc(dev, dt, dt, gdt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.rows, 2 * D, D, D);
+                AECF_TRY(aecf_gemm(&d, gr->d_kv, t->key, nullptr, at(gr->d_in_proj_weight, DD, ges), w.gemm, w.gemm_bytes, stream));
+                AECF_TRY(aecf_gemm(&d, at(gr->d_kv, D, es), t->value, nullptr, at(gr->d_in_proj_weight, 2 * DD, ges), w.gemm,
                                    w.gemm_bytes, stream));
             }
         }
@@ -409,14 +412,14 @@ int aecf_fusion_bwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, co
         if (gr->d_in_proj_weight || gr->d_query || gr->d_in_proj_bias) {
             ScopedSite site(AECF_SITE_D_QUERY);
             TimedLaunch timed(s);
-            AECF_TRY(launch_query_tail(dt, D, w.d_qp, t->query, t->in_proj_weight, w.d_bias_kv, gr->d_in_proj_weight,
+            AECF_TRY(launch_query_tail(dt, gdt, D, w.d_qp, t->query, t->in_proj_weight, w.d_bias_kv, gr->d_in_proj_weight,
                                        gr->d_query, gr->d_in_proj_bias, s));
         }
         return AECF_OK;
     }
     if (gr->d_in_proj_weight) {   // ---- query rows of the in-projection weight gradient: dW_q = d_q^T Q -------------
         ScopedSite site(AECF_SITE_D_Q_WEIGHT);
-        const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.QR, D, D, D);
+        const aecf_gemm_desc d = gemm_desc(dev, dt, dt, gdt, dt, AECF_MN_MAJOR, AECF_MN_MAJOR, D, D, g.QR, D, D, D);
         AECF_TRY(aecf_gemm(&d, gr->d_q_rows, t->query, nullptr, gr->d_in_proj_weight, w.gemm, w.gemm_bytes, stream));
     }
     if (gr->d_query) {                // ---- gradient of the (unprojected) per-row queries ------------------------
@@ -424,12 +427,12 @@ int aecf_fusion_bwd(const aecf_pool_desc* desc, const aecf_fusion_tensors* t, co
         const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_K_MAJOR, AECF_MN_MAJOR, g.QR, D, D, D, D, D);
         AECF_TRY(aecf_gemm(&d, gr->d_q_rows, t->in_proj_weight, nullptr, gr->d_query, w.gemm, w.gemm_bytes, stream));
     }
-    if (gr->d_in_proj_bias) {         // ---- [d_bq | d_bk | d_bv] in the parameter dtype ------------------------
+    if (gr->d_in_proj_bias) {         // ---- [d_bq | d_bk | d_bv] in the gradient dtype -------------------------
         ScopedSite site(AECF_SITE_D_IN_BIAS);
         AECF_TRY(aecf_colsum(dev, dt, AECF_F32, gr->d_q_rows, g.QR, D, D, w.d_bq, w.colsum, w.colsum_bytes, stream));
         TimedLaunch timed(s);
         const int n = 3 * D;
-        if (dt == AECF_BF16)
+        if (gdt == AECF_BF16)
             AECF_CUDA_OK(launch_pdl(pack_in_bias_kernel<__nv_bfloat16>, dim3((n + 255) / 256), dim3(256), 0, s, w.d_bq, w.d_bias_kv,
                                     D, static_cast<__nv_bfloat16*>(gr->d_in_proj_bias)));
         else

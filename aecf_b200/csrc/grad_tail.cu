@@ -11,8 +11,9 @@
 //   grad_peer_sum (world > 1) S summed over the ranks in fp32 through NVLink peer mappings: flag barrier, rank r sums
 //                 slice r of every rank's S in rank order and stores it into every rank's reduced buffer, flag barrier
 //                 (the scheme of peer_allreduce.cu, from one buffer into another)
-//   grad_finish   S -> parameter gradients in the parameter dtype: dWv, dWk = scale q (x) R, d_qp = scale Wk . R,
-//                 dWq = d_qp (x) q0, the three in-projection bias thirds, dWo, d_out_proj_bias; grad_dquery then forms
+//   grad_finish   S -> parameter gradients in the parameter dtype (fp32 in mixed precision, next to bf16 shadows of the
+//                 parameters): dWv, dWk = scale q (x) R, d_qp = scale Wk . R, dWq = d_qp (x) q0, the three in-projection
+//                 bias thirds, dWo, d_out_proj_bias; grad_dquery then forms
 //                 d_query = d_qp . Wq (reference: what autograd derives from torch/nn/functional.py:5854-5855, 6653 for a
 //                 shared query)
 //
@@ -315,7 +316,9 @@ template <> __device__ __forceinline__ float4 load4<__nv_bfloat16>(const __nv_bf
 // One warp per in-projection row i (head h = i / head_dim), 8 rows per block:
 //   dWv[i, :] = G[i, :]     dWk[i, :] = scale q[i] R[h, :]     d_qp[i] = scale Wk[i, :] . R[h, :]     dWo[i, :] = O[i, :]
 //   dWq[i, :] = d_qp[i] q0[:]     d_in_b = [ d_qp | d_bias_k | d_bias_v ]     d_out_b = colsum(d_out)
-template <typename T>
+// T: the parameters it reads (in_proj_weight, query, out_proj_weight); TG: the parameter gradients it writes (fp32 in mixed
+// precision, where the parameters are bf16 shadows of fp32 masters).
+template <typename T, typename TG>
 __global__ void __launch_bounds__(TAIL_THREADS, 1)
 grad_finish_kernel(const FinishParams p) {
     __shared__ float qps[8];                                    // d_qp of the block's 8 rows
@@ -325,7 +328,7 @@ grad_finish_kernel(const FinishParams p) {
     pdl_wait();
     const T* W = static_cast<const T*>(p.in_proj_weight);
     const T* q0 = static_cast<const T*>(p.query);
-    T* d_in_w = static_cast<T*>(p.d_in_w);
+    TG* d_in_w = static_cast<TG*>(p.d_in_w);
     float d_qp = 0.f;
     if (i < D) {
     const int h = i / (D / p.H);
@@ -355,11 +358,11 @@ grad_finish_kernel(const FinishParams p) {
             dot = fmaf(w[u].x, r[u].x, dot); dot = fmaf(w[u].y, r[u].y, dot);
             dot = fmaf(w[u].z, r[u].z, dot); dot = fmaf(w[u].w, r[u].w, dot);
             if (d_in_w != nullptr) {
-                store4<T>(d_in_w + (static_cast<long long>(D) + i) * D + d, sq * r[u].x, sq * r[u].y, sq * r[u].z, sq * r[u].w);
-                store4<T>(d_in_w + (2LL * D + i) * D + d, g[u].x, g[u].y, g[u].z, g[u].w);
+                store4<TG>(d_in_w + (static_cast<long long>(D) + i) * D + d, sq * r[u].x, sq * r[u].y, sq * r[u].z, sq * r[u].w);
+                store4<TG>(d_in_w + (2LL * D + i) * D + d, g[u].x, g[u].y, g[u].z, g[u].w);
             }
             if (p.d_out_w != nullptr)
-                store4<T>(static_cast<T*>(p.d_out_w) + static_cast<long long>(i) * D + d, o[u].x, o[u].y, o[u].z, o[u].w);
+                store4<TG>(static_cast<TG*>(p.d_out_w) + static_cast<long long>(i) * D + d, o[u].x, o[u].y, o[u].z, o[u].w);
         }
     }
 #pragma unroll
@@ -373,7 +376,7 @@ grad_finish_kernel(const FinishParams p) {
 #pragma unroll
             for (int u = 0; u < 4; ++u)
                 if (d0 + 128 * u < D)
-                    store4<T>(d_in_w + static_cast<long long>(i) * D + d0 + 128 * u, d_qp * q[u].x, d_qp * q[u].y, d_qp * q[u].z,
+                    store4<TG>(d_in_w + static_cast<long long>(i) * D + d0 + 128 * u, d_qp * q[u].x, d_qp * q[u].y, d_qp * q[u].z,
                               d_qp * q[u].w);
         }
     }
@@ -398,17 +401,17 @@ grad_finish_kernel(const FinishParams p) {
     }
     if (lane == 0) {
         if (p.d_in_b != nullptr) {
-            T* db = static_cast<T*>(p.d_in_b);
-            db[i] = from_float<T>(d_qp);
+            TG* db = static_cast<TG*>(p.d_in_b);
+            db[i] = from_float<TG>(d_qp);
             if (p.out_proj_weight != nullptr) {
-                db[D + i] = from_float<T>(0.f);                                    // d_bias_k
-                db[2 * D + i] = from_float<T>(bias_v);                             // d_bias_v
+                db[D + i] = from_float<TG>(0.f);                                    // d_bias_k
+                db[2 * D + i] = from_float<TG>(bias_v);                             // d_bias_v
             } else {
-                db[D + i] = from_float<T>(p.sums[p.lay.pool + 2LL * D + i]);       // d_bias_k
-                db[2 * D + i] = from_float<T>(p.sums[p.lay.pool + D + i]);         // d_bias_v
+                db[D + i] = from_float<TG>(p.sums[p.lay.pool + 2LL * D + i]);       // d_bias_k
+                db[2 * D + i] = from_float<TG>(p.sums[p.lay.pool + D + i]);         // d_bias_v
             }
         }
-        if (p.d_out_b != nullptr) static_cast<T*>(p.d_out_b)[i] = from_float<T>(p.sums[p.lay.bo + i]);
+        if (p.d_out_b != nullptr) static_cast<TG*>(p.d_out_b)[i] = from_float<TG>(p.sums[p.lay.bo + i]);
     }
     }   // i < D
     // this block's share of d_query[c] = sum_i d_qp[i] Wq[i, c] (torch/nn/functional.py:5854 backward): a thread owns its
@@ -506,6 +509,7 @@ int launch_grad_gather(const GradTailArgs& a, int which, cudaStream_t s) {
 
 int launch_grad_finish(const GradTailArgs& a, const float* sums, cudaStream_t s) {
     if (a.D % 4 != 0) return AECF_ERR_UNSUPPORTED;
+    if (a.dtype != a.grad_dtype && (a.dtype != AECF_BF16 || a.grad_dtype != AECF_F32)) return AECF_ERR_INVALID;
     FinishParams p{};
     p.sums = sums; p.lay = tail_layout(a.D, a.HSP);
     p.q_proj = a.q_proj; p.in_proj_weight = a.in_proj_weight; p.query = a.query; p.out_proj_weight = a.out_proj_weight;
@@ -515,13 +519,14 @@ int launch_grad_finish(const GradTailArgs& a, const float* sums, cudaStream_t s)
     p.d_qp = reinterpret_cast<float*>(static_cast<char*>(a.scratch) + align256(static_cast<size_t>(a.sms) * a.D * sizeof(float)));
     const dim3 grid(static_cast<unsigned>((a.D + 7) / 8)), block(TAIL_THREADS);
     TimedLaunch timed(s, AECF_SITE_GRAD_FINISH);
-    if (a.dtype == AECF_BF16) AECF_CUDA_OK(launch_pdl(grad_finish_kernel<__nv_bfloat16>, grid, block, 0, s, p));
-    else AECF_CUDA_OK(launch_pdl(grad_finish_kernel<float>, grid, block, 0, s, p));
+    if (a.dtype != a.grad_dtype) AECF_CUDA_OK(launch_pdl(grad_finish_kernel<__nv_bfloat16, float>, grid, block, 0, s, p));
+    else if (a.dtype == AECF_BF16) AECF_CUDA_OK(launch_pdl(grad_finish_kernel<__nv_bfloat16, __nv_bfloat16>, grid, block, 0, s, p));
+    else AECF_CUDA_OK(launch_pdl(grad_finish_kernel<float, float>, grid, block, 0, s, p));
     count_launch();
-    if (a.d_query != nullptr) {
+    if (a.d_query != nullptr) {                                 // (reads fp32 partials only: one type, the gradient's)
         const dim3 g2(static_cast<unsigned>((a.D + 7) / 8));
         const int rows = (a.D + 7) / 8;
-        if (a.dtype == AECF_BF16)
+        if (a.grad_dtype == AECF_BF16)
             AECF_CUDA_OK(launch_pdl(grad_dquery_fold_kernel<__nv_bfloat16>, g2, block, 0, s, static_cast<const float*>(p.d_qp), rows, a.D,
                                     static_cast<__nv_bfloat16*>(a.d_query)));
         else

@@ -20,6 +20,7 @@ inline TailLayout tail_layout(int D, int HSP) {
 
 struct GradTailArgs {
     int dtype, D, H, HSP, sms;
+    int grad_dtype;                     // of d_in_w ... d_query: dtype, or fp32 next to bf16 parameters (mixed precision)
     GemmPartials g, o;                  // [dWv ; R] and dWo as left by gemm_partials (o.partial null: no dWo wanted)
     const void* d_out; long long rows;  // column sums of d_out -> d_out_proj_bias (null: not wanted)
     // the pool backward's per-sample [s | sum_m ds] ([samples][2 HSP] fp32) and d_ctx: d_bias_v = sum_b s[b, h] d_ctx[b, :],

@@ -84,6 +84,36 @@ colsum_stage2(const float* __restrict__ partial, long long cols, int splits, TO*
     out[c] = from_float<TO>(s);
 }
 
+// ---- parameter shadow -----------------------------------------------------------------------
+// fp32 segments -> one bf16 block, round to nearest even (NaN stays NaN, +-inf stays +-inf).  blockIdx.y is the segment;
+// blocks stride over its 8-element chunks (two 16-byte loads, one 16-byte store), the last count % 8 elements -- and every
+// element of a source that is not 16-byte aligned -- go one at a time.
+struct ParamCastParams {
+    const float* src[AECF_PARAM_CAST_MAX_SEGMENTS];
+    long long count[AECF_PARAM_CAST_MAX_SEGMENTS];
+    long long offset[AECF_PARAM_CAST_MAX_SEGMENTS];            // in elements of dst, multiples of 8
+    long long chunks[AECF_PARAM_CAST_MAX_SEGMENTS];            // 8-element chunks of the vectorised body (0: src not aligned)
+};
+
+__global__ void __launch_bounds__(256)
+param_cast_kernel(const ParamCastParams p, __nv_bfloat16* __restrict__ dst) {
+    pdl_wait();
+    const int seg = blockIdx.y;
+    const float* src = p.src[seg];
+    const long long n = p.count[seg];
+    __nv_bfloat16* out = dst + p.offset[seg];
+    const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
+    const long long t0 = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    const long long chunks = p.chunks[seg];
+    for (long long c = t0; c < chunks; c += stride) {
+        const float4 a = *reinterpret_cast<const float4*>(src + 8 * c);
+        const float4 b = *reinterpret_cast<const float4*>(src + 8 * c + 4);
+        const float f[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+        stg_vec(out + 8 * c, Vec<__nv_bfloat16>::pack(f));
+    }
+    for (long long i = 8 * chunks + t0; i < n; i += stride) out[i] = from_float<__nv_bfloat16>(src[i]);
+}
+
 static int colsum_splits(long long rows) {
     long long s = (rows + 255) / 256;
     if (s < 1) s = 1;
@@ -536,6 +566,32 @@ int aecf_colsum(int32_t device, int32_t dtype_x, int32_t dtype_out, const void* 
     else
         AECF_CUDA_OK(launch_pdl(colsum_stage2<float>, g2, dim3(256), 0, s, partial, cols, splits, static_cast<float*>(out)));
     count_launch(2);
+    return AECF_OK;
+}
+
+int aecf_param_cast(int32_t device, int32_t segments, const float* const* src, const int64_t* counts, void* dst,
+                    void* stream) {
+    if (!src || !counts || !dst || segments <= 0 || segments > AECF_PARAM_CAST_MAX_SEGMENTS) return AECF_ERR_INVALID;
+    if (!aligned16(dst)) return AECF_ERR_ALIGNMENT;
+    ParamCastParams p{};
+    long long offset = 0, widest = 0;
+    for (int i = 0; i < segments; ++i) {
+        if (counts[i] < 0 || (counts[i] > 0 && !src[i])) return AECF_ERR_INVALID;
+        p.src[i] = src[i]; p.count[i] = counts[i]; p.offset[i] = offset;
+        p.chunks[i] = aligned16(src[i]) ? counts[i] / 8 : 0;
+        offset += (counts[i] + 7) / 8 * 8;                     // the next segment starts on a 16-byte boundary
+        widest = counts[i] > widest ? counts[i] : widest;
+    }
+    if (widest == 0) return AECF_OK;
+    DeviceScope device_scope__(device);
+    int rc = device_scope__.rc;
+    if (rc != AECF_OK) return rc;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    TimedLaunch timed(s, AECF_SITE_PARAM_CAST);
+    const long long blocks = (widest + 8 * 256 - 1) / (8 * 256);
+    const dim3 grid(static_cast<unsigned>(blocks < 1024 ? blocks : 1024), static_cast<unsigned>(segments));
+    AECF_CUDA_OK(launch_pdl(param_cast_kernel, grid, dim3(256), 0, s, p, static_cast<__nv_bfloat16*>(dst)));
+    count_launch();
     return AECF_OK;
 }
 

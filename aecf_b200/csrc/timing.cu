@@ -29,7 +29,7 @@ thread_local int g_site = AECF_SITE_OTHER;
 const char* kSiteNames[AECF_SITE_COUNT] = {
     "other", "q_proj", "kv_proj", "pool_fwd", "out_proj", "d_out_bias", "d_out_weight", "d_ctx", "pool_bwd",
     "pool_bwd_finalize", "d_x", "d_kv_weight", "d_q_weight", "d_query", "d_in_bias", "entropy_loss", "fold_prepare",
-    "fold_finish", "grad_gather", "grad_peer_sum", "grad_finish"};
+    "fold_finish", "grad_gather", "grad_peer_sum", "grad_finish", "param_cast"};
 char g_site_gemm[AECF_SITE_COUNT][96];                 // the GEMM kernel last launched from each site (diagnostics)
 }  // namespace
 

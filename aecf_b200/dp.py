@@ -76,19 +76,31 @@ def _map_peer_tensors(tensors: List[torch.Tensor], group=None) -> List[List[int]
     return out
 
 
+def compute_dtype_of(pool) -> torch.dtype:
+    """The dtype the folded backward of ``pool`` runs in by default: its parameter dtype -- except for fp32 parameters
+    whose key projection is not forced to fold, where the folded backward only runs in mixed precision, on bf16 inputs."""
+    dtype = pool.attention.in_proj_weight.dtype
+    if dtype == torch.float32 and getattr(pool, "fold_key_projection", None) is not True:
+        return torch.bfloat16
+    return dtype
+
+
 class FusedGradSum:
     """The cross-rank gradient sum of the folded backward (``aecf_dp_desc``): raw-sum and reduced-sum buffers of every
     rank mapped into this process, plus the flag blocks of the kernel's two barriers.  Construction is collective.
     The pool's backward passes ``pointer()`` to ``aecf_fusion_bwd`` whenever ``usable(desc)``."""
 
-    def __init__(self, pool, group=None, average: bool = True, *, local_ranks: Optional[Tuple[int, int, list, list]] = None):
+    def __init__(self, pool, group=None, average: bool = True, *, local_ranks: Optional[Tuple[int, int, list, list]] = None,
+                 compute_dtype: Optional[torch.dtype] = None):
         """``local_ranks = (rank, world, buffers, flag blocks)``: W ranks EMULATED on one device (tests): the W buffers
-        (``None`` entries are allocated) and flag blocks are plain local tensors shared by the W instances, no IPC."""
+        (``None`` entries are allocated) and flag blocks are plain local tensors shared by the W instances, no IPC.
+        ``compute_dtype``: the dtype the backward runs in, which sets the layout of the raw sums (``compute_dtype_of``)."""
         import ctypes as C
 
         from . import _lib, ops
         att = pool.attention
-        dev, dtype = att.in_proj_weight.device, att.in_proj_weight.dtype
+        dev = att.in_proj_weight.device
+        dtype = compute_dtype or compute_dtype_of(pool)
         if local_ranks is not None:
             self.rank, self.world = local_ranks[0], local_ranks[1]
         else:
@@ -125,7 +137,11 @@ class FusedGradSum:
         self.ran = False                                 # set by the backward that used it (GradientSync.finish looks)
 
     def usable(self, desc) -> bool:
-        return (self.world > 1 and desc.fold_key == 1 and desc.embed_dim == self.embed_dim and desc.num_heads == self.num_heads)
+        """Whether the backward of ``desc`` can sum through these buffers: its raw sums must have the layout they were sized
+        for (embed_dim, num_heads and the compute dtype, whose 16-byte rounding of the heads sets the columns of R)."""
+        from . import ops
+        return (self.world > 1 and desc.fold_key == 1 and desc.embed_dim == self.embed_dim and desc.num_heads == self.num_heads
+                and desc.dtype == ops.dtype_code(self.dtype))
 
     def pointer(self):
         return self._ptr

@@ -9,6 +9,9 @@ Backward (SURVEY.md Appendix B; autograd of the same lines in the reference):
     colsum + dWo GEMM + dctx GEMM -> fused recompute pool backward -> dX GEMM + dWkv GEMM
     -> the small query-side products                        [aecf_fusion_bwd]
 Nothing the forward computed is kept except the projected K/V and the context.
+Mixed precision (``PoolConfig.mixed``): fp32 parameters, bf16 activations.  The forward first rounds the parameters to one
+bf16 block (``aecf_param_cast``), runs the bf16 step on those shadows and keeps them for the backward, which writes the
+parameter gradients in fp32 (``aecf_pool_desc::param_grads_f32``).
 """
 from __future__ import annotations
 
@@ -53,6 +56,9 @@ class PoolConfig:
     dp: Optional[object] = None
     # int64 [nb] device tensor: pool only these samples of the batch, in place (aecf_pool_desc::row_index)
     sample_index: Optional[torch.Tensor] = None
+    # mixed precision: fp32 parameters (and shared query), bf16 key / value.  The forward rounds the parameters to a bf16
+    # shadow (one launch, every call: never cached) and runs the bf16 step on it; the parameter gradients come out fp32
+    mixed: bool = False
 
 
 class SideStream:
@@ -111,12 +117,18 @@ class FusedPoolFunction(torch.autograd.Function):
             base_mask_prob=cfg.base_mask_prob, entropy_target=cfg.entropy_target, dropout_p=cfg.dropout_p,
             seed=cfg.seed, offset=cfg.offset, row0=cfg.row0, bias_strides=cfg.bias_strides, kv_strides=kv_strides,
             fold_key=fold, rng_state=cfg.rng_state, tgt_len=S,
-            q_strides=(1, B) if (S > 1 and cfg.seq_first) else (0, 0), row_index=index, src_rows=B if index is not None else 0)
+            q_strides=(1, B) if (S > 1 and cfg.seq_first) else (0, 0), row_index=index, src_rows=B if index is not None else 0,
+            param_grads_f32=cfg.mixed)
         IR = NB * S                                            # rows of the info tensors
 
         q_in = q_src.reshape(D) if cfg.q_shared else q_src.reshape(R, D)
         if not q_in.is_contiguous():
             q_in = q_in.contiguous()
+        if cfg.mixed:                                          # the bf16 shadows stand in for the fp32 parameters from here on
+            _, (in_w, in_b, out_w, out_b, q_sh) = ops.param_cast(
+                [in_w, in_b, out_w, out_b, q_in if cfg.q_shared else None])
+            if cfg.q_shared:
+                q_in = q_sh
         qp = torch.empty((D,), dtype=torch.float32, device=dev) if cfg.q_shared else torch.empty((R, D), dtype=dt, device=dev)
         kv = torch.empty((B * M, D if fold else 2 * D), dtype=dt, device=dev)     # folded: the values only
         scores = torch.empty((B * M, hs), dtype=torch.float32, device=dev) if fold else None
@@ -197,11 +209,15 @@ class FusedPoolFunction(torch.autograd.Function):
         if fused_dp is not None:
             notify = None
 
+        # the parameter gradients: in the parameter dtype -- fp32 in mixed precision, where `like` is the bf16 shadow
+        grad_dtype = torch.float32 if cfg.mixed else None
+
         def grad_like(name, like):
+            dtype = grad_dtype or like.dtype
             b = bufs.get(name)
-            if b is not None and b.numel() == like.numel() and b.dtype == like.dtype and b.is_contiguous():
+            if b is not None and b.numel() == like.numel() and b.dtype == dtype and b.is_contiguous():
                 return b.view(like.shape)
-            return torch.empty_like(like)
+            return torch.empty_like(like, dtype=dtype)
 
         d_q = (grad_like("query", q_in) if cfg.q_shared else new(q_in.shape, q_in.dtype)) if need_q else None
         d_in_w = grad_like("in_proj_weight", in_w) if need_in_w else None

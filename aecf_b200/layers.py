@@ -373,13 +373,22 @@ class MultimodalAttentionPool(nn.Module):
         # several queries per sample run on their own kernels (csrc/pool_multi.cuh)
         multi = tgt_len > 1
         att = self.attention
-        dt = att.in_proj_weight.dtype
-        if query.dtype != dt or key.dtype != dt or (value is not None and value.dtype != dt):
-            raise RuntimeError(f"expected query/key/value of dtype {dt} (the module's parameter dtype), "
-                               f"got {query.dtype}/{key.dtype}")
-
+        pdt = att.in_proj_weight.dtype
         q_src = None if multi else self._shared_query_source(query, batch)
         q_shared = q_src is not None
+        # Mixed precision: fp32 parameters, bf16 key / value (what torch.autocast hands over from bf16 encoders).  The step
+        # runs in bf16 on a bf16 rounding of the parameters, made on every call, and the parameter gradients are fp32.  The
+        # query is then either bf16 rows of its own or the shared fp32 fusion query (a parameter, rounded like the others).
+        dt = key.dtype
+        if q_shared and batch == 1 and pdt == torch.float32 and dt == torch.bfloat16 and query.dtype == torch.bfloat16:
+            q_src, q_shared = None, False                       # one sample: a bf16 query is that row's own
+        mixed = (pdt == torch.float32 and dt == torch.bfloat16
+                 and query.dtype == (torch.float32 if q_shared else torch.bfloat16))
+        if not mixed:
+            dt = pdt
+        if (not mixed and (query.dtype != dt or key.dtype != dt)) or (value is not None and value.dtype != dt):
+            raise RuntimeError(f"expected query/key/value of dtype {pdt} (the module's parameter dtype), "
+                               f"got {query.dtype}/{key.dtype}")
         if multi:
             q_src = query.contiguous()             # [B, S, D] or [S, B, D], used in place (rows (b, s) by strides)
         elif not q_shared:
@@ -424,7 +433,7 @@ class MultimodalAttentionPool(nn.Module):
             seq_first=not self.batch_first, fold=fold, want_mask_bits=self._want_mask_bits, bias_strides=bias_strides,
             tgt_len=tgt_len, grad_ready=self._grad_ready, grad_buffers=self._grad_buffers,
             loss_target=cm._loss_target() if (masking == 1 and return_info and os.environ.get("AECF_FUSED_LOSS", "1") != "0") else None,
-            side=self._side_stream(key.device) if fold else None, dp=self._dp, sample_index=index)
+            side=self._side_stream(key.device) if fold else None, dp=self._dp, sample_index=index, mixed=mixed)
         info_rows = batch if index is None else int(index.numel())
         out, pooled, entropy, mask_rate, masked, bits, fused_loss = FusedPoolFunction.apply(
             q_src, key_c, value_c, att.in_proj_weight, att.in_proj_bias, att.out_proj.weight, att.out_proj.bias,

@@ -111,6 +111,37 @@ def colsum(x2d: torch.Tensor, out_dtype: Optional[torch.dtype] = None, name="col
     return out
 
 
+def param_cast(tensors) -> Tuple[torch.Tensor, list]:
+    """bf16 shadows of fp32 parameters, one launch (``aecf_param_cast``): returns the block and, per entry of
+    ``tensors`` (``None`` entries stay ``None``), a view of it with that tensor's shape.  Each view starts on a 16-byte
+    boundary of the block, so it is a valid GEMM operand."""
+    present = [t for t in tensors if t is not None]
+    if len(present) > _lib.PARAM_CAST_MAX_SEGMENTS:
+        raise ValueError(f"param_cast: at most {_lib.PARAM_CAST_MAX_SEGMENTS} tensors per launch, got {len(present)}")
+    dev = require_cuda(*present)
+    offsets, total = [], 0
+    for t in present:
+        if t.dtype != torch.float32 or not t.is_contiguous():
+            raise TypeError("param_cast: the parameters must be contiguous float32 tensors")
+        offsets.append(total)
+        total += (t.numel() + 7) // 8 * 8
+    block = torch.empty(max(total, 8), dtype=torch.bfloat16, device=dev)
+    if present:
+        n = len(present)
+        src = (C.c_void_p * n)(*[t.data_ptr() for t in present])
+        counts = (C.c_int64 * n)(*[t.numel() for t in present])
+        rc = _lib.load().aecf_param_cast(dev.index or 0, n, src, counts, block.data_ptr(), _stream(dev))
+        _lib.check(rc, f"aecf_param_cast segments={n}")
+    views, i = [], 0
+    for t in tensors:
+        if t is None:
+            views.append(None)
+            continue
+        views.append(block[offsets[i]:offsets[i] + t.numel()].view(t.shape))
+        i += 1
+    return block, views
+
+
 def make_pool_desc(dev: torch.device, dtype: torch.dtype, *, batch: int, num_tokens: int, embed_dim: int,
                    num_heads: int, training: bool, masking: int, min_active: int, q_is_shared: bool,
                    base_mask_prob: float, entropy_target: float, dropout_p: float, seed: int, offset: int,
@@ -119,9 +150,11 @@ def make_pool_desc(dev: torch.device, dtype: torch.dtype, *, batch: int, num_tok
                    rng_state: Optional[torch.Tensor] = None, tgt_len: int = 1,
                    q_strides: Tuple[int, int] = (0, 0), loss_out: Optional[torch.Tensor] = None,
                    loss_workspace: Optional[torch.Tensor] = None, loss_target: float = 0.0,
-                   row_index: Optional[torch.Tensor] = None, src_rows: int = 0) -> _lib.PoolDesc:
+                   row_index: Optional[torch.Tensor] = None, src_rows: int = 0,
+                   param_grads_f32: bool = False) -> _lib.PoolDesc:
     """``bias_strides`` = (batch, head[, query]) element strides of the additive score bias; ``tgt_len`` > 1 and
-    ``q_strides`` (rows of query (b, s): b*q_strides[0] + s*q_strides[1]) describe several queries per sample."""
+    ``q_strides`` (rows of query (b, s): b*q_strides[0] + s*q_strides[1]) describe several queries per sample.
+    ``param_grads_f32``: mixed precision (bf16 shadows of fp32 parameters in, fp32 parameter gradients out)."""
     return _lib.PoolDesc(device=dev.index or 0, dtype=dtype_code(dtype), batch=batch, num_tokens=num_tokens,
                          embed_dim=embed_dim, num_heads=num_heads, training=int(training), masking=int(masking),
                          min_active=int(min_active), q_is_shared=int(q_is_shared),
@@ -135,7 +168,8 @@ def make_pool_desc(dev: torch.device, dtype: torch.dtype, *, batch: int, num_tok
                          loss_out=None if loss_out is None else loss_out.data_ptr(),
                          loss_workspace=None if loss_workspace is None else loss_workspace.data_ptr(),
                          loss_target=float(loss_target),
-                         row_index=None if row_index is None else row_index.data_ptr(), src_rows=int(src_rows))
+                         row_index=None if row_index is None else row_index.data_ptr(), src_rows=int(src_rows),
+                         param_grads_f32=int(param_grads_f32))
 
 
 def fold_score_cols(dtype: torch.dtype, num_heads: int) -> Tuple[int, int]:

@@ -10,6 +10,10 @@ own (``aecf_gemm``: tcgen05 for bf16, SIMT for fp32) instead of ``nn.Linear`` ->
 
 ``lin`` is any module with ``weight [N, K]`` and ``bias [N] | None`` (``nn.Linear`` as the reference builds it), so
 state_dicts stay interchangeable with the reference model's.
+
+Mixed precision: an fp32 ``lin`` applied to a bf16 input runs in bf16 on a bf16 rounding of its weight and bias (one
+``aecf_param_cast`` launch per call, never cached) and returns bf16; ``d_weight`` / ``d_bias`` come out fp32, straight from
+the fp32 sums the bf16 call would round, and the input gradient is bf16.
 """
 from __future__ import annotations
 
@@ -24,6 +28,19 @@ def _dx(g2d: torch.Tensor, weight: torch.Tensor) -> torch.Tensor:
     return ops.matmul_nn(g2d, weight, name="projection d_x")
 
 
+def _is_mixed(x: torch.Tensor, weight: torch.Tensor) -> bool:
+    return x.dtype == torch.bfloat16 and weight.dtype == torch.float32
+
+
+def _shadows(tensors: Sequence) -> List:
+    """bf16 roundings of the given fp32 tensors (``None`` stays ``None``), at most one launch per 8 of them."""
+    out: List = []
+    step = _lib.PARAM_CAST_MAX_SEGMENTS
+    for i in range(0, len(tensors), step):
+        out.extend(ops.param_cast(list(tensors[i:i + step]))[1])
+    return out
+
+
 class _ProjectTokens(torch.autograd.Function):
     @staticmethod
     def forward(ctx, count: int, *args):
@@ -31,11 +48,18 @@ class _ProjectTokens(torch.autograd.Function):
         dev = ops.require_cuda(*xs, *weights)
         B, D = xs[0].shape[0], weights[0].shape[0]
         tokens = torch.empty((B, count, D), dtype=xs[0].dtype, device=dev)
+        mixed = [_is_mixed(x, w) for x, w in zip(xs, weights)]
+        if any(mixed):                                              # fp32 weights, bf16 inputs: compute on bf16 shadows
+            pick = [t if mixed[m % count] else None for m, t in enumerate((*weights, *biases))]
+            cast = _shadows(pick)
+            weights = tuple(c if c is not None else w for c, w in zip(cast[:count], weights))
+            biases = tuple(c if mixed[m] else b for m, (c, b) in enumerate(zip(cast[count:], biases)))
         for m, (x, w, b) in enumerate(zip(xs, weights, biases)):
             if x.dim() != 2 or x.shape[0] != B or w.shape != (D, x.shape[1]):
                 raise ValueError("project_tokens: every modality needs a [B, K_m] input and a [D, K_m] weight")
             ops.linear(x.contiguous(), w, b, out=tokens[:, m, :], ldc=count * D, name=f"token projection {m}")
         ctx.count = count
+        ctx.mixed = mixed
         ctx.has_bias = [b is not None for b in biases]
         ctx.save_for_backward(*xs, *weights)
         return tokens
@@ -53,10 +77,11 @@ class _ProjectTokens(torch.autograd.Function):
             g = d_tokens[:, m, :]                                   # [B, D], row stride count * D, read in place
             if ctx.needs_input_grad[1 + m]:
                 d_x[m] = _dx(g, weights[m])
+            grad_dtype = torch.float32 if ctx.mixed[m] else None    # fp32 gradients of fp32 masters
             if ctx.needs_input_grad[1 + count + m]:
-                d_w[m] = ops.matmul_tn(g, xs[m].contiguous(), name=f"token projection {m} d_weight")
+                d_w[m] = ops.matmul_tn(g, xs[m].contiguous(), out_dtype=grad_dtype, name=f"token projection {m} d_weight")
             if ctx.has_bias[m] and ctx.needs_input_grad[1 + 2 * count + m]:
-                d_b[m] = ops.colsum(g)
+                d_b[m] = ops.colsum(g, out_dtype=grad_dtype)
         return (None, *d_x, *d_w, *d_b)
 
 
@@ -72,6 +97,9 @@ class _Linear(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, weight, bias):
         ops.require_cuda(x, weight, bias)
+        ctx.mixed = _is_mixed(x, weight)
+        if ctx.mixed:                                               # fp32 weight, bf16 input: compute on bf16 shadows
+            weight, bias = _shadows([weight, bias])
         ctx.save_for_backward(x, weight)
         ctx.has_bias = bias is not None
         return ops.linear(x, weight, bias, name="linear")
@@ -80,9 +108,10 @@ class _Linear(torch.autograd.Function):
     def backward(ctx, g):
         x, weight = ctx.saved_tensors
         g = g.contiguous()
+        grad_dtype = torch.float32 if ctx.mixed else None          # fp32 gradients of fp32 masters
         d_x = _dx(g, weight) if ctx.needs_input_grad[0] else None
-        d_w = ops.matmul_tn(g, x, name="linear d_weight") if ctx.needs_input_grad[1] else None
-        d_b = ops.colsum(g) if (ctx.has_bias and ctx.needs_input_grad[2]) else None
+        d_w = ops.matmul_tn(g, x, out_dtype=grad_dtype, name="linear d_weight") if ctx.needs_input_grad[1] else None
+        d_b = ops.colsum(g, out_dtype=grad_dtype) if (ctx.has_bias and ctx.needs_input_grad[2]) else None
         return d_x, d_w, d_b
 
 

@@ -4,6 +4,7 @@
 
     python examples/train_vlm.py --steps 30
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 examples/train_vlm.py --steps 30
+    python examples/train_vlm.py --dtype mixed     # fp32 master parameters, bf16 features and compute
 
 The fusion parameters go through aecf_b200.dp.GradientSync (summed over the ranks inside the pool's backward); the two
 encoder projections and the classifier are the model's nn.Linear PARAMETERS driven by the library's GEMMs
@@ -34,7 +35,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--batch", type=int, default=16384, help="rows per GPU")
     ap.add_argument("--heads", type=int, default=1, help="the README model uses the default single head")
-    ap.add_argument("--dtype", choices=["bf16", "fp32"], default="bf16")
+    ap.add_argument("--dtype", choices=["bf16", "fp32", "mixed"], default="bf16",
+                    help="mixed: fp32 parameters and optimizer, bf16 features; every GEMM and the pool run in bf16")
     ap.add_argument("--launch-list", action="store_true", help="rank 0: kernel names of one step (torch profiler)")
     args = ap.parse_args()
 
@@ -45,10 +47,11 @@ def main():
     if world > 1:
         os.environ.setdefault("NCCL_DEBUG", "WARN")
         dist.init_process_group("nccl", device_id=dev)
-    dtype = torch.bfloat16 if args.dtype == "bf16" else torch.float32
+    dtype = torch.float32 if args.dtype == "fp32" else torch.bfloat16          # of the features
+    param_dtype = torch.bfloat16 if args.dtype == "bf16" else torch.float32
 
     torch.manual_seed(0)                                       # same init on every rank
-    model = VisionLanguageModel(num_heads=args.heads).to(dev, dtype)
+    model = VisionLanguageModel(num_heads=args.heads).to(dev, param_dtype)
     sync = GradientSync(model.fusion_pool, model.fusion_query).attach()
     sync.set_shard(args.batch * world)
     fusion_ids = {id(p) for p in sync.params.values()}

@@ -108,7 +108,10 @@ typedef struct aecf_pool_desc {
     float*   loss_out;        /* [1] fp32, nullable */
     void*    loss_workspace;  /* aecf_pool_loss_workspace_bytes() bytes, zeroed ONCE by the caller (the kernel re-arms it) */
     float    loss_target;     /* entropy_target * log(_last_seq_len), the value CurriculumMasking.entropy_loss would use */
-    int32_t  reserved0;
+    /* Whole-step entry points only: 1 = mixed precision (see "mixed precision" there): the parameter pointers of
+     * aecf_fusion_tensors are bf16 shadows of fp32 parameters and the parameter gradients of aecf_fusion_grads are fp32.
+     * Needs dtype == AECF_BF16; 0 = every tensor not marked fp32 is in dtype; any other value is AECF_ERR_INVALID. */
+    int32_t  param_grads_f32;
     /* Row indirection (reference xrays/train_xrays_example.py:202-222 gathers the rows where both modalities are present,
      * pools them and scatters the result back; here the pool kernels do both ends themselves).  With row_index non-null,
      * `batch` counts the LISTED rows: row i of this call -- its Philox row (row0 + i), its pooled / entropy / mask_rate /
@@ -286,12 +289,32 @@ AECF_API int aecf_sdpa_bwd(int32_t device, int32_t dtype, const void* q, const v
                   void* d_q, void* d_k, void* d_v, void* workspace, size_t workspace_bytes, int64_t batch,
                   int32_t tgt_len, int32_t src_len, int32_t embed_dim, void* stream);
 
+/* ---- parameter shadow (mixed precision) ---------------------------------------------------------
+ * One launch rounds up to AECF_PARAM_CAST_MAX_SEGMENTS fp32 segments to bf16 (round to nearest even, like
+ * Tensor.bfloat16(); NaN stays NaN, +-inf stays +-inf, values past the bf16 range round to +-inf) into one block:
+ * segment i of counts[i] elements lands at element offset(i) of dst, offset(0) = 0 and
+ * offset(i + 1) = offset(i) + counts[i] rounded up to 8, so every segment starts on a 16-byte boundary (a valid
+ * GEMM / TMA operand).  Padding elements are not written.  src / counts are HOST arrays of `segments` entries
+ * (device pointers / element counts); dst must be 16-byte aligned. */
+#define AECF_PARAM_CAST_MAX_SEGMENTS 8
+AECF_API int aecf_param_cast(int32_t device, int32_t segments, const float* const* src, const int64_t* counts, void* dst,
+                             void* stream);
+
 /* ---- whole-step entry points -------------------------------------------------------------
  * The complete forward and backward of MultimodalAttentionPool (reference aecf/AECFLayer.py:515-541 and
  * the autograd graph behind it) as one call each, so the host pays one FFI crossing per direction instead
  * of one per kernel.  They run exactly the calls above, in order, on `stream`.
  * All pointers are device pointers; nullable ones are marked.  `dtype` of the descriptor is the type of
- * every tensor not marked fp32. */
+ * every tensor not marked fp32.
+ *
+ * Mixed precision (desc->param_grads_f32 = 1, dtype = AECF_BF16): fp32 master parameters, bf16 compute, as
+ * torch.autocast trains.  The caller rounds the fp32 parameters to bf16 once per forward (aecf_param_cast) and passes
+ * those shadows as in_proj_weight / in_proj_bias / out_proj_weight / out_proj_bias (and, with a shared query, as
+ * query); the forward and the backward then compute exactly what dtype = AECF_BF16 computes with those parameters.
+ * The parameter gradients -- d_in_proj_weight, d_in_proj_bias, d_out_proj_weight, d_out_proj_bias and, with a shared
+ * query, d_query -- are written in fp32, from the fp32 values the bf16 call would have rounded: rounded to bf16
+ * they are bit for bit the bf16 call's gradients.  Every other tensor (key, value, per-row query and their
+ * gradients, out, ctx, d_out ...) stays bf16. */
 typedef struct aecf_fusion_tensors {
     /* inputs */
     const void*  query;            /* q_is_shared ? [D] : [B, D] */
@@ -406,7 +429,7 @@ typedef enum aecf_site {
     AECF_SITE_D_OUT_BIAS, AECF_SITE_D_OUT_WEIGHT, AECF_SITE_D_CTX, AECF_SITE_POOL_BWD, AECF_SITE_POOL_BWD_FINALIZE,
     AECF_SITE_D_X, AECF_SITE_D_KV_WEIGHT, AECF_SITE_D_Q_WEIGHT, AECF_SITE_D_QUERY, AECF_SITE_D_IN_BIAS,
     AECF_SITE_ENTROPY_LOSS, AECF_SITE_FOLD_PREPARE, AECF_SITE_FOLD_FINISH, AECF_SITE_GRAD_GATHER, AECF_SITE_GRAD_PEER_SUM,
-    AECF_SITE_GRAD_FINISH, AECF_SITE_COUNT
+    AECF_SITE_GRAD_FINISH, AECF_SITE_PARAM_CAST, AECF_SITE_COUNT
 } aecf_site;
 AECF_API int         aecf_timing_enable(int32_t enable);                    /* clears earlier records */
 AECF_API int         aecf_timing_collect(float* total_ms, int32_t* launches); /* arrays of AECF_SITE_COUNT; syncs */

@@ -5,6 +5,8 @@
     python scripts/sass_diff.py compare BEFORE AFTER --pair ARG
                                                        # the same, after a new trailing template argument: an old function
                                                        # is compared with the new one whose last template argument is ARG
+                                                       # (ARG "=": the one whose last argument repeats the one before it,
+                                                       # f<float> -> f<float, float> and f<bf16> -> f<bf16, bf16> at once)
     python scripts/sass_diff.py manifest DIR OUT.json  # {demangled function: [sha1, instructions]} of a snapshot
     python scripts/sass_diff.py check OUT.json DIR     # a snapshot against a committed manifest (exit 1 on a change)
 
@@ -64,14 +66,21 @@ def paired(a, b, arg):
     old = {v: k for k, v in demangle_all(sorted(a)).items()}
     out, pairs = {}, 0
     for k, v in b.items():
-        head, sep, tail = names[k].rpartition(f", {arg}>(")
+        if arg == "=":
+            head, sep, tail = names[k].rpartition(">(")
+            pre, comma, last = head.rpartition(", ")
+            sep = sep if comma and re.split(r"<|, ", pre)[-1] == last else ""
+            head = pre
+        else:
+            head, sep, tail = names[k].rpartition(f", {arg}>(")
         key = old.get(head + ">(" + tail) if sep else None
         if key is not None:
             out[key] = v
             pairs += 1
         else:
             out[k] = v
-    print(f"{pairs} functions paired with their name before the trailing template argument {arg}")
+    what = "a repeated" if arg == "=" else "the"
+    print(f"{pairs} functions paired with their name before {what} trailing template argument" + ("" if arg == "=" else f" {arg}"))
     return out
 
 
