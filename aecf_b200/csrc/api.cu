@@ -2,7 +2,6 @@
 #include <atomic>
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <type_traits>
 
@@ -26,11 +25,6 @@ int use_device(int device) {
     return AECF_OK;
 }
 
-bool pdl_enabled() {
-    static const bool on = [] { const char* e = getenv("AECF_PDL"); return !(e && e[0] == '0'); }();
-    return on;
-}
-
 int sm_count(int device) {
     static std::atomic<int> cached[64];
     if (device < 0 || device >= 64) return 148;
@@ -43,7 +37,7 @@ int sm_count(int device) {
 }
 
 constexpr int POOL_BWD_MAX_BLOCKS = 2048;
-constexpr long long POOL_BWD_CHUNK = 16;     // samples per CTA of the pool backward (0: persistent grid-stride schedule)
+constexpr long long POOL_BWD_CHUNK = 16;     // samples per CTA of the pool backward without batch sums (chunked schedule)
 
 // Sum the per-block partials: d_q[D] (scaled) and d_bias_kv[2D] = [dbk | dbv].  Block (32 columns x 32
 // lanes): lane y sums partials y, y+32, ... in order (all loads issued together), the 32 lane sums are
@@ -325,17 +319,13 @@ static int pool_bwd_impl(const aecf_pool_desc* desc, bool fold, const void* q, c
     int grid = static_cast<int>(want < cap ? want : cap);
     if (grid < 1) grid = 1;
     // Chunked schedule (pool_bwd.cuh), for the kernel without batch sums: CTA b owns `chunk` consecutive samples, several
-    // CTAs per resident slot, handed out by the block scheduler as CTAs retire.  AECF_POOL_BWD_CHUNK: samples per CTA
-    // (0: the persistent schedule) -- a measurement switch.
+    // CTAs per resident slot, handed out by the block scheduler as CTAs retire.  POOL_BWD_CHUNK samples per CTA, rounded
+    // up to whole slices of SPC samples and doubled until the grid fits in an int.
     if (no_sums) {
-        static const long long env_chunk = [] { const char* e = getenv("AECF_POOL_BWD_CHUNK"); return e ? atoll(e) : -1LL; }();
-        long long chunk = env_chunk >= 0 ? env_chunk : POOL_BWD_CHUNK;
-        if (chunk > 0) {
-            chunk = (chunk + p.SPC - 1) / p.SPC * p.SPC;
-            while ((p.B + chunk - 1) / chunk > 0x7fffffffLL) chunk *= 2;
-            p.chunk = chunk;
-            grid = static_cast<int>((p.B + chunk - 1) / chunk);
-        }
+        long long chunk = (POOL_BWD_CHUNK + p.SPC - 1) / p.SPC * p.SPC;
+        while ((p.B + chunk - 1) / chunk > 0x7fffffffLL) chunk *= 2;
+        p.chunk = chunk;
+        grid = static_cast<int>((p.B + chunk - 1) / chunk);
     }
 
     {

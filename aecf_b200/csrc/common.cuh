@@ -80,8 +80,7 @@ int launch_query_tail(int dtype, int grad_dtype, int D, const float* d_qp, const
 // pdl_wait(): its CTAs may be scheduled while the previous kernel of the stream is still draining
 // (launch latency and per-CTA prologues -- barrier init, TMEM allocation, tensor-map prefetch --
 // overlap that tail), but nothing touches global memory before the previous kernel has completed and
-// flushed.  AECF_PDL=0 in the environment falls back to ordinary launches.
-bool pdl_enabled();
+// flushed.
 #ifdef AECF_CUDA_EMU
 __device__ __forceinline__ void pdl_wait() {}
 
@@ -105,7 +104,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 // An ordinary launch (kernels that do not start with pdl_wait()).

@@ -14,7 +14,6 @@
 // restated in cute/arch/mma_sm100_desc.hpp (SmemDescriptor, InstrDescriptor).
 #include <cuda.h>
 
-#include <cstdlib>
 #include <mutex>
 
 #include "gemm.cuh"
@@ -57,10 +56,6 @@ struct Params {
     int c_cols, aux_cols;
     long long aux_ld;
     float* aux;
-    // MEASUREMENT ONLY (AECF_GEMM_DEBUG_SKIP, scripts/gemm_bench.py): bit 0 = no operand loads and no MMAs (the epilogue
-    // alone, on whatever the accumulator holds), bit 1 = no epilogue (the main loop alone, nothing stored).  Results are
-    // garbage; the two times say which half of a kernel bounds it.
-    int debug_skip;
 };
 
 #ifdef AECF_CUDA_EMU
@@ -331,7 +326,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         // ===== TMA producer: the whole warp walks the loop, one elected lane issues (see elect_one) =====
         constexpr int PART = BN / CL;                 // this CTA's share of the B tile
         int it = 0;
-        for (int item = first_item; item < items && !(p.debug_skip & 1); item += item_stride) {
+        for (int item = first_item; item < items; item += item_stride) {
             const WorkItem w = decode<CL>(p, item, cta_rank);
             for (int kb = 0; kb < w.kb_count; ++kb, ++it) {
                 const int s = it % STAGES;
@@ -379,7 +374,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             mbar_wait(&tmem_empty[as], ((tile_it >> 1) & 1) ^ 1);          // epilogue drained this accumulator
             tc_fence_after();
             const uint32_t tmem_d = tmem_base + as * C::ACC_STRIDE;
-            for (int kb = 0; kb < w.kb_count && !(p.debug_skip & 1); ++kb, ++it) {
+            for (int kb = 0; kb < w.kb_count; ++kb, ++it) {
                 const int s = it % STAGES;
                 mbar_wait(&full[s], (it / STAGES) & 1);
                 tc_fence_after();
@@ -415,7 +410,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             const bool direct = (p.splits == 1);
             mbar_wait(&tmem_full[as], (tile_it >> 1) & 1);
             tc_fence_after();
-            if (p.debug_skip & 2) { tc_fence_before(); mbar_arrive(&tmem_empty[as]); continue; }
             // fp32 bias slice of this tile, in the buffer of this tile's parity.  All four warps write the same
             // values; a warp two tiles ahead would reuse this buffer, but it cannot pass the tmem_full wait
             // above before every thread has finished the tile that last used it (tmem_empty arrives after the
@@ -670,8 +664,7 @@ static Plan make_plan(const aecf_gemm_desc* d, int aux_cols = 0) {
     pl.kb_total = static_cast<int>((d->k + tc::BK - 1) / tc::BK);
     // Pairs of CTAs (a cluster of 2) on vertically adjacent row blocks share the B tile by TMA multicast:
     // a third less L2 -> SM traffic per FLOP, which is what bounds these K = 512..1024 products.
-    static const bool no_cluster = [] { const char* e = getenv("AECF_GEMM_CLUSTER"); return e && e[0] == '1'; }();
-    pl.cluster = (pl.tiles_m >= 2 && !no_cluster) ? 2 : 1;
+    pl.cluster = pl.tiles_m >= 2 ? 2 : 1;
     pl.two_sm = false;        // decided below, once the k range of a work item is known
     pl.groups_m = (pl.tiles_m + pl.cluster - 1) / pl.cluster;
     const int sms = sm_count(d->device);
@@ -689,10 +682,9 @@ static Plan make_plan(const aecf_gemm_desc* d, int aux_cols = 0) {
     // fewer operand bytes delivered per FLOP, and a deeper ring).  A/B on one box with the warp-uniform issue loops
     // (profiles/r1_gemm_experiments.md, run 24): it wins from 9 k-blocks per work item on -- dX (K = 520) 109 -> 103 us,
     // [dWv ; R] 121 -> 112 us even though its 520 rows fill only 2.03 of 3 CTA pairs -- and loses on the 8-k-block
-    // products (out_proj 38 -> 42 us), whose per-tile pair handshake is not amortised.  AECF_GEMM_2SM=0/1 forces it.
-    static const int force_2sm = [] { const char* e = getenv("AECF_GEMM_2SM"); return e ? (e[0] == '1' ? 1 : 0) : -1; }();
+    // products (out_proj 38 -> 42 us), whose per-tile pair handshake is not amortised.
     const bool long_k = pl.kb_per_split >= 9;
-    pl.two_sm = pl.cluster == 2 && pl.bn == 256 && (force_2sm < 0 ? long_k : force_2sm == 1);
+    pl.two_sm = pl.cluster == 2 && pl.bn == 256 && long_k;
     if (aux_cols > 0 && pl.splits != 1) return pl;       // the side output is written by the direct epilogue only
     pl.ok = true;
     return pl;
@@ -744,8 +736,6 @@ int gemm_tcgen05(const aecf_gemm_desc* d, const void* A, const void* B, const vo
     p.c_is_f32 = c_f32;
     p.has_bias = bias != nullptr; p.bias_is_bf16 = d->dtype_bias == AECF_BF16; p.bias = bias;
     p.partial_rows = pl.tiles_m * BM;              // padded: a ragged last row block must not spill into the next split
-    static const int debug_skip = [] { const char* e = getenv("AECF_GEMM_DEBUG_SKIP"); return e ? atoi(e) & 3 : 0; }();
-    p.debug_skip = debug_skip;
 
     const long long items = static_cast<long long>(pl.groups_m) * pl.tiles_n * pl.splits;     // one per cluster
     const int sms = sm_count(d->device);
@@ -761,7 +751,7 @@ int gemm_tcgen05(const aecf_gemm_desc* d, const void* A, const void* B, const vo
     attr[0].val.clusterDim.x = pl.cluster; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 2 : 1;
+    cfg.attrs = attr; cfg.numAttrs = 2;
 #define AECF_TC_LAUNCH(BN_, CL_)                                                                                  \
     do {                                                                                                          \
         auto kernel = gemm_tcgen05_kernel<BN_, CL_>;                                                              \

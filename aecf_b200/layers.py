@@ -432,7 +432,7 @@ class MultimodalAttentionPool(nn.Module):
             seed=seed, offset=offset, rng_state=rng_state, row0=int(self.row_offset), q_shared=q_shared,
             seq_first=not self.batch_first, fold=fold, want_mask_bits=self._want_mask_bits, bias_strides=bias_strides,
             tgt_len=tgt_len, grad_ready=self._grad_ready, grad_buffers=self._grad_buffers,
-            loss_target=cm._loss_target() if (masking == 1 and return_info and os.environ.get("AECF_FUSED_LOSS", "1") != "0") else None,
+            loss_target=cm._loss_target() if (masking == 1 and return_info) else None,
             side=self._side_stream(key.device) if fold else None, dp=self._dp, sample_index=index, mixed=mixed)
         info_rows = batch if index is None else int(index.numel())
         out, pooled, entropy, mask_rate, masked, bits, fused_loss = FusedPoolFunction.apply(

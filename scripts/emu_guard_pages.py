@@ -1,6 +1,6 @@
 """Offline check: every tensor torch.empty/zeros/randn hands out ends right before a PROT_NONE page, then the emulated
 product path runs a set of cases; an out-of-bounds access past any buffer's end is a segfault (faulthandler prints it)."""
-import ctypes, faulthandler, mmap, os, sys
+import ctypes, faulthandler, mmap, sys
 import torch
 faulthandler.enable()
 sys.path.insert(0, __import__("os").path.dirname(__import__("os").path.dirname(__import__("os").path.abspath(__file__))))
@@ -58,7 +58,5 @@ for c in cases:
         P.test_bf16_masks_exact_against_stage_rounded_oracle(c, True); P.test_bf16_masks_exact_against_stage_rounded_oracle(c, False); n += 2
 for c in MULTI_QUERY_CASES[:3]:
     MQ.test_fp32_matches_oracle(c, True); MQ.test_fp32_matches_oracle(c, False); n += 2
-for env in (None, "1"):
-    if env: os.environ["AECF_POOL_BWD_STREAM"] = env
-    P.test_bf16_masks_exact_against_stage_rounded_oracle(cases[1], True); n += 1
+P.test_bf16_masks_exact_against_stage_rounded_oracle(cases[1], True); n += 1
 print("ok:", n, "runs with every buffer ending at a guard page,", len(keep), "guarded buffers")

@@ -2,11 +2,9 @@
 
     python scripts/gemm_bench.py [--cublas] [--tag NAME]
 
-Kernel variants are chosen by the library's environment switches (read once per process), so an A/B is one process
-per variant (scripts/gpu_r2_run2.sh).  Every product rotates over enough operand sets that no call finds its
-operands in the 126 MB L2.  --cublas also times torch.matmul on the same shapes (a yardstick, not a product path).
-AECF_GEMM_DEBUG_SKIP=1|2 (measurement only) removes the main loop / the epilogue: results are then garbage and the
-correctness check is skipped.
+The library picks each product's kernel from its shape, as in a training step; the kernel that ran is reported per
+product.  Every product rotates over enough operand sets that no call finds its operands in the 126 MB L2.  --cublas also
+times torch.matmul on the same shapes (a yardstick, not a product path).
 """
 import argparse
 import json
@@ -44,7 +42,6 @@ def main():
     ap.add_argument("--tag", default="")
     ap.add_argument("--only", default="")
     args = ap.parse_args()
-    skip = int(os.environ.get("AECF_GEMM_DEBUG_SKIP", "0"))
     rows = B * M
     bf = torch.bfloat16
     rnd = lambda *s: (torch.randn(*s, device=DEV) * 0.1).to(bf)
@@ -61,11 +58,9 @@ def main():
         kern = _lib.gemm_last_kernel()
         flops = ops_sets[0]["flops"]
         r = {"us": us, "tflops": flops / us / 1e6, "kernel": kern}
-        if skip == 0:
-            got, want = ops_sets[0]["call"](), ops_sets[0]["ref"]()
-            torch.cuda.synchronize()
-            err = float((got.float() - want.float()).abs().max() / want.float().abs().max())
-            r["rel_err"] = err
+        got, want = ops_sets[0]["call"](), ops_sets[0]["ref"]()
+        torch.cuda.synchronize()
+        r["rel_err"] = float((got.float() - want.float()).abs().max() / want.float().abs().max())
         if args.cublas:
             r["cublas_us"] = time_us(lambda i: ops_sets[i]["ref"](), sets)
         res[name] = r

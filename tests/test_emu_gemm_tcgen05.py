@@ -49,8 +49,6 @@ def test_cta_pair_kernels_with_an_odd_number_of_row_blocks():
     """TMA stores of the emulation read their staging box at the latest moment the kernel allows.  Five row blocks on CTA
     pairs leave a filler tile; every epilogue round commits one (possibly empty) bulk group, so `wait_group.read 1` keeps
     protecting the buffer of the previous tile's last store.  (The round-1 instantiation without that commit failed here.)"""
-    if os.environ.get("AECF_GEMM_CLUSTER") == "1":
-        pytest.skip("without clusters the product runs on the single-CTA kernel")
     G.test_tcgen05_gemm((640, 256, 640), _lib.K_MAJOR, _lib.K_MAJOR)
 
 
@@ -75,16 +73,15 @@ def test_whole_step_on_the_tensor_core_gemms():
 def test_reported_kernel():
     """aecf_gemm_last_kernel() names what ran (bench.py records it per launch site)."""
     from aecf_b200 import ops
-    cluster = "1" if os.environ.get("AECF_GEMM_CLUSTER") == "1" else "2"
     bf = torch.bfloat16
     a, b = torch.randn(512, 128, dtype=bf), torch.randn(256, 128, dtype=bf)
     ops.gemm(a, b, m=512, n=256, k=128, a_layout=_lib.K_MAJOR, b_layout=_lib.K_MAJOR, lda=128, ldb=128)           # 2 k-blocks
-    assert _lib.gemm_last_kernel() == f"tcgen05 1sm bn256 cluster{cluster} splits1"
+    assert _lib.gemm_last_kernel() == "tcgen05 1sm bn256 cluster2 splits1"
     a, b = torch.randn(512, 640, dtype=bf), torch.randn(256, 640, dtype=bf)
     ops.gemm(a, b, m=512, n=256, k=640, a_layout=_lib.K_MAJOR, b_layout=_lib.K_MAJOR, lda=640, ldb=640)           # 10 k-blocks
-    assert _lib.gemm_last_kernel() == ("tcgen05 2sm bn256 splits1" if cluster == "2" else "tcgen05 1sm bn256 cluster1 splits1")
+    assert _lib.gemm_last_kernel() == "tcgen05 2sm bn256 splits1"
     a, b = torch.randn(640, 512, dtype=bf), torch.randn(520, 512, dtype=bf)
     ops.gemm_aux(a, b, m=640, n=512, k=512, aux_cols=8)
-    assert _lib.gemm_last_kernel() == f"tcgen05 1sm bn192 cluster{cluster} splits1"
+    assert _lib.gemm_last_kernel() == "tcgen05 1sm bn192 cluster2 splits1"
     ops.gemm(a[:64].float(), b[:64].float(), m=64, n=64, k=512, a_layout=_lib.K_MAJOR, b_layout=_lib.K_MAJOR, lda=512, ldb=512)
     assert _lib.gemm_last_kernel() == "simt"
