@@ -180,11 +180,12 @@ static int folded_backward(const aecf_pool_desc* desc, const Geometry& g, const 
         const aecf_gemm_desc d = gemm_desc(dev, dt, dt, dt, dt, AECF_K_MAJOR, AECF_MN_MAJOR, g.QR, D, D, D, D, D);
         AECF_TRY(aecf_gemm(&d, gr->d_out, t->out_proj_weight, nullptr, gr->d_ctx, w.gemm, w.gemm_bytes, s));
     }
-    // The value and key thirds of the in-projection bias gradient (pool_bwd.cuh).  No dropout, every sample pooled: the
-    // softmax weights of a sample sum to one, so d_bias_v = sum_b d_ctx[b, :] = Wo^T colsum(d_out) and d_bias_k = 0 -- the tail
-    // forms them from the column sums of d_out and the pool backward carries no batch sums at all.  Otherwise the kernel
-    // leaves [s | sum_m ds] per sample and head and the tail walks d_ctx once more.
-    const bool bias_from_bo = desc->row_index == nullptr && !(desc->training && desc->dropout_p > 0.f);
+    // The value and key thirds of the in-projection bias gradient (pool_bwd.cuh).  No dropout, no mask, every sample pooled:
+    // the softmax weights of a sample sum to one, so d_bias_v = sum_b d_ctx[b, :] = Wo^T colsum(d_out) and d_bias_k = 0 -- the
+    // tail forms them from the column sums of d_out and the pool backward carries no batch sums at all.  Otherwise the kernel
+    // leaves [s | sum_m ds] per sample and head and the tail walks d_ctx once more.  A mask can cover every token of a
+    // sample: its weights are then NaN, not summing to one, and these sums are NaN as in torch.
+    const bool bias_from_bo = desc->row_index == nullptr && t->score_bias == nullptr && !(desc->training && desc->dropout_p > 0.f);
     float* rowsum = (gr->d_in_proj_bias && !bias_from_bo) ? w.rowsum : nullptr;
     if (desc->row_index != nullptr) {                            // unlisted samples: zero rows of [dV | ds], no share in the bias sums
         AECF_CUDA_OK(cudaMemsetAsync(gr->d_kv, 0, static_cast<size_t>(g.rows) * KF * g.es, s));

@@ -260,7 +260,9 @@ __global__ void curriculum_mask_kernel(const float* __restrict__ weights, long l
     if (mask_rate) mask_rate[row] = __fsub_rn(1.0f, static_cast<float>(active) / static_cast<float>(len));
 }
 
-// d_weights[i] = d_entropy * -(log w_i + 1) inside the clamp, else 0 (eval-mode entropy stays attached, :151-156)
+// Eval-mode entropy stays attached (:151-156).  d_weights[i] = -g (xlogy(w_i != 0, w_i) + w_i / w_i) with g = d_entropy
+// inside the clamp, else 0: autograd's backward of clamp(-sum xlogy(w, w)) term by term, so that a zero weight gets
+// 0 / 0 = NaN as it does in torch -- also where the clamp passes no gradient -- and not -(log 0 + 1) = +inf.
 __global__ void entropy_bwd_kernel(const float* __restrict__ weights, long long rows, int len, float log_len,
                                    const float* __restrict__ d_entropy, float* __restrict__ d_weights) {
     const long long row = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -270,8 +272,9 @@ __global__ void entropy_bwd_kernel(const float* __restrict__ weights, long long 
     float raw;
     entropy_of(w, len, log_len, &raw);
     const bool inside = (raw >= 0.f) && (raw <= log_len);
-    const float g = d_entropy[row];
-    for (int i = 0; i < len; ++i) d_weights[row * len + i] = inside ? -(logf(w[i]) + 1.0f) * g : 0.f;
+    const float g = inside ? d_entropy[row] : 0.f;
+    for (int i = 0; i < len; ++i)
+        d_weights[row * len + i] = -((w[i] != 0.f ? logf(w[i]) : 0.f) + w[i] / w[i]) * g;
 }
 
 // ---- projection-free single-head attention (reference aecf/AECFLayer.py:556-581) ------------

@@ -76,7 +76,7 @@ pool_bwd_kernel(const PoolParams p) {
     //   d_bias_v[d] = sum_b s[b, h(d)] d_ctx[b, d],  s = sum_m wd       d_bias_k[d] = scale q[d] sum_b sum_m ds[b, m, h(d)]
     // Without dropout s = sum_m softmax = 1 and sum_m ds = 0 identically, so d_bias_v = sum_b d_ctx[b, :] = Wo^T d_bias_o and
     // d_bias_k = 0: the gradient tail forms them from the column sums of d_out it already has (grad_tail.cu), and nothing is
-    // left to do here (p.rowsum == null).  With dropout, or when only listed samples are pooled, the kernel leaves
+    // left to do here (p.rowsum == null).  With dropout, a mask, or when only listed samples are pooled, the kernel leaves
     // [s | sum_m ds] per sample and head in p.rowsum and the tail walks d_ctx once more.
     const bool sums = p.partials != nullptr;
     if (sums) for (int i = lane; i < Smem::PER_WARP; i += 32) strip[i] = 0.f;

@@ -269,12 +269,14 @@ def pool_backward(query: Tensor, key: Tensor, value: Optional[Tensor],
     d_pooled = None if grad_pooled is None else grad_pooled.reshape(B, S, M)
     if grad_entropy is not None:
         # eval mode only: entropy = clamp(-sum xlogy(p, p), 0, log M) stays attached
-        # (reference aecf/AECFLayer.py:151-156); d/dp = -(log p + 1) inside the clamp.
+        # (reference aecf/AECFLayer.py:151-156).  Autograd's chain term by term: the clamp passes the gradient inside
+        # its range and 0 outside; xlogy(p, p) contributes xlogy(p != 0, p) + p / p, which is 0 / 0 = NaN at p = 0
+        # whatever the clamp passed.
         pooled = wd.mean(dim=1)                                       # [B,S,M]
         raw = -torch.xlogy(pooled, pooled).sum(-1, keepdim=True)
         inside = (raw >= 0.0) & (raw <= math.log(M))
-        d_h = torch.where(inside, -(pooled.log() + 1.0), torch.zeros((), dtype=pooled.dtype))
-        d_h = d_h * grad_entropy.reshape(B, S, 1)
+        g_raw = torch.where(inside, grad_entropy.reshape(B, S, 1), torch.zeros((), dtype=pooled.dtype))
+        d_h = -g_raw * (torch.xlogy((pooled != 0).to(pooled.dtype), pooled) + pooled / pooled)
         d_pooled = d_h if d_pooled is None else d_pooled + d_h
     if d_pooled is not None:
         d_wd = d_wd + d_pooled.reshape(B, 1, S, M) / H

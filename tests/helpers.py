@@ -2,6 +2,7 @@
 from __future__ import annotations
 
 import json
+import math
 import os
 from typing import Dict, Optional
 
@@ -57,15 +58,32 @@ def run_oracle(case: Case, inp: Optional[dict] = None, dtype: Optional[torch.dty
     return fwd, grads
 
 
+def finite_scale(t) -> float:
+    """The largest magnitude among the finite elements of t (0 when there are none)."""
+    t = torch.as_tensor(t).detach().double()
+    t = t[torch.isfinite(t)]
+    return float(t.abs().max()) if t.numel() else 0.0
+
+
 def assert_close(name, got, want, rtol, atol=None):
+    """got matches want: NaN exactly where want has NaN, +inf and -inf exactly where want has them, and the finite
+    elements within atol + rtol |want|.  The default atol is rtol times the largest finite |want|.  A test that allows
+    no non-finite value at all says so with torch.isfinite(...).all()."""
     got = torch.as_tensor(got).double().reshape(-1)
     want = torch.as_tensor(want).double().reshape(-1)
     assert got.shape == want.shape, f"{name}: shape {got.shape} vs {want.shape}"
+    finite = torch.isfinite(want)
+    same = torch.where(finite, torch.isfinite(got), torch.isnan(want) & torch.isnan(got) | (got == want))
+    assert bool(same.all()), (
+        f"{name}: non-finite pattern differs at {int((~same).sum())}/{got.numel()} elements, first at "
+        f"{int((~same).nonzero()[0])} (got {int((~torch.isfinite(got)).sum())} non-finite, want {int((~finite).sum())})")
     if atol is None:                       # relative to the tensor's own scale
-        atol = rtol * max(float(want.abs().max()), 1e-30)
+        atol = rtol * max(finite_scale(want), 1e-30)
+    assert math.isfinite(atol), f"{name}: atol {atol} is not finite"
+    got, want = got[finite], want[finite]
     err = (got - want).abs()
     bound = atol + rtol * want.abs()
     bad = err > bound
     assert not bool(bad.any()), (
         f"{name}: {int(bad.sum())}/{got.numel()} beyond rtol={rtol} atol={atol:.3e}; "
-        f"max abs err {float(err.max()):.3e} (scale {float(want.abs().max()):.3e})")
+        f"max abs err {float(err.max()):.3e} (scale {finite_scale(want):.3e})")
