@@ -33,7 +33,7 @@ EXPORTS = (
     "aecf_peer_flag_bytes", "aecf_peer_enable_access", "aecf_peer_allreduce", "aecf_peer_export", "aecf_peer_import",
     "aecf_timing_enable", "aecf_timing_collect", "aecf_timing_site_name", "aecf_timing_site_gemm_kernel",
     "aecf_abi_version", "aecf_strerror", "aecf_last_cuda_error", "aecf_launch_count", "aecf_build_info",
-    "aecf_gemm_last_kernel",
+    "aecf_gemm_last_kernel", "aecf_pool_last_kernel",
 )
 
 
@@ -201,6 +201,8 @@ def _declare(lib):
     lib.aecf_build_info.argtypes = []
     lib.aecf_gemm_last_kernel.restype = C.c_char_p
     lib.aecf_gemm_last_kernel.argtypes = []
+    lib.aecf_pool_last_kernel.restype = C.c_char_p
+    lib.aecf_pool_last_kernel.argtypes = []
 
 
 def load():
@@ -245,6 +247,12 @@ def launch_count() -> int:
 def gemm_last_kernel() -> str:
     """Which kernel the last aecf_gemm / aecf_gemm_aux call of this thread launched (diagnostics, A/B runs)."""
     return load().aecf_gemm_last_kernel().decode()
+
+
+def pool_last_kernel() -> str:
+    """Which pool kernel and schedule the last pool launch of this thread took (the backward of an autograd call runs on
+    autograd's device thread: read it there, e.g. from a gradient hook)."""
+    return load().aecf_pool_last_kernel().decode()
 
 
 def build_info() -> str:

@@ -1,6 +1,7 @@
 // C-ABI entry points for the fused pool, plus library bookkeeping.  See include/aecf_b200.h.
 #include <atomic>
 #include <cmath>
+#include <cstdarg>
 #include <cstdio>
 #include <cstring>
 #include <type_traits>
@@ -11,6 +12,14 @@ namespace aecf {
 
 static std::atomic<unsigned long long> g_launches{0};
 static thread_local char g_cuda_error[256] = "";
+static thread_local char g_last_pool_kernel[128] = "";
+
+void note_pool_kernel(const char* fmt, ...) {
+    va_list ap;
+    va_start(ap, fmt);
+    std::vsnprintf(g_last_pool_kernel, sizeof(g_last_pool_kernel), fmt, ap);
+    va_end(ap);
+}
 
 void count_launch(unsigned n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
 
@@ -199,6 +208,7 @@ const char* aecf_strerror(int status) {
 }
 
 const char* aecf_last_cuda_error(void) { return g_cuda_error; }
+const char* aecf_pool_last_kernel(void) { return g_last_pool_kernel; }
 uint64_t aecf_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 const char* aecf_build_info(void) {
     return "aecf_b200 abi " AECF_STR(AECF_ABI_VERSION) ", sm_100a, nvcc " AECF_STR(__CUDACC_VER_MAJOR__) "." AECF_STR(__CUDACC_VER_MINOR__);
@@ -240,6 +250,7 @@ static int pool_fwd_impl(const aecf_pool_desc* desc, bool fold, const void* q, c
         plan.mq.bias = score_bias;
         p.bias = nullptr;
         const int rows_grid = static_cast<int>((p.B * plan.mq.S + p.SPC - 1) / p.SPC);
+        note_pool_kernel("multi fwd M=%d J=%d PAD=%d grid=%d", plan.M, plan.J, int(plan.pad), rows_grid);
         return with_pool_types(plan, [&](auto t, auto drop, auto pad) {
             return launch_pool_fwd_multi<decltype(t), drop, pad>(plan.M, plan.J, p, plan.mq, rows_grid, stream);
         });
@@ -326,6 +337,11 @@ static int pool_bwd_impl(const aecf_pool_desc* desc, bool fold, const void* q, c
         while ((p.B + chunk - 1) / chunk > 0x7fffffffLL) chunk *= 2;
         p.chunk = chunk;
         grid = static_cast<int>((p.B + chunk - 1) / chunk);
+        note_pool_kernel("bwd chunked M=%d J=%d PAD=%d fold=%d grid=%d chunk=%lld", plan.M, plan.J, int(plan.pad), int(fold),
+                         grid, chunk);
+    } else {                                            // passes: slices of SPC samples per CTA, the last pass partial
+        note_pool_kernel("%s M=%d J=%d PAD=%d fold=%d grid=%d passes=%lld", plan.multi ? "multi bwd" : "bwd grid-stride",
+                         plan.M, plan.J, int(plan.pad), int(fold), grid, (want + grid - 1) / grid);
     }
 
     {

@@ -147,9 +147,10 @@ struct PoolCore {
     static __device__ __forceinline__ size_t row_offset(const PoolParams& p, long long row, int c0) {
         return static_cast<size_t>(row) * p.kv_sb * sizeof(T) + lane_bytes(p, c0);
     }
-    // ... and, relative to it, of chunk column j of the K half (half = 0) or V half (half = 1) of token m
-    static __device__ __forceinline__ int kv_rel(const PoolParams& p, int c0, int m, int half, int j) {
-        return (m * static_cast<int>(p.kv_sm) + half * p.D) * static_cast<int>(sizeof(T)) + col_bytes(p, c0, j);
+    // ... and, relative to it, of chunk column j of the K half (half = 0) or V half (half = 1) of token m.  64-bit: in a
+    // sequence-first layout the token stride is B * 2D elements, so (M - 1) tokens span more than 2^31 bytes at large B.
+    static __device__ __forceinline__ long long kv_rel(const PoolParams& p, int c0, int m, int half, int j) {
+        return (m * p.kv_sm + half * p.D) * static_cast<long long>(sizeof(T)) + col_bytes(p, c0, j);
     }
 
     // the same two offsets inside d_kv (its rows are wider than kv's in the folded layout)

@@ -38,4 +38,6 @@ template <typename T, bool DROP, bool PAD> int pool_bwd_blocks_per_sm(int M, int
 template <typename T, bool DROP, bool PAD> int launch_pool_fwd_multi(int M, int J, const PoolParams& p, const MultiQuery& mq, int grid, void* stream);
 template <typename T, bool DROP, bool PAD> int launch_pool_bwd_multi(int M, int J, const PoolParams& p, const MultiQuery& mq, int grid, void* stream);
 
+void note_pool_kernel(const char* fmt, ...);         // api.cu: records what aecf_pool_last_kernel() reports
+
 }  // namespace aecf

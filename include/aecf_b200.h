@@ -444,6 +444,10 @@ AECF_API uint64_t    aecf_launch_count(void);         /* kernels launched by thi
 AECF_API const char* aecf_build_info(void);           /* "sm_100a nvcc 12.9 ..." */
 AECF_API const char* aecf_gemm_last_kernel(void);     /* host string, thread-local: which kernel the last aecf_gemm[_aux] call of this
                                                          thread launched, e.g. "tcgen05 1sm bn192 cluster2 epi1", "tcgen05 2sm bn256 ew4", "simt" */
+AECF_API const char* aecf_pool_last_kernel(void);     /* host string, thread-local: which pool kernel and schedule the last pool launch
+                                                         of this thread took, e.g. "stream M=3 J=1 PAD=0 fold=1 warps=24 rows_per_warp=19
+                                                         ctas=148", "slice ... grid=N", "bwd grid-stride ... grid=G passes=P",
+                                                         "bwd chunked ... grid=G chunk=C", "multi fwd ... grid=N", "multi bwd ... passes=P" */
 
 #ifdef __cplusplus
 }
